@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the d3d hot path on B200 next to the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--op all|voxel|iou|nms|scatter|dist3d|crop] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--op all|voxel|iou|nms|scatter|dist3d|crop] [--impl reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W      (N > 1)
 
 One JSON line on rank 0.  BASELINE.json's metric is a triple (rotated-IoU pairs/s, NMS boxes/s, voxelized
@@ -380,7 +380,8 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------ GPU timing helpers
-def timed(fn, steps, warmup, barrier):
+def timed(fn, steps, warmup, barrier, last=None):
+    """ms per step of `steps` calls of fn after `warmup` untimed ones; `last` (a list) receives what the final timed call returned"""
     import torch
     for _ in range(warmup):
         fn()
@@ -388,17 +389,20 @@ def timed(fn, steps, warmup, barrier):
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
-        fn()
+    for i in range(steps):
+        if last is not None and i == steps - 1:
+            last.append(fn())
+        else:
+            fn()
     e1.record()
     torch.cuda.synchronize()
     barrier()
     return e0.elapsed_time(e1) / steps   # ms per step
 
 
-def timed_flushed(fn, steps, warmup, barrier):
+def timed_flushed(fn, steps, warmup, barrier, last=None, before_last=None):
     """for operators whose working set fits L2: every step is timed by its own event pair and a 256 MB memset (outside the
-    pairs) evicts L2 between steps"""
+    pairs) evicts L2 between steps; `last` as in timed(); `before_last` runs ahead of the final step's memset"""
     import torch
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
     for _ in range(warmup):
@@ -406,16 +410,63 @@ def timed_flushed(fn, steps, warmup, barrier):
     torch.cuda.synchronize()
     barrier()
     evs = []
-    for _ in range(steps):
+    for i in range(steps):
+        if before_last is not None and i == steps - 1:
+            before_last()
         flush.zero_()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        fn()
+        if last is not None and i == steps - 1:
+            last.append(fn())
+        else:
+            fn()
         e1.record()
         evs.append((e0, e1))
     torch.cuda.synchronize()
     barrier()
     return sum(a.elapsed_time(b) for a, b in evs) / steps
+
+
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_SAMPLE = 1 << 18   # elements kept of one output array: at most 2 MB each, well under 64 MB for all operators together
+DUMP_LIMIT = 64 << 20
+OUTPUTS = {}            # name -> host array of the last timed step, written by main() when --dump-outputs is given
+
+
+def keep_output(args, name, t):
+    """Record what the timed path returned in its last step, as float32 (float32 and bool outputs) or float64 (float64 and integer
+    outputs, exact).  An array of more than DUMP_SAMPLE elements is reduced to the elements at a fixed, seeded set of flat positions,
+    so that two builds run with the same arguments can be compared output for output."""
+    if not args.dump_outputs:
+        return
+    import torch
+    flat = t.detach().reshape(-1)
+    if flat.numel() > DUMP_SAMPLE:
+        idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), DUMP_SAMPLE))
+        a = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    else:
+        a = t.detach().cpu().numpy()
+    OUTPUTS[name] = a.astype(np.float32 if a.dtype in (np.float32, np.bool_) else np.float64)
+
+
+def keep_voxel_outputs(args, prefix, res):
+    """the packed arrays of a VoxelBatch up to its totals: every frame's result dict is a slice of these"""
+    if not args.dump_outputs:
+        return
+    rows = res.rows_host()
+    K, V = int(rows[-1, 0]), int(rows[-1, 1])
+    keep_output(args, f"{prefix}_rows", rows)
+    for k, v in res.packed.items():
+        keep_output(args, f"{prefix}_{k}", v[:K] if k in res.POINT_KEYS else v[:V])
+
+
+def write_outputs(d):
+    total = sum(a.nbytes for a in OUTPUTS.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(d, exist_ok=True)
+    for name, a in OUTPUTS.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def bind_to_gpu_numa(local):
@@ -566,10 +617,13 @@ def bench_voxel(args, rank, world, barrier):
     N = int(dev_pts.shape[0])
     alg_bytes = 16.0 * N + 32.0 * K + 28.0 * V
     del res
+    last = [] if args.dump_outputs else None
     l0 = c.launch_count()
     with ClockSampler(torch.cuda.current_device()) as cs:
-        ms = timed(lambda: gen.batch_packed(dev_pts, offs, offs_dev), args.steps, args.warmup, barrier)
+        ms = timed(lambda: gen.batch_packed(dev_pts, offs, offs_dev), args.steps, args.warmup, barrier, last)
         l1 = c.launch_count()
+        if last:
+            keep_voxel_outputs(args, "voxel", last.pop())
         cs.hold(lambda: gen.batch_packed(dev_pts, offs, offs_dev))
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -629,6 +683,7 @@ def bench_iou(args, rank, world, barrier, f64=False):
     with ClockSampler(torch.cuda.current_device()) as cs:
         ms = timed(lambda: _pairwise(tA, tB, c.iou2dr, out), args.steps, args.warmup, barrier)
         l1 = c.launch_count()
+        keep_output(args, "iou_f64" if f64 else "iou", out)
         cs.hold(lambda: _pairwise(tA, tB, c.iou2dr, out))
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -688,6 +743,7 @@ def bench_dist3d(args, rank, world, barrier):
     with ClockSampler(torch.cuda.current_device()) as cs:
         ms = timed(step, args.steps, args.warmup, barrier)
         l1 = c.launch_count()
+        keep_output(args, "dist3d", out)
         cs.hold(step)
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -738,6 +794,7 @@ def bench_crop(args, rank, world, barrier):
     with ClockSampler(torch.cuda.current_device()) as cs:
         ms = timed(step, args.steps, args.warmup, barrier)
         l1 = c.launch_count()
+        keep_output(args, "crop_mask", mask)
         cs.hold(step)
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -783,13 +840,20 @@ def bench_scatter(args, rank, world, barrier):
 
     def step():
         plan = ScatterPlan(n, 2, fm.shape[0], _dims(fm.shape), fm.device)   # what AlignedScatter does: the backward reuses the forward's binning
-        fwd(plan)
+        out = fwd(plan)
         aligned_scatter_backward_cuda(coords, grad, AlignType.LINEAR, image_grad, plan)   # accumulates in place (the caller zeroes once, d3d/point/__init__.py:32)
+        return out
     anchor = float(fwd().double().sum().item())
+    last = [] if args.dump_outputs else None
     l0 = c.launch_count()
     with ClockSampler(torch.cuda.current_device()) as cs:
-        ms = timed_flushed(step, args.steps, args.warmup, barrier)
+        # when dumping, the map gradient is zeroed ahead of the last step (before its L2 flush) so that it holds that step's backward alone;
+        # the backward reduce-adds into the map, so it is equal from run to run up to fp32 rounding
+        ms = timed_flushed(step, args.steps, args.warmup, barrier, last, image_grad.zero_ if args.dump_outputs else None)
         l1 = c.launch_count()
+        if last:
+            keep_output(args, "scatter_forward", last.pop())
+            keep_output(args, "scatter_image_grad", image_grad)
         ms_fwd = timed_flushed(fwd, args.steps, 1, barrier)
         cs.hold(step)
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
@@ -838,10 +902,13 @@ def bench_nms(args, rank, world, barrier):
     tP, ts = torch.from_numpy(P).cuda(), torch.from_numpy(s).cuda()
     keep = box2d_nms(tP, ts, "rbox", iou_threshold=0.5)
     kept = int(keep.sum().item())
+    last = [] if args.dump_outputs else None
     l0 = c.launch_count()
     with ClockSampler(torch.cuda.current_device()) as cs:
-        ms = timed_flushed(lambda: box2d_nms(tP, ts, "rbox", iou_threshold=0.5), args.steps, args.warmup, barrier)
+        ms = timed_flushed(lambda: box2d_nms(tP, ts, "rbox", iou_threshold=0.5), args.steps, args.warmup, barrier, last)
         l1 = c.launch_count()
+        if last:
+            keep_output(args, "nms_keep", last.pop())
         cs.hold(lambda: box2d_nms(tP, ts, "rbox", iou_threshold=0.5))
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -917,6 +984,9 @@ def bench_c5(args, rank, world, barrier):
     with ClockSampler(torch.cuda.current_device()) as cs:
         ms = timed(step, args.steps, args.warmup, barrier)
         l1 = c.launch_count()
+        if nf:
+            keep_voxel_outputs(args, "c5_voxel", state["vox"])
+            keep_output(args, "c5_keep", state["keep"])
         cs.hold(step)
     launches = (l1 - l0) // (args.steps + args.warmup) * args.steps
     ms = max_over_ranks(ms, world)
@@ -1019,12 +1089,20 @@ def main():
     ap.add_argument("--iou-e2e-rows", type=int, default=8192)
     ap.add_argument("--nms-n", type=int, default=50_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float32 or float64; larger outputs as a fixed, seeded sample; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
 
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
+    if rank != 0:
+        args.dump_outputs = None
     local = int(os.environ.get("LOCAL_RANK", "0"))
     ops = ["voxel", "iou", "nms", "iou_f64", "c5", "scatter", "dist3d", "crop"] if args.op == "all" else [args.op]
 
@@ -1092,6 +1170,8 @@ def main():
             line["c5_weak_frames_per_s"] = res["c5"]["weak"]["value"]
         if len(ops) > 1:
             line["ops"] = {op: res[op] for op in ops[1:]}
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

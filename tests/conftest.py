@@ -1,3 +1,4 @@
+import hashlib
 import os
 import sys
 
@@ -66,3 +67,46 @@ def soft_inputs(n, gen):
     if gen == "boxes":
         return gen_boxes(rng, n), rng.random(n)
     return proposals(rng, n, max(n // 25, 1))
+
+
+# inputs of the comparisons with the reference's own code in test_oracle_pinned.py; tests/golden/make_golden.py write_live_ref
+# stores the outputs on them in live_ref.npz
+LIVE_VOXEL = ([0, 70.4, -40, 40, -3, 1], [352, 400, 40], dict(max_points=3, max_points_filter="trim", max_voxels=900, max_voxels_filter="trim"))
+
+
+def live_iou_nms_voxel_inputs():
+    rng = np.random.default_rng(11)
+    A, B = gen_boxes(rng, 300), gen_boxes(rng, 200)
+    s = rng.random(300)
+    return A, B, s, lidar(rng, 4000)
+
+
+def live_dist3d_inputs():
+    rng = np.random.default_rng(8)
+    mk = lambda n: np.concatenate([(rng.random((n, 2)) - .5) * 10, rng.normal(0, 0.5, (n, 1)), rng.random((n, 3)) * 4 + .3,  # noqa: E731
+                                   (rng.random((n, 1)) - .5) * 10], 1).astype(np.float32)
+    a, b = mk(150), mk(120)
+    return a, b, ((rng.random((200, 3)) - .5) * 8).astype(np.float32)
+
+
+def live_pdist_inputs():
+    rng = np.random.default_rng(3)
+    pts, bx = (rng.random((2000, 2)) - .5) * 14, gen_boxes(rng, 50)
+    p3, b3 = (rng.random((500, 3)) - .5) * 10, np.concatenate([gen_boxes(rng, 20)[:, :2], rng.random((20, 1)), rng.random((20, 3)) * 4 + .2, rng.random((20, 1)) * 6], 1)
+    return pts, bx, p3, b3
+
+
+def assert_pinned(g, name, a):
+    """`a` equals golden entry `name` bit for bit: the stored array, or for a large one (make_golden.py pin) the SHA-256 of its bytes,
+    after a stored sample of its values that shows where they differ"""
+    a = np.ascontiguousarray(a)
+    if name in g.files:
+        exp = g[name]
+        assert a.dtype == exp.dtype and a.shape == exp.shape and np.array_equal(a, exp), name
+        return
+    idx, val = g[name + ".idx"], g[name + ".val"]
+    assert a.dtype == val.dtype and a.shape == tuple(g[name + ".shape"]), (name, a.dtype, a.shape)
+    got = a.reshape(-1)[idx]
+    bad = np.flatnonzero(got != val)
+    assert not len(bad), (name, idx[bad[:5]], got[bad[:5]], val[bad[:5]])
+    assert hashlib.sha256(a.tobytes()).hexdigest() == str(g[name + ".sha256"]), name

@@ -5,6 +5,7 @@ Run in the authoring container, where /root/reference exists:
 The fixtures are small on purpose (the whole directory stays < 2 MB) and are what pins the C oracle
 and the CUDA path on machines where the reference cannot be built (the GPU box has no /root/reference).
 """
+import hashlib
 import os
 import shutil
 import sys
@@ -12,11 +13,12 @@ import sys
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+OUT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(OUT))
+from oracle import build_ref  # noqa: E402
 from oracle import ref as R  # noqa: E402
 from oracle import oracle as O  # noqa: E402
-
-OUT = os.path.dirname(os.path.abspath(__file__))
 PI = np.pi
 
 
@@ -140,6 +142,41 @@ def write_dist3d():
     b[:5] = a[:5]                      # identical boxes
     b[5, 2] += 50                      # no z overlap
     np.savez_compressed(os.path.join(OUT, "dist3d.npz"), src=a, dst=b, riou=R.box3d_iou_distance(a, b, "riou"), iou=R.box3d_iou_distance(a, b, "iou"))
+
+
+def pin(out, name, a, sample=1024):
+    """store a large array for conftest.assert_pinned: the SHA-256 of its bytes, its shape and its values at a fixed sample of positions"""
+    a = np.ascontiguousarray(a)
+    idx = np.sort(np.random.default_rng(0).choice(a.size, min(sample, a.size), replace=False))
+    out[name + ".sha256"] = np.array(hashlib.sha256(a.tobytes()).hexdigest())
+    out[name + ".shape"] = np.array(a.shape, np.int64)
+    out[name + ".idx"], out[name + ".val"] = idx, a.reshape(-1)[idx]
+
+
+def write_live_ref():
+    """outputs on the inputs of the comparisons of tests/test_oracle_pinned.py with the reference's own code (conftest live_*_inputs):
+    rotated / axis-aligned IoU, NMS and voxelization (box_impl, voxel_impl), evaluator distances and box3dr_pdist (dgal_wrap.h),
+    pdist2dr_forward (box_impl).  They come from the reference where oracle/_ref is built; elsewhere from the oracle, which then pins the
+    oracle on these inputs to the values it had when the file was written.  `source` records which of the two wrote the file."""
+    from conftest import LIVE_VOXEL, live_dist3d_inputs, live_iou_nms_voxel_inputs, live_pdist_inputs
+    ref = R.available() and os.path.exists(build_ref.WRAP_SO)
+    out = dict(source=np.array("reference" if ref else "oracle"))
+    A, B, s, pts = live_iou_nms_voxel_inputs()
+    pin(out, "rbox", R.box2d_iou(A, B, "rbox") if ref else O.iou2dr(A, B))
+    pin(out, "box", R.box2d_iou(A, B, "box") if ref else O.iou2d(A, B))
+    out["nms_keep"] = (R.box2d_nms if ref else O.box2d_nms)(A, s, "rbox", iou_threshold=0.4, score_threshold=0.1)
+    bounds, shape, kw = LIVE_VOXEL
+    for k, v in (R if ref else O).VoxelGenerator(bounds, shape, **kw)(pts).items():
+        out["voxel." + k] = v
+    a, b, p3 = live_dist3d_inputs()
+    for metric in ("riou", "iou"):
+        out["dist3d." + metric] = (R if ref else O).box3d_iou_distance(a, b, metric)
+    out["box3dr_pdist"] = np.stack([R.box3dr_pdist_scalar(a[k], p3) if ref else O.box3dr_pdist(p3, a[k:k + 1])[0] for k in range(5)])
+    pts, bx, _, _ = live_pdist_inputs()
+    d, ie = R.pdist2dr(pts, bx) if ref else O.pdist2dr(pts, bx, return_iedge=True)
+    pin(out, "pdist2dr", d)
+    out["pdist2dr.iedge"] = ie
+    np.savez_compressed(os.path.join(OUT, "live_ref.npz"), **out)
 
 
 def main():
@@ -286,6 +323,7 @@ def main():
                 sc[f"{tag}.d{dim}.{meth}"] = R.aligned_scatter_forward(crd, img, meth)
     np.savez_compressed(os.path.join(OUT, "scatter.npz"), **sc)
     write_crop()
+    write_live_ref()
     tot = sum(os.path.getsize(os.path.join(OUT, f)) for f in os.listdir(OUT) if f.endswith(".npz"))
     print("golden fixtures written, total bytes:", tot)
 

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -82,5 +83,5 @@ def test_import_fails_loudly_without_extension(tmp_path):
     import shutil
     dst = tmp_path / "d3d_b200"
     shutil.copytree(os.path.join(ROOT, "d3d_b200"), dst, ignore=shutil.ignore_patterns("*.so", "*.o", "csrc", "__pycache__"))
-    r = subprocess.run(["python", "-c", "import d3d_b200"], cwd=tmp_path, capture_output=True, text=True)
+    r = subprocess.run([sys.executable, "-c", "import d3d_b200"], cwd=tmp_path, capture_output=True, text=True)
     assert r.returncode != 0 and "ImportError" in r.stderr
