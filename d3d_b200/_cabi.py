@@ -74,6 +74,9 @@ nms2d = {F32: _sig("d3d_nms2d_f32", C.c_int, _nms_sig), F64: _sig("d3d_nms2d_f64
 nms_batch_workspace_bytes = _sig("d3d_nms2d_batch_workspace_bytes", _sz, [_i64, _i64, _i64, C.c_int])
 _nmsb_sig = [_vp, _vp, _i64, _vp, _i64, _i64, C.c_int, C.c_int, _f, _f, _vp, _vp, _sz, _vp]
 nms2d_batch = {F32: _sig("d3d_nms2d_batch_f32", C.c_int, _nmsb_sig), F64: _sig("d3d_nms2d_batch_f64", C.c_int, _nmsb_sig)}
+nms_batch_soft_workspace_bytes = _sig("d3d_nms2d_batch_soft_workspace_bytes", _sz, [_i64, _i64, _i64, C.c_int])
+_nmsbs_sig = [_vp, _vp, _i64, _vp, _i64, _i64, C.c_int, C.c_int, _f, _f, _f, _vp, _vp, _sz, _vp]
+nms2d_batch_soft = {F32: _sig("d3d_nms2d_batch_soft_f32", C.c_int, _nmsbs_sig), F64: _sig("d3d_nms2d_batch_soft_f64", C.c_int, _nmsbs_sig)}
 voxelize_workspace_bytes = _sig("d3d_voxelize_workspace_bytes", _sz, [_i64, _i64, _i64])
 voxelize_sparse = _sig("d3d_voxelize_sparse_f32", C.c_int,
                        [_vp, _i64, _i32, _vp, _i64, C.POINTER(VoxelParams), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp])

@@ -188,15 +188,19 @@ def box2d_iou(boxes1, boxes2, method="box", precise=True):
     return result
 
 
-def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold=0, score_threshold=0, precise=True, offsets_dev=None):
+def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold=0, score_threshold=0, precise=True, offsets_dev=None,
+                    supression_method="hard", supression_param=0):
     '''
-    Hard NMS on a batch of frames in one launch sequence (the reference has no batch form; per frame the result equals
-    :func:`box2d_nms`).  Two call forms: lists of per-frame ``boxes`` / ``scores`` (returns a list of keep masks), or the frames
-    packed back to back as ``boxes`` [total, 5] / ``scores`` [total] with ``offsets`` (int64 [nframes + 1], CPU tensor) (returns one
-    keep mask bool[total]).  Frames of more than 8192 boxes fall back to one :func:`box2d_nms` call per frame.
+    NMS on a batch of frames in one launch sequence (the reference has no batch form; per frame the result equals
+    :func:`box2d_nms` with the same arguments, bit for bit).  Two call forms: lists of per-frame ``boxes`` / ``scores`` (returns a list
+    of keep masks), or the frames packed back to back as ``boxes`` [total, 5] / ``scores`` [total] with ``offsets`` (int64
+    [nframes + 1], CPU tensor) (returns one keep mask bool[total]).  Frames of more than 8192 boxes fall back to one :func:`box2d_nms`
+    call per frame.
 
     :param iou_method: 'box' - axis-aligned box, 'rbox' - rotated box
     :param offsets_dev: the same offsets already on the device (saves the copy)
+    :param supression_method: 'hard', or 'linear' / 'gaussian' (soft-NMS: one CTA walks each frame, the frames run side by side)
+    :param supression_param: parameter of the soft decay, as in :func:`box2d_nms`
     '''
     as_list = isinstance(boxes, (list, tuple))
     if as_list:
@@ -226,6 +230,7 @@ def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold
     iou_type = getattr(IouType, iou_method.upper())
     if iou_type not in (IouType.BOX, IouType.RBOX):
         raise ValueError("Unsupported iou type!")
+    sup_type = getattr(SupressionType, supression_method.upper())
     b, s_ = _c.to_device(boxes), _c.to_device(scores)
     if precise:
         b, s_ = b.to(torch.float64), s_.to(torch.float64)
@@ -239,14 +244,21 @@ def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold
         for f in range(nframes):
             lo, hi = int(offsets[f]), int(offsets[f + 1])
             if hi > lo:
-                suppressed[lo:hi] = nms2d_cuda(b[lo:hi], s_[lo:hi], iou_type, SupressionType.HARD, iou_threshold, score_threshold, 0).view(torch.uint8)
+                suppressed[lo:hi] = nms2d_cuda(b[lo:hi], s_[lo:hi], iou_type, sup_type, iou_threshold, score_threshold, supression_param).view(torch.uint8)
     elif total > 0:
         code = _c.dtype_code(b.dtype)
         od = offsets.to(b.device, non_blocking=True) if offsets_dev is None else offsets_dev
-        ws = _c.workspace(_c.nms_batch_workspace_bytes(total, nframes, max_frame, code), b.device)
-        with torch.cuda.device(b.device):
-            st = _c.nms2d_batch[code](_c.ptr(b), _c.ptr(s_), total, _c.ptr(od), nframes, max_frame, int(iou_type), int(SupressionType.HARD),
-                                      float(iou_threshold), float(score_threshold), _c.ptr(suppressed), _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        if sup_type == SupressionType.HARD:
+            ws = _c.workspace(_c.nms_batch_workspace_bytes(total, nframes, max_frame, code), b.device)
+            with torch.cuda.device(b.device):
+                st = _c.nms2d_batch[code](_c.ptr(b), _c.ptr(s_), total, _c.ptr(od), nframes, max_frame, int(iou_type), int(SupressionType.HARD),
+                                          float(iou_threshold), float(score_threshold), _c.ptr(suppressed), _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        else:
+            ws = _c.workspace(_c.nms_batch_soft_workspace_bytes(total, nframes, max_frame, code), b.device)
+            with torch.cuda.device(b.device):
+                st = _c.nms2d_batch_soft[code](_c.ptr(b), _c.ptr(s_), total, _c.ptr(od), nframes, max_frame, int(iou_type), int(sup_type),
+                                               float(iou_threshold), float(score_threshold), float(supression_param), _c.ptr(suppressed),
+                                               _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box2d_nms_batch")
     keep = ~suppressed.view(torch.bool)
     if odev.type != "cuda":

@@ -975,6 +975,78 @@ __device__ __forceinline__ bool soft_before(const SoftState<T> &S, const uint32_
     return pos[a] < pos[b];
 }
 
+// re-sort of the range [_i + 1, Sp) after the decay of step _i (the reference's insertion sort, nms.cpp:74-94), by all NT threads of
+// the CTA.  *s_cnt must be 0 on entry.  Boxes whose score changed are marked in S.mk; positions >= E count as changed.
+template <typename T, uint32_t NT>
+__device__ __forceinline__ void soft_resort(const SoftState<T> &S, uint32_t *pos, uint32_t _i, uint32_t Sp, uint32_t &E, uint32_t *s_red,
+                                            uint32_t *s_cnt, uint32_t *s_dirty, uint32_t *Bp)
+{
+    const uint32_t tid = threadIdx.x;
+    if (Sp <= _i + 2) return;   // zero or one box in the range: nothing to sort (uniform); marks stay for a later sort
+    const uint32_t r0 = _i + 1, m = Sp - r0;   // range [r0, Sp)
+    // split the range into unchanged boxes (still mutually sorted) and the rest
+    const uint32_t per = (m + NT - 1) / NT, q0 = r0 + tid * per, q1 = min(q0 + per, Sp);
+    uint32_t na = 0;
+    for (uint32_t q = q0; q < q1; q++) { const uint32_t j = S.ord[q]; if (!(S.mk[j] || q >= E)) na++; }
+    // exclusive prefix of na over the threads
+    uint32_t inc = na;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, inc, d); if ((tid & 31u) >= (unsigned)d) inc += x; }
+    if ((tid & 31u) == 31u) s_red[tid >> 5] = inc;
+    __syncthreads();
+    if (tid < 32) {
+        uint32_t v = tid < NT / 32 ? s_red[tid] : 0u, iv = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, iv, d); if (tid >= (unsigned)d) iv += x; }
+        if (tid < NT / 32) s_red[tid] = iv - v;
+        if (tid == 31) *s_dirty = iv;   // unchanged boxes in the range
+    }
+    __syncthreads();
+    uint32_t abase = s_red[tid >> 5] + inc - na;
+    const uint32_t nA = *s_dirty, nB = m - nA;
+    if (nB == 0) return;        // nothing changed inside the range: it is still sorted
+    const bool brute = nB > (uint32_t)SOFT_BCAP;
+    for (uint32_t q = q0; q < q1; q++) {
+        const uint32_t j = S.ord[q];
+        if (!(S.mk[j] || q >= E)) S.tmp[abase++] = j;
+        else if (!brute) Bp[atomicAdd(s_cnt, 1u)] = j;
+    }
+    __syncthreads();
+    if (!brute) {
+        // unchanged box a at compact index ia: new position = r0 + ia + (changed boxes before it)
+        for (uint32_t ia = tid; ia < nA; ia += NT) {
+            const uint32_t a = S.tmp[ia];
+            uint32_t c = 0;
+            for (uint32_t k = 0; k < nB; k++) c += soft_before<T>(S, pos, Bp[k], a) ? 1u : 0u;
+            S.ord[r0 + ia + c] = a;
+        }
+        // changed box b: unchanged boxes before it (binary search: they are sorted) + changed boxes before it
+        for (uint32_t kb = tid; kb < nB; kb += NT) {
+            const uint32_t b = Bp[kb];
+            uint32_t lo = 0, hi = nA;
+            while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (soft_before<T>(S, pos, S.tmp[mid], b)) lo = mid + 1; else hi = mid; }
+            uint32_t c = lo;
+            for (uint32_t k = 0; k < nB; k++) c += (k != kb && soft_before<T>(S, pos, Bp[k], b)) ? 1u : 0u;
+            S.ord[r0 + c] = b;
+        }
+    } else {
+        // many changed boxes: count all pairs (tmp receives a copy of the range first)
+        __syncthreads();
+        for (uint32_t q = r0 + tid; q < Sp; q += NT) S.tmp[q - r0] = S.ord[q];
+        __syncthreads();
+        for (uint32_t x = tid; x < m; x += NT) {
+            const uint32_t a = S.tmp[x];
+            uint32_t c = 0;
+            for (uint32_t y = 0; y < m; y++) c += (y != x && soft_before<T>(S, pos, S.tmp[y], a)) ? 1u : 0u;
+            S.ord[r0 + c] = a;
+        }
+    }
+    __syncthreads();
+    for (uint32_t q = r0 + tid; q < Sp; q += NT) { const uint32_t j = S.ord[q]; pos[j] = q; S.mk[j] = 0; }
+    E = Sp;
+    __syncthreads();
+}
+
 template <typename T, bool AABB>
 __global__ void __launch_bounds__(SOFT_THREADS) nms_soft_kernel(const BoxRec<T> *__restrict__ recs, const AABBRec<T> *__restrict__ arecs, const T *__restrict__ scores,
                                                                 const uint32_t *__restrict__ order, int64_t n64, T thr, T sthr, T param, int sup_type,
@@ -1017,70 +1089,7 @@ __global__ void __launch_bounds__(SOFT_THREADS) nms_soft_kernel(const BoxRec<T> 
             if ((tid & 31u) == 0) atomicMax(&s_S, smax);
         }
         __syncthreads();
-        const uint32_t Sp = s_S;
-        if (Sp <= _i + 2) continue;   // zero or one box in the range: nothing to sort (uniform); marks stay for a later sort
-        const uint32_t r0 = _i + 1, m = Sp - r0;   // range [r0, Sp)
-        // split the range into unchanged boxes (still mutually sorted) and the rest
-        const uint32_t per = (m + NT - 1) / NT, q0 = r0 + tid * per, q1 = min(q0 + per, Sp);
-        uint32_t na = 0;
-        for (uint32_t q = q0; q < q1; q++) { const uint32_t j = S.ord[q]; if (!(S.mk[j] || q >= E)) na++; }
-        // exclusive prefix of na over the threads
-        uint32_t inc = na;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, inc, d); if ((tid & 31u) >= (unsigned)d) inc += x; }
-        if ((tid & 31u) == 31u) s_red[tid >> 5] = inc;
-        __syncthreads();
-        if (tid < 32) {
-            uint32_t v = s_red[tid], iv = v;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, iv, d); if (tid >= (unsigned)d) iv += x; }
-            s_red[tid] = iv - v;
-            if (tid == 31) s_dirty = iv;   // unchanged boxes in the range
-        }
-        __syncthreads();
-        uint32_t abase = s_red[tid >> 5] + inc - na;
-        const uint32_t nA = s_dirty, nB = m - nA;
-        if (nB == 0) continue;        // nothing changed inside the range: it is still sorted
-        const bool brute = nB > (uint32_t)SOFT_BCAP;
-        for (uint32_t q = q0; q < q1; q++) {
-            const uint32_t j = S.ord[q];
-            if (!(S.mk[j] || q >= E)) S.tmp[abase++] = j;
-            else if (!brute) Bp[atomicAdd(&s_cnt, 1u)] = j;
-        }
-        __syncthreads();
-        if (!brute) {
-            // unchanged box a at compact index ia: new position = r0 + ia + (changed boxes before it)
-            for (uint32_t ia = tid; ia < nA; ia += NT) {
-                const uint32_t a = S.tmp[ia];
-                uint32_t c = 0;
-                for (uint32_t k = 0; k < nB; k++) c += soft_before<T>(S, pos, Bp[k], a) ? 1u : 0u;
-                S.ord[r0 + ia + c] = a;
-            }
-            // changed box b: unchanged boxes before it (binary search: they are sorted) + changed boxes before it
-            for (uint32_t kb = tid; kb < nB; kb += NT) {
-                const uint32_t b = Bp[kb];
-                uint32_t lo = 0, hi = nA;
-                while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (soft_before<T>(S, pos, S.tmp[mid], b)) lo = mid + 1; else hi = mid; }
-                uint32_t c = lo;
-                for (uint32_t k = 0; k < nB; k++) c += (k != kb && soft_before<T>(S, pos, Bp[k], b)) ? 1u : 0u;
-                S.ord[r0 + c] = b;
-            }
-        } else {
-            // many changed boxes: count all pairs (tmp receives a copy of the range first)
-            __syncthreads();
-            for (uint32_t q = r0 + tid; q < Sp; q += NT) S.tmp[q - r0] = S.ord[q];
-            __syncthreads();
-            for (uint32_t x = tid; x < m; x += NT) {
-                const uint32_t a = S.tmp[x];
-                uint32_t c = 0;
-                for (uint32_t y = 0; y < m; y++) c += (y != x && soft_before<T>(S, pos, S.tmp[y], a)) ? 1u : 0u;
-                S.ord[r0 + c] = a;
-            }
-        }
-        __syncthreads();
-        for (uint32_t q = r0 + tid; q < Sp; q += NT) { const uint32_t j = S.ord[q]; pos[j] = q; S.mk[j] = 0; }
-        E = Sp;
-        __syncthreads();
+        soft_resort<T, SOFT_THREADS>(S, pos, _i, s_S, E, s_red, &s_cnt, &s_dirty, Bp);
     }
     __syncthreads();
     for (uint32_t p = tid; p < n; p += NT) suppressed[order[p]] = S.sup[p];
@@ -1703,6 +1712,286 @@ nmsb_fix_kernel(const uint32_t *__restrict__ edges_all, const uint32_t *__restri
     for (uint32_t j = tid; j < n; j += 1024u) suppressed[b + order[j]] = state[j] == NMS_KEPT ? 0 : 1;
 }
 
+// ------------------------------------------------------------------------------------------------ batched soft-NMS
+// LINEAR / GAUSSIAN suppression of a batch of frames: the walk of nms_soft_kernel, one CTA per frame, its whole state in shared memory.
+// A kept box only decays boxes whose IoU with it exceeds the threshold; for a threshold >= 0 those are a few spatial neighbours, so the
+// frame's candidate pairs are found once, before the walk (nmsbs_cand_kernel), and every step clips the kept box against its own
+// candidates instead of against every box behind it.  The lists hold candidates, not IoU values: the re-sorts decide which box of a pair
+// is visited first, and the clip iou(visited, later) is the one the reference evaluates.
+constexpr int NMSBS_PAIRS_PER_BOX = 32;   // candidate pairs per frame = 32 x max_frame_boxes; more -> that frame decays over all boxes
+constexpr int NMSBS_THREADS = 512;    // 1024 threads leave 64 registers: the fp64 clip spills
+
+// one CTA per (64-box row block, frame): every pair p < q of sorted positions that may have IoU > threshold (threshold >= 0) goes to the
+// frame's pair list as p | q << 16.  The tests only drop pairs whose IoU cannot exceed the threshold, whichever box comes first:
+// rbox: bounding circles meet (single precision, widened by what the converted centres may be off by; a record that is not finite is a
+// candidate of every box); box: the closed AABBs overlap (a NaN coordinate fails every comparison and keeps the pair).
+// pcount[f] counts every pair found, also those past the capacity: pcount[f] > pcap flags the frame's list as incomplete.
+template <typename T, bool AABB>
+__global__ void __launch_bounds__(256) nmsbs_cand_kernel(const BoxRec<T> *__restrict__ recs_all, const AABBRec<T> *__restrict__ arecs_all,
+                                                         const int64_t *__restrict__ offs, int64_t stride, uint32_t *__restrict__ pairs_all,
+                                                         uint32_t *__restrict__ pcount, uint32_t pcap)
+{
+    const int64_t f = blockIdx.y, rb = blockIdx.x;
+    const int64_t n = min(offs[f + 1] - offs[f], stride);
+    if (rb * NMS_TILE >= n) return;
+    const int64_t nb = (n + NMS_TILE - 1) / NMS_TILE;
+    __shared__ float4 rowc[NMS_TILE], colc[NMS_TILE];         // rbox: centre, widened radius
+    __shared__ AABBRec<T> rowa[NMS_TILE], cola[NMS_TILE];     // box
+    __shared__ uint32_t hits[NMS_TILE * NMS_TILE];
+    __shared__ uint32_t s_n, s_base;
+    uint32_t *pairs = pairs_all + (size_t)f * pcap;
+    const unsigned tid = threadIdx.x;
+    auto stage = [&](int64_t blk, float4 *c, AABBRec<T> *a) {
+        const int64_t p = blk * NMS_TILE + tid;
+        if (AABB) a[tid] = arecs_all[f * stride + p];
+        else {
+            const BoxRec<T> r = recs_all[f * stride + p];
+            const float fx = (float)r.cx, fy = (float)r.cy, fr = __double2float_ru((double)r.rho) + (fabsf(fx) + fabsf(fy)) * 2.4e-7f;
+            c[tid] = isfinite(fx) && isfinite(fy) && isfinite(fr) ? make_float4(fx, fy, fr, 0.f) : make_float4(0.f, 0.f, INFINITY, 0.f);
+        }
+    };
+    if (tid < NMS_TILE) stage(rb, rowc, rowa);
+    for (int64_t cb = rb + blockIdx.z; cb < nb; cb += gridDim.z) {
+        __syncthreads();   // the previous tile's readers are done with the columns and the hits
+        if (tid < NMS_TILE) stage(cb, colc, cola);
+        if (tid == 0) s_n = 0;
+        __syncthreads();
+        for (unsigned k = tid; k < NMS_TILE * NMS_TILE; k += 256) {
+            const unsigned rl = k >> 6, cl = k & 63u;
+            const int64_t p = rb * NMS_TILE + rl, q = cb * NMS_TILE + cl;
+            if (p >= q || q >= n) continue;
+            bool cand;
+            if (AABB) {
+                const AABBRec<T> &a = rowa[rl], &b = cola[cl];
+                cand = !(a.maxx < b.minx || b.maxx < a.minx || a.maxy < b.miny || b.maxy < a.miny);
+            } else {
+                const float4 a = rowc[rl], b = colc[cl];
+                const float dx = a.x - b.x, dy = a.y - b.y, rs = a.z + b.z;
+                cand = !(dx * dx + dy * dy > rs * rs * 1.00001f);
+            }
+            if (cand) hits[atomicAdd(&s_n, 1u)] = (uint32_t)p | ((uint32_t)q << 16);
+        }
+        __syncthreads();
+        const uint32_t nh = s_n;
+        if (nh == 0) continue;   // (uniform)
+        if (tid == 0) s_base = atomicAdd(pcount + f, nh);
+        __syncthreads();
+        const uint32_t base = s_base;
+        for (uint32_t h = tid; h < nh; h += 256) if (base + h < pcap) pairs[base + h] = hits[h];
+    }
+}
+
+// one CTA per frame: the walk of nms_soft_kernel over the frame's score order (nmsb_sort_kernel), state in dynamic shared memory.
+// Prologue: the frame's pair list becomes a symmetric adjacency (CSR: nboff / nblst, sorted positions) when it is complete.
+// Step _i (kept box i): the decay runs over i's candidates whose position is behind _i -- the pairs left out have IoU <= threshold and
+// the reference's decay does not touch them.  The end S of the re-sort range (last position holding a suppressed box) is then a running
+// value: suppressed boxes stay behind S (the re-sort of [_i + 1, S) keeps them in the range, positions >= S are not moved), so S only
+// grows, by the positions of the boxes suppressed at this step.  A decay can lift a score back over the threshold (negative scores):
+// then S is found again by a scan of all positions behind _i.  Frames without a complete list (negative threshold: every pair decays;
+// an overflowed list) take the decay of nms_soft_kernel over every position behind _i.  The re-sort is nms_soft_kernel's.
+template <typename T, bool AABB>
+__global__ void __launch_bounds__(NMSBS_THREADS, 1)
+nmsbs_walk_kernel(const BoxRec<T> *__restrict__ recs_all, const AABBRec<T> *__restrict__ arecs_all, const T *__restrict__ scores,
+                  const int64_t *__restrict__ offs, int64_t stride, const uint32_t *__restrict__ order_all, const uint32_t *__restrict__ pairs_all,
+                  const uint32_t *__restrict__ pcount, uint32_t pcap, uint32_t *__restrict__ nboff_all, uint16_t *__restrict__ nblst_all,
+                  T thr, T sthr, T param, int sup_type, uint8_t *__restrict__ suppressed)
+{
+    extern __shared__ __align__(16) unsigned char sw_dyn[];   // sc T[stride] | ord, tmp, pos u32[stride] | sup, mk u8[stride]
+    __shared__ uint32_t s_red[32], s_cnt, s_S, s_dirty, s_rev;
+    __shared__ uint32_t Bp[SOFT_BCAP];
+    constexpr uint32_t NT = NMSBS_THREADS;
+    const int64_t f = blockIdx.x, b = offs[f];
+    const uint32_t n = (uint32_t)min(offs[f + 1] - b, stride), tid = threadIdx.x, lane = tid & 31u;
+    if (n == 0) return;
+    SoftState<T> S;
+    S.sc = reinterpret_cast<T *>(sw_dyn);
+    S.ord = reinterpret_cast<uint32_t *>(S.sc + stride); S.tmp = S.ord + stride;
+    uint32_t *pos = S.tmp + stride;
+    S.sup = reinterpret_cast<uint8_t *>(pos + stride); S.mk = S.sup + stride;
+    const uint32_t *order = order_all + f * stride;
+    const BoxRec<T> *recs = recs_all ? recs_all + f * stride : nullptr;
+    const AABBRec<T> *arecs = arecs_all ? arecs_all + f * stride : nullptr;
+    const uint32_t np = pairs_all ? pcount[f] : 0u;
+    const bool nbr = pairs_all && np <= pcap;   // (uniform)
+    uint32_t *nboff = nboff_all + f * (stride + 1);
+    uint16_t *nbl = nblst_all + (size_t)f * 2 * pcap;
+    if (nbr) {
+        const uint32_t *pairs = pairs_all + (size_t)f * pcap;
+        uint32_t *cnt = reinterpret_cast<uint32_t *>(S.sc);   // degrees, then fill cursors (the scores take this memory afterwards)
+        for (uint32_t p = tid; p < n; p += NT) cnt[p] = 0;
+        __syncthreads();
+        for (uint32_t e = tid; e < np; e += NT) { const uint32_t pq = pairs[e]; atomicAdd(&cnt[pq & 0xffffu], 1u); atomicAdd(&cnt[pq >> 16], 1u); }
+        __syncthreads();
+        // exclusive prefix of the degrees: a thread owns the boxes [tid * per, tid * per + per)
+        const uint32_t per = (n + NT - 1) / NT;
+        uint32_t mine = 0;
+        for (uint32_t k = 0; k < per; k++) { const uint32_t j = tid * per + k; if (j < n) mine += cnt[j]; }
+        uint32_t inc = mine;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, inc, d); if (lane >= (unsigned)d) inc += x; }
+        if (lane == 31u) s_red[tid >> 5] = inc;
+        __syncthreads();
+        if (tid < 32) {
+            const uint32_t x = tid < NT / 32 ? s_red[tid] : 0u;
+            uint32_t y = x;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { const uint32_t z = __shfl_up_sync(0xffffffffu, y, d); if (tid >= (unsigned)d) y += z; }
+            if (tid < NT / 32) s_red[tid] = y - x;
+        }
+        __syncthreads();
+        uint32_t run = s_red[tid >> 5] + inc - mine;
+        for (uint32_t k = 0; k < per; k++) { const uint32_t j = tid * per + k; if (j < n) { nboff[j] = run; run += cnt[j]; } }
+        if (tid == NT - 1) nboff[n] = run;   // the last thread's range ends at n (or it owns no box: run = the total)
+        __syncthreads();
+        for (uint32_t e = tid; e < np; e += NT) {
+            const uint32_t pq = pairs[e], p = pq & 0xffffu, q = pq >> 16;
+            nbl[nboff[p] + atomicSub(&cnt[p], 1u) - 1u] = (uint16_t)q;
+            nbl[nboff[q] + atomicSub(&cnt[q], 1u) - 1u] = (uint16_t)p;
+        }
+        __syncthreads();
+    }
+    if (tid == 0) s_S = 0;
+    __syncthreads();
+    uint32_t smax = 0;
+    for (uint32_t p = tid; p < n; p += NT) {
+        const T v = scores[b + order[p]];
+        S.sc[p] = v; S.ord[p] = p; pos[p] = p; S.mk[p] = 0;
+        S.sup[p] = v > sthr ? 0 : 1;   // reference CUDA rule (nms_cuda.cu:223), as for hard NMS
+        if (S.sup[p]) smax = p;
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) smax = max(smax, __shfl_xor_sync(0xffffffffu, smax, d));
+    if (lane == 0) atomicMax(&s_S, smax);
+    __syncthreads();
+    uint32_t Srun = s_S;   // last position holding a suppressed box (0: none)
+    uint32_t E = n;        // positions (_i, E) that are not marked are mutually sorted
+    for (uint32_t _i = 0; _i < n; _i++) {
+        __syncthreads();       // the previous step's reads of the shared words are done
+        const uint32_t i = S.ord[_i];
+        if (S.sup[i]) break;   // nms.cpp:37-42: everything behind a suppressed box is suppressed
+        if (tid == 0) { s_S = _i; s_cnt = 0; s_dirty = 0; s_rev = 0; }
+        __syncthreads();
+        // decay: i's candidates behind _i, or every position behind _i
+        {
+            BoxRec<T> A; AABBRec<T> AA;
+            if (AABB) AA = arecs[i]; else A = recs[i];
+            const uint32_t k0 = nbr ? nboff[i] : _i + 1, k1 = nbr ? nboff[i + 1] : n;
+            uint32_t sm = _i, rev = 0;
+            for (uint32_t k = k0 + tid; k < k1; k += NT) {
+                uint32_t j, q;
+                if (nbr) { j = nbl[k]; q = pos[j]; if (q <= _i) continue; }
+                else { q = k; j = S.ord[q]; }
+                const T iou = AABB ? aabb_iou<T>(AA, arecs[j]) : rbox_iou<T>(A, recs[j]);
+                if (iou > thr) {
+                    const T coef = sup_type == D3D_SUP_LINEAR ? T(1) - pow(iou, param) : exp(-iou * iou / param);
+                    const T v = S.sc[j] * coef;
+                    const uint8_t was = S.sup[j];
+                    S.sc[j] = v; S.sup[j] = v < sthr ? 1 : 0; S.mk[j] = 1;
+                    if (was && !S.sup[j]) rev = 1;
+                }
+                if (S.sup[j]) sm = max(sm, q);
+            }
+#pragma unroll
+            for (int d = 16; d; d >>= 1) { sm = max(sm, __shfl_xor_sync(0xffffffffu, sm, d)); rev |= __shfl_xor_sync(0xffffffffu, rev, d); }
+            if (lane == 0) { atomicMax(&s_S, sm); if (rev) s_rev = 1; }
+        }
+        __syncthreads();
+        uint32_t Sp = s_S;
+        if (nbr) {
+            if (s_rev) {   // a suppressed box came back: the last suppressed position is found again (uniform)
+                uint32_t sm = _i;
+                for (uint32_t q = _i + 1 + tid; q < n; q += NT) if (S.sup[S.ord[q]]) sm = q;
+#pragma unroll
+                for (int d = 16; d; d >>= 1) sm = max(sm, __shfl_xor_sync(0xffffffffu, sm, d));
+                __syncthreads();   // every thread has read s_S
+                if (tid == 0) s_S = _i;
+                __syncthreads();
+                if (lane == 0) atomicMax(&s_S, sm);
+                __syncthreads();
+                Sp = s_S;
+            } else Sp = max(Sp, Srun);
+            Srun = Sp;
+        }
+        soft_resort<T, NT>(S, pos, _i, Sp, E, s_red, &s_cnt, &s_dirty, Bp);
+    }
+    __syncthreads();
+    for (uint32_t p = tid; p < n; p += NT) suppressed[b + order[p]] = S.sup[p];
+}
+
+template <typename T> static size_t nmsbs_ws_bytes(int64_t nframes, int64_t max_frame_boxes)
+{
+    if (nframes < 1) nframes = 1;
+    if (max_frame_boxes < 1) max_frame_boxes = 1;
+    const int64_t stride = cdiv(max_frame_boxes, NMS_TILE) * NMS_TILE;
+    const size_t rec = sizeof(BoxRec<T>) > sizeof(AABBRec<T>) ? sizeof(BoxRec<T>) : sizeof(AABBRec<T>), pcap = (size_t)stride * NMSBS_PAIRS_PER_BOX;
+    const size_t per = align_up((size_t)stride * 4) + align_up((size_t)stride * rec) + align_up((size_t)stride) +   // order, records, valid
+                       align_up(pcap * 4) + align_up((size_t)(stride + 1) * 4) + align_up(pcap * 2 * 2);            // pairs, CSR offsets and lists
+    return per * (size_t)nframes + align_up((size_t)nframes * 4) + align_up(64 * 4) + 4096;
+}
+
+template <typename T>
+static int nmsbs_impl(const T *boxes, const T *scores, int64_t total, const int64_t *offs, int64_t nframes, int64_t max_frame_boxes, int iou_type, int sup_type,
+                      float iou_thr, float score_thr, float sup_param, uint8_t *suppressed, void *ws, size_t ws_bytes, cudaStream_t st)
+{
+    if (total < 0 || nframes < 0) return D3D_ERR_INVALID_ARGUMENT;
+    if (iou_type != D3D_IOU_BOX && iou_type != D3D_IOU_RBOX) return D3D_ERR_INVALID_ARGUMENT;
+    if (sup_type != D3D_SUP_LINEAR && sup_type != D3D_SUP_GAUSSIAN) return D3D_ERR_INVALID_ARGUMENT;   // hard NMS: d3d_nms2d_batch_*
+    if (nframes == 0 || total == 0) return D3D_OK;
+    if (!boxes || !scores || !offs || !suppressed) return D3D_ERR_INVALID_ARGUMENT;
+    if (max_frame_boxes <= 0 || max_frame_boxes > total) max_frame_boxes = total;
+    if (max_frame_boxes > NMSB_MAX) return D3D_ERR_UNSUPPORTED;   // the walk state lives in shared memory: use d3d_nms2d_* per frame
+    if (nframes > 65535) return D3D_ERR_INVALID_ARGUMENT;
+    if (!ws || ws_bytes < nmsbs_ws_bytes<T>(nframes, max_frame_boxes)) return D3D_ERR_WORKSPACE;
+    const int64_t stride = cdiv(max_frame_boxes, NMS_TILE) * NMS_TILE, nwords = stride / 64;
+    const bool aabb = iou_type == D3D_IOU_BOX;
+    const uint32_t pcap = (uint32_t)(stride * NMSBS_PAIRS_PER_BOX);
+    Arena a(ws, ws_bytes);
+    uint32_t *order = a.take<uint32_t>((size_t)nframes * stride);
+    void *recs = a.take<char>((size_t)nframes * stride * (sizeof(BoxRec<T>) > sizeof(AABBRec<T>) ? sizeof(BoxRec<T>) : sizeof(AABBRec<T>)));
+    uint8_t *valid = a.take<uint8_t>((size_t)nframes * stride);
+    uint32_t *pairs = a.take<uint32_t>((size_t)nframes * pcap);
+    uint32_t *nboff = a.take<uint32_t>((size_t)nframes * (stride + 1));
+    uint16_t *nblst = a.take<uint16_t>((size_t)nframes * 2 * pcap);
+    uint32_t *pcount = a.take<uint32_t>(nframes);
+    uint32_t *fail = a.take<uint32_t>(64);   // [0] a frame was longer than max_frame_boxes (cut)
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    uint32_t npow = 64;
+    while (npow < (uint32_t)stride) npow <<= 1;
+    const size_t sort_smem = (size_t)npow * 12;
+    const T thr = (T)iou_thr;   // (T)(float), as d3d_nms2d_*
+    BoxRec<T> *br = aabb ? nullptr : (BoxRec<T> *)recs;
+    AABBRec<T> *ar = aabb ? (AABBRec<T> *)recs : nullptr;
+    D3D_CUDA_TRY(cudaMemsetAsync(fail, 0, 256, st));
+    if (aabb) {
+        if (sort_smem > 40 * 1024) D3D_CUDA_TRY(cudaFuncSetAttribute(nmsb_sort_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_smem));
+        nmsb_sort_kernel<T, true><<<(unsigned)nframes, NMSB_SORT_THREADS, sort_smem, st>>>(boxes, scores, offs, stride, score_thr, order, nullptr, ar, nullptr, valid, fail, nullptr);
+    } else {
+        if (sort_smem > 40 * 1024) D3D_CUDA_TRY(cudaFuncSetAttribute(nmsb_sort_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_smem));
+        nmsb_sort_kernel<T, false><<<(unsigned)nframes, NMSB_SORT_THREADS, sort_smem, st>>>(boxes, scores, offs, stride, score_thr, order, br, nullptr, nullptr, valid, fail, nullptr);
+    }
+    D3D_LAUNCHED();
+    // candidate pairs exist for a threshold >= 0 only (a negative one lets every pair decay: every frame walks over all positions)
+    const bool lists = thr >= T(0);
+    if (lists) {
+        D3D_CUDA_TRY(cudaMemsetAsync(pcount, 0, (size_t)nframes * 4, st));
+        if (aabb) nmsbs_cand_kernel<T, true><<<dim3((unsigned)nwords, (unsigned)nframes, 4), 256, 0, st>>>(nullptr, ar, offs, stride, pairs, pcount, pcap);
+        else nmsbs_cand_kernel<T, false><<<dim3((unsigned)nwords, (unsigned)nframes, 4), 256, 0, st>>>(br, nullptr, offs, stride, pairs, pcount, pcap);
+        D3D_LAUNCHED();
+    }
+    const size_t walk_smem = (size_t)stride * (sizeof(T) + 3 * 4 + 2);
+    if (aabb) {
+        D3D_CUDA_TRY(cudaFuncSetAttribute(nmsbs_walk_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_smem));
+        nmsbs_walk_kernel<T, true><<<(unsigned)nframes, NMSBS_THREADS, walk_smem, st>>>(nullptr, ar, scores, offs, stride, order, lists ? pairs : nullptr, pcount, pcap,
+                                                                                       nboff, nblst, thr, (T)score_thr, (T)sup_param, sup_type, suppressed);
+    } else {
+        D3D_CUDA_TRY(cudaFuncSetAttribute(nmsbs_walk_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_smem));
+        nmsbs_walk_kernel<T, false><<<(unsigned)nframes, NMSBS_THREADS, walk_smem, st>>>(br, nullptr, scores, offs, stride, order, lists ? pairs : nullptr, pcount, pcap,
+                                                                                        nboff, nblst, thr, (T)score_thr, (T)sup_param, sup_type, suppressed);
+    }
+    D3D_LAUNCHED();
+    return D3D_OK;
+}
+
 template <typename T> static size_t nmsb_ws_bytes(int64_t nframes, int64_t max_frame_boxes)
 {
     if (nframes < 1) nframes = 1;
@@ -1965,6 +2254,19 @@ extern "C" int d3d_nms2d_f32(const float *boxes, const float *scores, int64_t n,
 extern "C" int d3d_nms2d_f64(const double *boxes, const double *scores, int64_t n, int iou_type, int sup_type, float iou_thr, float score_thr, float sup_param,
                              uint8_t *suppressed, void *ws, size_t wsb, void *stream)
 { return nms_impl<double>(boxes, scores, n, iou_type, sup_type, iou_thr, score_thr, sup_param, suppressed, ws, wsb, (cudaStream_t)stream); }
+extern "C" size_t d3d_nms2d_batch_soft_workspace_bytes(int64_t total, int64_t nframes, int64_t max_frame_boxes, int dtype)
+{
+    if (max_frame_boxes <= 0 || max_frame_boxes > total) max_frame_boxes = total;
+    return dtype == D3D_F64 ? nmsbs_ws_bytes<double>(nframes, max_frame_boxes) : nmsbs_ws_bytes<float>(nframes, max_frame_boxes);
+}
+extern "C" int d3d_nms2d_batch_soft_f32(const float *boxes, const float *scores, int64_t total, const int64_t *frame_offsets, int64_t nframes,
+                                        int64_t max_frame_boxes, int iou_type, int sup_type, float iou_thr, float score_thr, float sup_param,
+                                        uint8_t *suppressed, void *ws, size_t wsb, void *stream)
+{ return nmsbs_impl<float>(boxes, scores, total, frame_offsets, nframes, max_frame_boxes, iou_type, sup_type, iou_thr, score_thr, sup_param, suppressed, ws, wsb, (cudaStream_t)stream); }
+extern "C" int d3d_nms2d_batch_soft_f64(const double *boxes, const double *scores, int64_t total, const int64_t *frame_offsets, int64_t nframes,
+                                        int64_t max_frame_boxes, int iou_type, int sup_type, float iou_thr, float score_thr, float sup_param,
+                                        uint8_t *suppressed, void *ws, size_t wsb, void *stream)
+{ return nmsbs_impl<double>(boxes, scores, total, frame_offsets, nframes, max_frame_boxes, iou_type, sup_type, iou_thr, score_thr, sup_param, suppressed, ws, wsb, (cudaStream_t)stream); }
 extern "C" size_t d3d_nms2d_batch_workspace_bytes(int64_t total, int64_t nframes, int64_t max_frame_boxes, int dtype)
 {
     if (max_frame_boxes <= 0 || max_frame_boxes > total) max_frame_boxes = total;

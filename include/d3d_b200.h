@@ -189,6 +189,20 @@ int d3d_nms2d_batch_f64(const double *boxes, const double *scores, int64_t total
                         int64_t max_frame_boxes, int iou_type, int supression_type, float iou_threshold, float score_threshold,
                         uint8_t *suppressed, void *workspace, size_t workspace_bytes, void *stream);
 
+/* Frame-batched soft-NMS: supression_type D3D_SUP_LINEAR or D3D_SUP_GAUSSIAN (D3D_SUP_HARD or anything else: D3D_ERR_INVALID_ARGUMENT;
+ * hard NMS is d3d_nms2d_batch_*).  Same packing, offsets, max_frame_boxes bound, 8192-box frame limit (D3D_ERR_UNSUPPORTED beyond)
+ * and nframes <= 65535 as d3d_nms2d_batch_*; per frame exactly the keep mask of d3d_nms2d_* with the same arguments.  One CTA walks
+ * each frame with the walk state in shared memory.  For iou_threshold >= 0 the pairs of a frame that may overlap above the threshold
+ * (bounding circles / AABBs meet) are listed first and a kept box decays only its listed neighbours; a frame whose list overflows
+ * (more than 32 x max_frame_boxes pairs) and every frame under a negative threshold decay all boxes behind the kept one. */
+size_t d3d_nms2d_batch_soft_workspace_bytes(int64_t total, int64_t nframes, int64_t max_frame_boxes, int dtype);
+int d3d_nms2d_batch_soft_f32(const float *boxes, const float *scores, int64_t total, const int64_t *frame_offsets, int64_t nframes,
+                             int64_t max_frame_boxes, int iou_type, int supression_type, float iou_threshold, float score_threshold,
+                             float supression_param, uint8_t *suppressed, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_nms2d_batch_soft_f64(const double *boxes, const double *scores, int64_t total, const int64_t *frame_offsets, int64_t nframes,
+                             int64_t max_frame_boxes, int iou_type, int supression_type, float iou_threshold, float score_threshold,
+                             float supression_param, uint8_t *suppressed, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Voxelization of a BATCH of frames (one frame = one reference VoxelGenerator.__call__).
  * points f32[total, nfeat] (first 3 columns xyz); frame_offsets DEVICE i64[nframes+1], ascending,
