@@ -199,6 +199,58 @@ def iou2dr_ex(boxes1, boxes2, method="grbox"):
     return out
 
 
+def _ex_row(a, b, method):
+    """values of `method` of one box a [1, 5] against b [M, 5], float64"""
+    if method == "box":
+        return iou2d(a, b)[0]
+    if method == "rbox":
+        return iou2dr_truth(a, b)[0]
+    return iou2dr_ex(a, b, method)[0]
+
+
+def iou_ex_local(boxes1, boxes2, method):
+    """[N, M] values of box2d_iou's `method` ("box", "rbox", "grbox", "drbox") with each pair moved, in float64, into the frame of
+    its first box's centre: the pinned forwards above (iou2d, iou2dr_truth, iou2dr_ex) without the cancellation of coordinates far
+    from the origin.  Float32 boxes are widened exactly, so the shift is exact too.  One vectorised call per row."""
+    b1, b2 = np.asarray(boxes1, np.float64), np.asarray(boxes2, np.float64)
+    out = np.empty((len(b1), len(b2)))
+    for i in range(len(b1)):
+        a, b = b1[i:i + 1].copy(), b2.copy()
+        b[:, :2] -= a[0, :2]
+        a[0, :2] = 0
+        out[i] = _ex_row(a, b, method)
+    return out
+
+
+def iou_ex_grad_local(boxes1, boxes2, method, h=1e-4, smooth_tol=1e-9):
+    """Per-pair derivatives of iou_ex_local by five-point differences in each of the 5 box fields, taken in the local frame:
+    returns (value [N, M], d1 [N, M, 5] = d value / d boxes1[i], d2 [N, M, 5] = d value / d boxes2[j], smooth bool [N, M]).
+    A pair is smooth when the stencils at h and h/2 agree to `smooth_tol` in all ten derivatives; elsewhere (touching edges, a
+    corner on an edge, a switch of hull edge or diameter, AABB min/max ties) the value has a kink within the stencil and no
+    derivative to compare with.  Perturbing all of boxes2 at once is exact: value[i, j] depends on boxes2[j] alone."""
+    b1, b2 = np.asarray(boxes1, np.float64), np.asarray(boxes2, np.float64)
+    n, m = len(b1), len(b2)
+    val, d1, d2, smooth = np.empty((n, m)), np.empty((n, m, 5)), np.empty((n, m, 5)), np.ones((n, m), bool)
+    for i in range(n):
+        a, b = b1[i:i + 1].copy(), b2.copy()
+        b[:, :2] -= a[0, :2]
+        a[0, :2] = 0
+        val[i] = _ex_row(a, b, method)
+        for side, d in ((0, d1), (1, d2)):
+            for k in range(5):
+                est = []
+                for hh in (h, h / 2):
+                    f = []
+                    for s in (-2, -1, 1, 2):
+                        a_, b_ = a.copy(), b.copy()
+                        (b_ if side else a_)[:, k] += s * hh
+                        f.append(_ex_row(a_, b_, method))
+                    est.append((f[0] - 8 * f[1] + 8 * f[2] - f[3]) / (12 * hh))
+                d[i, :, k] = est[0]
+                smooth[i] &= np.abs(est[0] - est[1]) <= smooth_tol
+    return val, d1, d2, smooth
+
+
 def match_greedy(distance, src_scores, src_tags, dst_tags, thresholds):
     """ScoreMatcher.match (d3d/tracking/matcher.pyx:138-162) over BaseMatcher.match_by_order (:93-122) for one threshold set
     `thresholds[category]`: returns (src_assignment i32[N], dst_assignment i32[M]), -1 = unmatched.  The source order is

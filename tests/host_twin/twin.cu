@@ -1,7 +1,8 @@
-// twin.cu -- TEST INFRASTRUCTURE: compiles the product's clip math (d3d_b200/csrc/geom.cuh) as HOST code
-// so the algorithm can be checked against the CPU oracle on a machine without a GPU.  Nothing in the
-// product loads this library.
+// twin.cu -- TEST INFRASTRUCTURE: compiles the product's clip math (d3d_b200/csrc/geom.cuh) and the pair math of the
+// differentiable IoU family (d3d_b200/csrc/iou_grad.cuh) as HOST code so the algorithm can be checked against the CPU
+// oracle on a machine without a GPU.  Nothing in the product loads this library.
 #include "../../d3d_b200/csrc/geom.cuh"
+#include "../../d3d_b200/csrc/iou_grad.cuh"
 using namespace d3d;
 template <typename T> static void run(const T *b1, long n, const T *b2, long m, T *out, int aabb)
 {
@@ -18,3 +19,39 @@ template <typename T> static void run(const T *b1, long n, const T *b2, long m, 
 }
 extern "C" void twin_iou_f32(const float *b1, long n, const float *b2, long m, float *out, int aabb) { run<float>(b1, n, b2, m, out, aabb); }
 extern "C" void twin_iou_f64(const double *b1, long n, const double *b2, long m, double *out, int aabb) { run<double>(b1, n, b2, m, out, aabb); }
+
+// the differentiable family as iou_grad.cu runs it: values [n, m] as iou_ex_fwd_kernel computes them and, for the upstream gradient
+// `up` [n, m], the gradient sums g1 [n, 5] and g2 [m, 5] as iou_bwd_kernel computes them (one owned box against the other side)
+template <typename T, int TYPE> static void run_ex(const T *b1, long n, const T *b2, long m, const T *up, T *out, T *g1, T *g2)
+{
+    for (long i = 0; i < n; i++)
+        for (long j = 0; j < m; j++)
+            out[i * m + j] = g_pair<T, TYPE, false>(g_make<T>(b1 + 5 * i, b1[5 * i], b1[5 * i + 1]), g_make<T>(b2 + 5 * j, b1[5 * i], b1[5 * i + 1]),
+                                                    T(0), nullptr, nullptr);
+    for (long s = 0; s < 2; s++)
+        for (long o = 0; o < (s ? m : n); o++) {
+            const T *own = (s ? b2 : b1) + 5 * o;
+            const GBox<T> O = g_make<T>(own, own[0], own[1]);
+            T acc[5] = {0, 0, 0, 0, 0};
+            for (long p = 0; p < (s ? n : m); p++) {
+                const T u = s ? up[p * m + o] : up[o * m + p];
+                if (u == T(0)) continue;
+                const GBox<T> P = g_make<T>((s ? b1 : b2) + 5 * p, own[0], own[1]);
+                T dump[5] = {0, 0, 0, 0, 0};
+                if (s) g_pair<T, TYPE, true>(P, O, u, dump, acc);
+                else g_pair<T, TYPE, true>(O, P, u, acc, dump);
+            }
+            for (int k = 0; k < 5; k++) (s ? g2 : g1)[5 * o + k] = acc[k];
+        }
+}
+template <typename T> static void run_ex_type(const T *b1, long n, const T *b2, long m, int type, const T *up, T *out, T *g1, T *g2)
+{
+    if (type == GT_BOX) run_ex<T, GT_BOX>(b1, n, b2, m, up, out, g1, g2);
+    else if (type == GT_RBOX) run_ex<T, GT_RBOX>(b1, n, b2, m, up, out, g1, g2);
+    else if (type == GT_GIOU) run_ex<T, GT_GIOU>(b1, n, b2, m, up, out, g1, g2);
+    else run_ex<T, GT_DIOU>(b1, n, b2, m, up, out, g1, g2);
+}
+extern "C" void twin_iou_ex_f32(const float *b1, long n, const float *b2, long m, int type, const float *up, float *out, float *g1, float *g2)
+{ run_ex_type<float>(b1, n, b2, m, type, up, out, g1, g2); }
+extern "C" void twin_iou_ex_f64(const double *b1, long n, const double *b2, long m, int type, const double *up, double *out, double *g1, double *g2)
+{ run_ex_type<double>(b1, n, b2, m, type, up, out, g1, g2); }
