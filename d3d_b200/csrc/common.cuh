@@ -9,8 +9,8 @@ namespace d3d {
 
 extern std::atomic<int64_t> g_launches;
 // tuning knobs (core.cu): environment read once at first use, d3d_tuning_set() overrides
-enum { D3D_TUNE_NMS_PATH = 0, D3D_TUNE_NMS_STAGE, D3D_TUNE_NMS_NT, D3D_TUNE_CROP_PATH, D3D_TUNE_VOX_CLUSTER, D3D_TUNE_VOX_ROUTE, D3D_TUNE_VOX_MAXCL, D3D_TUNE_VOX_CF,
-       D3D_TUNE_VOX_ROLES, D3D_TUNE_NMS_STOP, D3D_TUNE_SCATTER_PATH, D3D_TUNE_NMS_FIX, D3D_TUNE_NMS_BATCH_PATH, D3D_TUNE_SORT_COOP, D3D_TUNE_COUNT };
+enum { D3D_TUNE_NMS_PATH = 0, D3D_TUNE_CROP_PATH, D3D_TUNE_VOX_ROUTE, D3D_TUNE_NMS_STOP, D3D_TUNE_SCATTER_PATH, D3D_TUNE_NMS_FIX, D3D_TUNE_NMS_BATCH_PATH,
+       D3D_TUNE_SORT_COOP, D3D_TUNE_COUNT };
 int tuning(int knob, int dflt);
 void set_cuda_error(cudaError_t e);
 

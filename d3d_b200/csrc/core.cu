@@ -13,14 +13,15 @@ void set_cuda_error(cudaError_t e)
 }
 
 // Tuning knobs.  The environment is read ONCE, at the first use of a knob (results of a call never depend on the environment at call
-// time); tests and tuning tools change a knob through d3d_tuning_set().  Knobs select between back ends that produce identical results.
-static const char *const g_tune_names[D3D_TUNE_COUNT] = {"D3D_B200_NMS_PATH", "D3D_B200_NMS_STAGE", "D3D_B200_NMS_NT", "D3D_B200_CROP_PATH", "D3D_B200_VOX_CLUSTER",
-                                                         "D3D_B200_VOX_ROUTE", "D3D_B200_VOX_MAXCL", "D3D_B200_VOX_CF", "D3D_B200_VOX_ROLES", "D3D_B200_NMS_STOP", "D3D_B200_SCATTER_PATH", "D3D_B200_NMS_FIX", "D3D_B200_NMS_BATCH_PATH", "D3D_B200_SORT_COOP"};
+// time); tests and tuning tools change a knob through d3d_tuning_set().  Knobs select between back ends that produce identical results;
+// the one exception is NMS_STOP, which is for measurement only: it ends d3d_nms2d_* after a phase and leaves the keep mask unwritten.
+static const char *const g_tune_names[D3D_TUNE_COUNT] = {"D3D_B200_NMS_PATH", "D3D_B200_CROP_PATH", "D3D_B200_VOX_ROUTE", "D3D_B200_NMS_STOP",
+                                                         "D3D_B200_SCATTER_PATH", "D3D_B200_NMS_FIX", "D3D_B200_NMS_BATCH_PATH", "D3D_B200_SORT_COOP"};
 static std::atomic<int> g_tune_val[D3D_TUNE_COUNT];
 static std::atomic<int> g_tune_state[D3D_TUNE_COUNT];   // 0 unread, 1 unset, 2 set
 static int tune_parse(int knob, const char *e)
 {
-    if (knob == D3D_TUNE_NMS_PATH) return e[0] == 'd' ? 2 : (e[0] == 't' ? 1 : (e[0] == 'w' ? 3 : atoi(e)));     // dense | tiles | warp (spatial, a warp per box) | (spatial, a CTA per cell)
+    if (knob == D3D_TUNE_NMS_PATH) return e[0] == 'd' ? 2 : (e[0] == 't' ? 1 : atoi(e));     // dense | tiles | (spatial)
     if (knob == D3D_TUNE_CROP_PATH) return e[0] == 'b' ? 1 : (e[0] == 'g' ? 2 : atoi(e));    // brute | grid | (auto)
     if (knob == D3D_TUNE_NMS_BATCH_PATH) return e[0] == 'd' ? 1 : atoi(e);                  // dense | (edges)
     if (knob == D3D_TUNE_SCATTER_PATH) return e[0] == 'g' ? 1 : (e[0] == 't' ? 2 : atoi(e)); // gather | tiles | (auto)

@@ -1248,15 +1248,11 @@ static int vc_shape(VcShape *out, int64_t max_frame_points)
         }
         return occ[cs];
     };
-    int forced = 0, route = DENSE ? 0 : 1;
-    forced = tuning(D3D_TUNE_VOX_CLUSTER, 0);   // tuning overrides
-    route = DENSE ? 0 : tuning(D3D_TUNE_VOX_ROUTE, route);
-    if (forced < 0 || forced > VC_MAX_CSIZE) forced = 0;
+    const int route = DENSE ? 0 : tuning(D3D_TUNE_VOX_ROUTE, 1);   // tuning override
     VcShape best = {0, 0, dyn, 0};
     if (route) {
         VrPlan pl;
         for (int cs = 8; cs >= 4; cs -= 2) {
-            if (forced && cs != forced) continue;
             if (!vr_plan((uint32_t)(max_frame_points > 0 ? max_frame_points : 1), cs, dyn, &pl)) continue;
             const int n = query(cs);
             if (n > 0 && n * cs > best.csize * best.max_clusters) best = {cs, n, dyn, 1};
@@ -1264,12 +1260,10 @@ static int vc_shape(VcShape *out, int64_t max_frame_points)
     }
     if (best.csize == 0) {
         for (int cs = 8; cs >= 4; cs -= 2) {   // 8, 6, 4: smaller clusters put more frames in flight than L2 holds
-            if (forced && cs != forced) continue;
             const int n = query(cs);
             if (n > 0 && n * cs > best.csize * best.max_clusters) best = {cs, n, dyn, route};
         }
     }
-    if (best.csize == 0 && forced) { const int n = query(forced); if (n > 0) best = {forced, n, dyn, route}; }
     if (best.csize == 0) return D3D_ERR_CUDA;
     *out = best;
     return D3D_OK;
@@ -1295,7 +1289,6 @@ static int vc_launch(VcArgs &args, int64_t nframes, int64_t max_frame_points, si
     at[0].val.clusterDim.x = csize; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     lc.attrs = at; lc.numAttrs = 1;
     int64_t ncl = shape.max_clusters;
-    { const int m = tuning(D3D_TUNE_VOX_MAXCL, 0); if (m > 0 && m < ncl) ncl = m; }   // tuning override
     if (ncl > nframes) ncl = nframes;
     if (ncl > VC_MAX_CLUSTERS) ncl = VC_MAX_CLUSTERS;
     const size_t state_bytes = 256 + align_up((size_t)nframes * 16);

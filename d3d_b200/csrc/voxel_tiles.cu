@@ -26,7 +26,7 @@
 //                                frames (decoupled look-back): voxel ids in order of first appearance, packed rows.
 //   write   (1024 points / CTA)  voxel rows and kept point rows streamed out; no barrier, no waiting.
 //
-// A batch is cut into chunks of frames (128 by default; D3D_B200_VOX_CF, read once, for tuning).  Small chunks keep the scratch
+// A batch is cut into chunks of 64 frames (vt_geom).  Small chunks keep the scratch
 // (queues, words, row tables: ~1.3 MB per frame, plus the frame itself) in L2 between the kernels, large chunks give fewer
 // and fuller launches; on B200 the large chunks win (C2 x 128 frames: 0.59 ms against 0.74 ms with chunks of 16) although
 // the scratch then travels through HBM (DRAM traffic ~1.9x the algorithmic 16 B/point in, 32 B/kept point + 28 B/voxel out).
@@ -550,10 +550,6 @@ __global__ void __launch_bounds__(VT_THREADS, D3D_VT_WCTAS) vt_write_kernel(cons
 // ------------------------------------------------------------------------------------------------ host side
 static uint32_t vt_lg2_ceil(uint64_t x) { uint32_t l = 0; while ((1ull << l) < x) l++; return l; }
 
-static int vt_env_cf() { const int v = tuning(D3D_TUNE_VOX_CF, 0); return v > 0 ? v : 0; }
-// tuning only: bit 0 split, 1 bucket, 2 scan, 3 write (later stages may only be dropped together with everything behind them)
-static int vt_env_roles() { return tuning(D3D_TUNE_VOX_ROLES, 15); }
-
 static bool vt_geom(int64_t max_frame_points, int64_t nframes, VtGeom *g)
 {
     if (max_frame_points < 1) max_frame_points = 1;
@@ -567,8 +563,7 @@ static bool vt_geom(int64_t max_frame_points, int64_t nframes, VtGeom *g)
     const uint32_t per = (g->lmax + g->P - 1) / g->P;            // points per bucket if every point is kept and the hash is even (<= 512)
     g->qcap = (per + per / 2 + 128 + 15) & ~15u;                 // multiple of 16 entries: every bucket's queue starts on a 128-byte line
     if (g->qcap > (uint32_t)VT_QCAP) g->qcap = VT_QCAP;
-    int cf = vt_env_cf();
-    if (cf <= 0) cf = 64;    // measured on C2 x 128 frames (one stream): 0.74 ms with chunks of 16 (scratch mostly L2-resident), 0.59 ms with one chunk of 128 (fewer, fuller launches)
+    int cf = 64;    // measured on C2 x 128 frames (one stream): 0.74 ms with chunks of 16 (scratch mostly L2-resident), 0.59 ms with one chunk of 128 (fewer, fuller launches)
     if ((int64_t)cf > nframes) cf = (int)(nframes > 0 ? nframes : 1);
     g->CF = (uint32_t)cf;
     g->nchunks = (uint32_t)((nframes + cf - 1) / cf);
@@ -671,7 +666,6 @@ int vox_tiles_sparse(const float *points, int64_t total, int nfeat, const int64_
     a.single_ok = cfg.min_points <= 1 ? 1 : 0;
 
     D3D_CUDA_TRY(cudaMemsetAsync(w + lay.zero, 0, lay.zero_end - lay.zero, st));
-    const int roles = vt_env_roles();
     // Two chunks are in flight at a time, each on its own internal stream with its own scratch: the four kernels of a chunk have
     // different bottlenecks (issue slots, shared-memory latency, a short dependent chain, DRAM stores) and fill each other's tails.
     // Inside a stream the kernels are chained with programmatic dependent launch (each may be scheduled while its predecessor
@@ -704,21 +698,21 @@ int vox_tiles_sparse(const float *points, int64_t total, int nfeat, const int64_
             lc.attrs = pdl; lc.numAttrs = 1;
             return lc;
         };
-        if (roles & 1) {
+        {
             cudaLaunchConfig_t lc = cfg_of(dim3(g.tpf, nf), VT_THREADS, dyn_split);
             if (nfeat == 4) D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_split_kernel<true>, al, dv, c));
             else D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_split_kernel<false>, al, dv, c));
             D3D_LAUNCHED();
         }
-        if (roles & 2) { cudaLaunchConfig_t lc = cfg_of(dim3(g.P, nf), VT_BT, 0); D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_bucket_kernel, al)); D3D_LAUNCHED(); }
+        { cudaLaunchConfig_t lc = cfg_of(dim3(g.P, nf), VT_BT, 0); D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_bucket_kernel, al)); D3D_LAUNCHED(); }
         if (lanes && c > 0) D3D_CUDA_TRY(cudaStreamWaitEvent(cs, lanes->scan_done[(c - 1) & 1u], 0));
-        if (roles & 4) {
+        {
             cudaLaunchConfig_t lc = cfg_of(dim3(nf * g.spf), VT_THREADS, 0);
             if (lanes && c > 0) lc.numAttrs = 0;   // its predecessor in the other lane is a full dependency (event), not a programmatic one
             D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_scan_kernel, al, c)); D3D_LAUNCHED();
         }
         if (lanes) D3D_CUDA_TRY(cudaEventRecord(lanes->scan_done[c & 1u], cs));
-        if (roles & 8) {
+        {
             cudaLaunchConfig_t lc = cfg_of(dim3(g.tpf, nf), VT_THREADS, 0);
             if (lanes) lc.numAttrs = 0;            // an event record sits between the scan and this launch
             if (nfeat == 4) D3D_CUDA_TRY(cudaLaunchKernelEx(&lc, vt_write_kernel<true>, al, dv, c));

@@ -53,11 +53,13 @@ enum d3d_voxel_algo { D3D_VOXEL_AUTO = 0, D3D_VOXEL_SORT = 1, D3D_VOXEL_CLUSTER 
 int d3d_abi_version(void);
 const char *d3d_error_string(int status);
 const char *d3d_last_cuda_error(void);
-/* Tuning knobs select between back ends that produce identical results (names = the environment variables D3D_B200_NMS_PATH,
- * D3D_B200_NMS_STAGE, D3D_B200_NMS_NT, D3D_B200_CROP_PATH, D3D_B200_VOX_CLUSTER, D3D_B200_VOX_ROUTE, D3D_B200_VOX_MAXCL, D3D_B200_VOX_CF,
- * D3D_B200_VOX_ROLES, D3D_B200_SCATTER_PATH (gather | tiles), D3D_B200_NMS_FIX (0 | 1 | 2: resolve by the block walk | the pulled parallel fixpoint | the fixpoint in rounds), D3D_B200_NMS_BATCH_PATH (dense),
- * D3D_B200_SORT_COOP (0 | 1 | 2), D3D_B200_NMS_PATH also takes "warp" (spatial candidates with a warp per box instead of a CTA per grid cell), and D3D_B200_NMS_STOP, which truncates d3d_nms2d_* after a phase for phase timing).  The environment is read once, at the first use of a knob; this call overrides (set != 0) or clears (set == 0) a
- * knob afterwards -- tests and tuning tools use it instead of changing the environment of a running process. */
+/* Tuning knobs force one of the back ends that produce identical results (names = the environment variables D3D_B200_NMS_PATH
+ * (tiles | dense), D3D_B200_NMS_FIX (0 | 1: resolve by the block walk | the pulled parallel fixpoint; batched NMS: 2 = rounds over the
+ * edge list), D3D_B200_NMS_BATCH_PATH (dense), D3D_B200_SORT_COOP (0 | 1 | 2), D3D_B200_CROP_PATH (brute | grid), D3D_B200_SCATTER_PATH
+ * (gather | tiles), D3D_B200_VOX_ROUTE (0), and D3D_B200_NMS_STOP, which truncates d3d_nms2d_* after a phase for phase timing and so
+ * is the one knob that changes a result).  The environment is read once, at the first use of a knob; this call overrides (set != 0) or
+ * clears (set == 0) a knob afterwards -- tests and tuning tools use it instead of changing the environment of a running process.
+ * An unknown name returns D3D_ERR_INVALID_ARGUMENT. */
 int d3d_tuning_set(const char *name, int value, int set);
 /* number of kernels this library has launched in the calling process (bench.py's gpu_launches) */
 int64_t d3d_launch_count(void);

@@ -58,6 +58,23 @@ def test_argument_validation_without_gpu():
     assert sc(8, 1, 4, 8, 1, 1, dims, 1, 0, 8, 0) == 1   # dim 4
 
 
+def test_tuning_knob_table():
+    """d3d_tuning_set accepts the knobs that force a path some input reaches on its own (plus NMS_STOP, the phase timing of bench.py)
+    and rejects the names of retired knobs with INVALID_ARGUMENT."""
+    lib = C.CDLL(LIB)
+    lib.d3d_tuning_set.argtypes = [C.c_char_p, C.c_int, C.c_int]
+    kept = ["NMS_PATH", "NMS_FIX", "NMS_BATCH_PATH", "SORT_COOP", "CROP_PATH", "SCATTER_PATH", "VOX_ROUTE", "NMS_STOP"]
+    retired = ["NMS_NT", "NMS_STAGE", "VOX_CLUSTER", "VOX_MAXCL", "VOX_CF", "VOX_ROLES"]
+    try:
+        for k in kept:
+            assert lib.d3d_tuning_set(b"D3D_B200_" + k.encode(), 0, 1) == 0, k
+        for k in retired:
+            assert lib.d3d_tuning_set(b"D3D_B200_" + k.encode(), 0, 1) == 1, k
+    finally:
+        for k in kept:
+            lib.d3d_tuning_set(b"D3D_B200_" + k.encode(), 0, 0)
+
+
 def test_product_never_touches_the_oracle():
     """The oracle is test infrastructure: nothing under d3d_b200/ may import, link or open it."""
     bad = []

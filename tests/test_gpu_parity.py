@@ -462,10 +462,9 @@ def test_nms_batch_equals_per_frame(dev, oracle):
 
 
 def test_nms_parallel_resolve_equals_list_walk(dev, oracle):
-    """the resolve phase has three forms -- the block-by-block walk in score order on one SM, the parallel fixpoint pulled over transposed
-    hit lists (default from 8192 boxes on) and the same fixpoint by rounds of keep / suppress decisions -- with the same keep mask: sizes on
-    both sides of the switch, both candidate back ends, score thresholds, and a chain of pairwise overlapping boxes whose depth exceeds the
-    round limit (the round form gives up and the walk decides; the pulled form follows the chain)"""
+    """the resolve phase has two forms -- the block-by-block walk in score order on one SM and the parallel fixpoint pulled over transposed
+    hit lists (default from 8192 boxes on) -- with the same keep mask: sizes on both sides of the switch, both candidate back ends, score
+    thresholds, and a chain of pairwise overlapping boxes 200 decisions deep that both forms follow to the end"""
     from d3d_b200.box import box2d_nms
     rng = np.random.default_rng(11)
     cases = [proposals(rng, n, nobj, extent=ext) for n, nobj, ext in ((64, 4, 10.0), (1000, 30, 30.0), (4097, 150, 60.0), (12000, 500, 75.0))]
@@ -477,7 +476,7 @@ def test_nms_parallel_resolve_equals_list_walk(dev, oracle):
         for thr, sthr in ((0.5, 0.0), (0.3, 0.4)):
             exp = oracle.box2d_nms(P, sc, "rbox", iou_threshold=thr, score_threshold=sthr, cuda_score_rule=True)
             for path in (None, 1):          # spatial candidates | dense tiles
-                for fix in (0, 1, 2):       # list walk | parallel fixpoint, pulled (no rounds) | parallel fixpoint by rounds
+                for fix in (0, 1):          # list walk | parallel fixpoint, pulled
                     _cabi.tuning_set("D3D_B200_NMS_PATH", path)
                     _cabi.tuning_set("D3D_B200_NMS_FIX", fix)
                     got = box2d_nms(_t(P, dev), _t(sc, dev), "rbox", iou_threshold=thr, score_threshold=sthr).cpu().numpy()
@@ -535,19 +534,19 @@ def test_sort_forms_agree(dev):
 
 
 def test_nms_back_ends_agree(dev):
-    """the NMS back ends (spatial candidate grid with a CTA per cell or a warp per box, dense tiles + list resolve, dense matrix + dense
-    resolve) give the same keep mask (the knob is set through d3d_tuning_set: the environment is read once)"""
+    """the NMS back ends (spatial candidate grid with a CTA per cell, dense tiles + list resolve, dense matrix + dense resolve) give the
+    same keep mask (the knob is set through d3d_tuning_set: the environment is read once)"""
     from d3d_b200.box import box2d_nms
     rng = np.random.default_rng(5)
     for n, nobj, extent in ((20000, 800, 75.0), (3000, 40, 30.0), (700, 700, 400.0)):
         P, s = proposals(rng, n, nobj, extent=extent)
         for dt in (np.float64, np.float32):
             out = {}
-            for path in ("", "warp", "tiles", "dense"):   # "": spatial grid, a CTA per cell (default); "warp": spatial grid, a warp per box
-                _cabi.tuning_set("D3D_B200_NMS_PATH", {"": None, "dense": 2, "tiles": 1, "warp": 3}[path])
+            for path in ("", "tiles", "dense"):   # "": spatial grid, a CTA per cell (default)
+                _cabi.tuning_set("D3D_B200_NMS_PATH", {"": None, "dense": 2, "tiles": 1}[path])
                 out[path] = box2d_nms(_t(P.astype(dt), dev), _t(s.astype(dt), dev), "rbox", iou_threshold=0.45, precise=dt == np.float64).cpu().numpy()
             _cabi.tuning_set("D3D_B200_NMS_PATH", None)
-            assert np.array_equal(out[""], out["dense"]) and np.array_equal(out["tiles"], out["dense"]) and np.array_equal(out["warp"], out["dense"]), (n, dt)
+            assert np.array_equal(out[""], out["dense"]) and np.array_equal(out["tiles"], out["dense"]), (n, dt)
             assert 0 < out[""].sum() < n
     # a negative threshold suppresses disjoint pairs too (IoU 0 > thr), like the reference: only the best box survives
     P, s = proposals(rng, 500, 50, extent=100.0)
