@@ -53,6 +53,8 @@ iou2dr = {F32: _sig("d3d_iou2dr_f32", C.c_int, _iou_sig), F64: _sig("d3d_iou2dr_
 iou2d = {F32: _sig("d3d_iou2d_f32", C.c_int, _iou_sig), F64: _sig("d3d_iou2d_f64", C.c_int, _iou_sig)}
 iou3d_distance_workspace_bytes = _sig("d3d_iou3d_distance_workspace_bytes", _sz, [_i64, _i64])
 iou3d_distance = _sig("d3d_iou3d_distance_f32", C.c_int, [_vp, _i64, _vp, _i64, C.c_int, _vp, _i64, _vp, _sz, _vp])
+iou3d_distance_batch_workspace_bytes = _sig("d3d_iou3d_distance_batch_workspace_bytes", _sz, [_i64, _i64, _i64])
+iou3d_distance_batch = _sig("d3d_iou3d_distance_batch_f32", C.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _sz, _vp])
 crop_workspace_bytes = _sig("d3d_crop2dr_workspace_bytes", _sz, [_i64, _i64, C.c_int])
 _crop_sig = [_vp, _i64, _vp, _i64, _vp, _vp, _sz, _vp]
 crop2dr = {F32: _sig("d3d_crop2dr_f32", C.c_int, _crop_sig), F64: _sig("d3d_crop2dr_f64", C.c_int, _crop_sig)}
@@ -67,6 +69,7 @@ _ibw_sig = [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp]
 iou_backward = {name: {F32: _sig(f"d3d_{name}_backward_f32", C.c_int, _ibw_sig), F64: _sig(f"d3d_{name}_backward_f64", C.c_int, _ibw_sig)}
                 for name in ("iou2d", "iou2dr", "giou2dr", "diou2dr")}
 match_greedy = _sig("d3d_match_greedy_f32", C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
+match_greedy_batch = _sig("d3d_match_greedy_batch_f32", C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
 iou_count_candidates = _sig("d3d_iou_count_candidates", C.c_int, [_vp, _i64, _vp, _i64, C.c_int, _vp, _vp, _sz, _vp])
 nms_workspace_bytes = _sig("d3d_nms2d_workspace_bytes", _sz, [_i64, C.c_int])
 _nms_sig = [_vp, _vp, _i64, C.c_int, C.c_int, _f, _f, _f, _vp, _vp, _sz, _vp]

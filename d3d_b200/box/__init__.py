@@ -413,6 +413,18 @@ def box3dr_pdist(points, boxes, project_axis=2):
                        torch.where(dist_2d > 0, dist_p, -torch.sqrt(dist_2d.square() + dist_p.square())))
 
 
+def _dist3d_input(boxes):
+    """float32 copy on the device with the sizes clamped to +-1e3: "prevent really weird boxes with unusual size" (matcher.pyx:50-52)"""
+    b = _c.to_device(boxes).to(torch.float32).contiguous().clone()
+    b[:, 3:6].clamp_(-1e3, 1e3)
+    return b
+
+
+def _check_boxes3d(src_boxes, dst_boxes):
+    if len(src_boxes.shape) != 2 or len(dst_boxes.shape) != 2 or src_boxes.shape[1] != 7 or dst_boxes.shape[1] != 7:
+        raise ValueError("Input boxes should be Nx7 tensors: x, y, z, lx, ly, lz, rz")
+
+
 def box3d_iou_distance(src_boxes, dst_boxes, metric="riou"):
     '''
     Distance matrix of the detection evaluator / tracking matcher: ``1 - iou2d * ziou`` in float32, the array
@@ -430,15 +442,11 @@ def box3d_iou_distance(src_boxes, dst_boxes, metric="riou"):
         assert isinstance(dst_boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
         src_boxes, dst_boxes = torch.from_numpy(src_boxes), torch.from_numpy(dst_boxes)
         convert_numpy = True
-    if len(src_boxes.shape) != 2 or len(dst_boxes.shape) != 2 or src_boxes.shape[1] != 7 or dst_boxes.shape[1] != 7:
-        raise ValueError("Input boxes should be Nx7 tensors: x, y, z, lx, ly, lz, rz")
+    _check_boxes3d(src_boxes, dst_boxes)
     if metric.lower() not in ("riou", "iou"):
         raise ValueError("Unrecognized distance metric!")
     odev = src_boxes.device
-    b1 = _c.to_device(src_boxes).to(torch.float32).contiguous().clone()
-    b2 = _c.to_device(dst_boxes).to(torch.float32).contiguous().clone()
-    b1[:, 3:6].clamp_(-1e3, 1e3)   # "prevent really weird boxes with unusual size" (matcher.pyx:50-52)
-    b2[:, 3:6].clamp_(-1e3, 1e3)
+    b1, b2 = _dist3d_input(src_boxes), _dist3d_input(dst_boxes)
     n, m = b1.shape[0], b2.shape[0]
     out = torch.empty((n, m), dtype=torch.float32, device=b1.device)
     if n and m:
@@ -515,6 +523,10 @@ def box2d_nms(boxes, scores, iou_method="box", supression_method="hard",
     return mask
 
 
+def _as_tensor(x, dt):
+    return (torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else torch.as_tensor(x)).to(dt)
+
+
 def match_greedy(distance, src_scores, src_tags, dst_tags, thresholds):
     '''
     Greedy score-ordered matching on a distance matrix: ``ScoreMatcher.match`` of the reference (d3d/tracking/matcher.pyx:138-162 over
@@ -530,19 +542,18 @@ def match_greedy(distance, src_scores, src_tags, dst_tags, thresholds):
         for a single threshold set.  numpy in -> numpy out.
     '''
     convert_numpy = isinstance(distance, np.ndarray)
-    as_t = lambda x, dt: (torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else torch.as_tensor(x)).to(dt)
-    distance = as_t(distance, torch.float32)
+    distance = _as_tensor(distance, torch.float32)
     odev = distance.device
     d = _c.to_device(distance).contiguous()
     dev = d.device
     if d.dim() != 2:
         raise ValueError("distance should be an NxM matrix")
     n, m = d.shape
-    thr = as_t(thresholds, torch.float32)
+    thr = _as_tensor(thresholds, torch.float32)
     single = thr.dim() == 1
     thr = thr.reshape(1, -1) if single else thr
-    scores = as_t(src_scores, torch.float64)
-    st, dt_ = as_t(src_tags, torch.int32).to(dev).contiguous(), as_t(dst_tags, torch.int32).to(dev).contiguous()
+    scores = _as_tensor(src_scores, torch.float64)
+    st, dt_ = _as_tensor(src_tags, torch.int32).to(dev).contiguous(), _as_tensor(dst_tags, torch.int32).to(dev).contiguous()
     if len(scores) != n or len(st) != n or len(dt_) != m:
         raise ValueError("scores / tags do not match the distance matrix")
     order = torch.flip(torch.argsort(scores.cpu(), stable=True), dims=[0]).to(torch.int32).to(dev).contiguous()   # np.flip(np.argsort(scores))
@@ -559,3 +570,179 @@ def match_greedy(distance, src_scores, src_tags, dst_tags, thresholds):
     if odev.type != "cuda" or convert_numpy:
         sa, da = sa.cpu(), da.cpu()
     return (sa.numpy(), da.numpy()) if convert_numpy else (sa, da)
+
+
+def _frame_offsets(offsets=None, lens=None):
+    """CPU int64 [nframes + 1] from given offsets or from frame lengths"""
+    if lens is not None:
+        off = torch.zeros(len(lens) + 1, dtype=torch.int64)
+        off[1:] = torch.tensor(lens, dtype=torch.int64).cumsum(0)
+        return off
+    off = torch.as_tensor(offsets).to(torch.int64).cpu().reshape(-1)
+    if off.numel() < 1 or int(off[0]) != 0 or bool((off[1:] < off[:-1]).any()):
+        raise ValueError("frame offsets must start at 0 and be ascending")
+    return off
+
+
+def _block_offsets(src_off, dst_off):
+    """start of every frame's [n_f, m_f] block in the packed distance buffer: the running sum of n_f * m_f"""
+    off = torch.zeros_like(src_off)
+    off[1:] = ((src_off[1:] - src_off[:-1]) * (dst_off[1:] - dst_off[:-1])).cumsum(0)
+    return off
+
+
+def box3d_iou_distance_batch(src_boxes, dst_boxes, src_offsets=None, dst_offsets=None, metric="riou"):
+    '''
+    :func:`box3d_iou_distance` on a batch of frames in one launch sequence (the detection evaluator computes one matrix per frame of a
+    validation set); per frame the matrix equals :func:`box3d_iou_distance` on that frame, bit for bit.  Two call forms, like
+    :func:`box2d_nms_batch`: lists of per-frame ``src_boxes`` [n_f, 7] / ``dst_boxes`` [m_f, 7] (returns the list of [n_f, m_f] float32
+    matrices, views into one packed buffer), or the frames packed back to back as ``src_boxes`` [total_src, 7] / ``dst_boxes``
+    [total_dst, 7] with ``src_offsets`` / ``dst_offsets`` (int64 [nframes + 1], CPU) (returns ``(dist_flat, dist_offsets)``: frame f's
+    matrix is ``dist_flat[dist_offsets[f]:dist_offsets[f + 1]].view(n_f, m_f)``).  numpy in -> numpy out, host tensors in -> host tensors out.
+
+    :param metric: 'riou' or 'iou', as in :func:`box3d_iou_distance`
+    '''
+    as_list = isinstance(src_boxes, (list, tuple))
+    if as_list:
+        if not isinstance(dst_boxes, (list, tuple)) or len(src_boxes) != len(dst_boxes):
+            raise ValueError("src_boxes and dst_boxes should hold the same number of frames")
+        if len(src_boxes) == 0:
+            return []
+        numpy_in = isinstance(src_boxes[0], np.ndarray)
+        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
+        slist, dlist = [tt(b) for b in src_boxes], [tt(b) for b in dst_boxes]
+        for a, b in zip(slist, dlist):
+            _check_boxes3d(a, b)
+        odev = slist[0].device
+        src_off, dst_off = _frame_offsets(lens=[len(b) for b in slist]), _frame_offsets(lens=[len(b) for b in dlist])
+        b1 = _dist3d_input(torch.cat([b.to(torch.float32) for b in slist]))   # one copy to the device per box set
+        b2 = _dist3d_input(torch.cat([b.to(torch.float32) for b in dlist]))
+    else:
+        numpy_in = isinstance(src_boxes, np.ndarray)
+        if numpy_in:
+            assert isinstance(dst_boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
+            src_boxes, dst_boxes = torch.from_numpy(src_boxes), torch.from_numpy(dst_boxes)
+        if src_offsets is None or dst_offsets is None:
+            raise ValueError("packed boxes need the frame offsets")
+        _check_boxes3d(src_boxes, dst_boxes)
+        odev = src_boxes.device
+        src_off, dst_off = _frame_offsets(src_offsets), _frame_offsets(dst_offsets)
+        b1, b2 = _dist3d_input(src_boxes), _dist3d_input(dst_boxes)
+    if src_off.numel() != dst_off.numel() or int(src_off[-1]) != len(b1) or int(dst_off[-1]) != len(b2):
+        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
+    if metric.lower() not in ("riou", "iou"):
+        raise ValueError("Unrecognized distance metric!")
+    nframes = src_off.numel() - 1
+    dist_off = _block_offsets(src_off, dst_off)
+    dist = torch.empty(int(dist_off[-1]), dtype=torch.float32, device=b1.device)
+    if dist.numel():
+        n_f, m_f = src_off[1:] - src_off[:-1], dst_off[1:] - dst_off[:-1]
+        offs = torch.cat([src_off, dst_off, dist_off]).to(b1.device, non_blocking=True)   # one copy of the three offset arrays
+        od1, od2, odd = offs[:nframes + 1], offs[nframes + 1:2 * nframes + 2], offs[2 * nframes + 2:]
+        ws = _c.workspace(_c.iou3d_distance_batch_workspace_bytes(len(b1), len(b2), nframes), b1.device)
+        with torch.cuda.device(b1.device):
+            st = _c.iou3d_distance_batch(_c.ptr(b1), len(b1), _c.ptr(od1), _c.ptr(b2), len(b2), _c.ptr(od2), nframes, int(n_f.max()), int(m_f.max()),
+                                         1 if metric.lower() == "riou" else 0, _c.ptr(odd), _c.ptr(dist), _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        _c.check(st, "box3d_iou_distance_batch")
+    if odev.type != "cuda" or numpy_in:
+        dist = dist.cpu()
+    if numpy_in:
+        dist, dist_off = dist.numpy(), dist_off.numpy()
+    if not as_list:
+        return dist, dist_off
+    return [dist[int(dist_off[f]):int(dist_off[f + 1])].reshape(int(src_off[f + 1] - src_off[f]), int(dst_off[f + 1] - dst_off[f])) for f in range(nframes)]
+
+
+def _frame_score_order(scores, src_off_dev, nframes):
+    """per frame np.flip(np.argsort(scores, kind="stable")) (descending, ties to the higher index, NaN first) in frame-local indices,
+    from device sorts and gathers without a host synchronise"""
+    dev, total = scores.device, scores.numel()
+    s = torch.where(torch.isnan(scores), float("nan"), scores + 0.0)   # one NaN and one zero, so the device sort orders like the host sort
+    fid = torch.repeat_interleave(torch.arange(nframes, device=dev), src_off_dev[1:] - src_off_dev[:-1], output_size=total)
+    o = torch.argsort(s, stable=True)                  # ascending over the whole batch
+    o = o[torch.argsort(fid[o], stable=True)]          # grouped by frame, ascending inside each frame
+    start = src_off_dev[:-1][fid]
+    rev = start + src_off_dev[1:][fid] - 1 - torch.arange(total, device=dev)   # reverse each frame's segment
+    return (o[rev] - start).to(torch.int32).contiguous()
+
+
+def match_greedy_batch(distance, src_scores, src_tags, dst_tags, thresholds, src_offsets=None, dst_offsets=None):
+    '''
+    :func:`match_greedy` on a batch of frames in one launch: per frame and threshold set the assignment equals :func:`match_greedy` on
+    that frame.  Two call forms, like :func:`box3d_iou_distance_batch`: lists of per-frame ``distance`` [n_f, m_f], ``src_scores``,
+    ``src_tags`` and ``dst_tags`` (returns a list of per-frame ``(src_assignment, dst_assignment)`` pairs shaped as :func:`match_greedy`
+    shapes them), or ``distance = (dist_flat, dist_offsets)`` as the packed :func:`box3d_iou_distance_batch` returns it, packed scores and
+    tags, and ``src_offsets`` / ``dst_offsets`` (int64 [nframes + 1], CPU) (returns ``(src_assignment [T, total_src], dst_assignment
+    [T, total_dst])`` with frame-local indices).  The thresholds (T x C, or C for a single set, which drops the leading dimension) are
+    shared by all frames.  Frames of more than 4096 destination boxes fall back to one :func:`match_greedy` call per frame.
+    numpy in -> numpy out, host tensors in -> host tensors out.
+    '''
+    as_list = src_offsets is None and dst_offsets is None
+    if as_list:
+        frames = list(distance)
+        if not len(frames) == len(src_scores) == len(src_tags) == len(dst_tags):
+            raise ValueError("distance, scores and tags should hold the same number of frames")
+        if not frames:
+            return []
+        numpy_in = isinstance(frames[0], np.ndarray)
+        dl = [_as_tensor(d, torch.float32) for d in frames]
+        if any(d.dim() != 2 for d in dl):
+            raise ValueError("distance should be an NxM matrix")
+        odev = dl[0].device
+        src_off, dst_off = _frame_offsets(lens=[d.shape[0] for d in dl]), _frame_offsets(lens=[d.shape[1] for d in dl])
+        dist_off = _block_offsets(src_off, dst_off)
+        d = _c.to_device(torch.cat([x.reshape(-1) for x in dl]))
+        cat = lambda xs, dt: torch.cat([_as_tensor(x, dt).reshape(-1) for x in xs])  # noqa: E731
+        scores, st, dt_ = cat(src_scores, torch.float64), cat(src_tags, torch.int32), cat(dst_tags, torch.int32)
+    else:
+        if src_offsets is None or dst_offsets is None:
+            raise ValueError("packed distances need the frame offsets")
+        d, given = distance
+        numpy_in = isinstance(d, np.ndarray)
+        d = _as_tensor(d, torch.float32)
+        odev = d.device
+        d = _c.to_device(d).reshape(-1)
+        src_off, dst_off = _frame_offsets(src_offsets), _frame_offsets(dst_offsets)
+        if src_off.numel() != dst_off.numel():
+            raise ValueError("Numbers of frames in the offsets are inconsistent!")
+        dist_off = _block_offsets(src_off, dst_off)
+        if not torch.equal(_frame_offsets(given), dist_off) or int(dist_off[-1]) != d.numel():
+            raise ValueError("distance blocks do not match the frame offsets")
+        scores, st, dt_ = _as_tensor(src_scores, torch.float64).reshape(-1), _as_tensor(src_tags, torch.int32), _as_tensor(dst_tags, torch.int32)
+    dev = d.device
+    nframes, total_src, total_dst = src_off.numel() - 1, int(src_off[-1]), int(dst_off[-1])
+    if len(scores) != total_src or len(st) != total_src or len(dt_) != total_dst:
+        raise ValueError("scores / tags do not match the distance matrix")
+    thr = _as_tensor(thresholds, torch.float32)
+    single = thr.dim() == 1
+    thr = (thr.reshape(1, -1) if single else thr).to(dev).contiguous()
+    T, ncat = thr.shape
+    scores, st, dt_ = scores.to(dev).contiguous(), st.to(dev).contiguous(), dt_.to(dev).contiguous()
+    n_f, m_f = src_off[1:] - src_off[:-1], dst_off[1:] - dst_off[:-1]
+    max_dst = int(m_f.max()) if nframes else 0
+    sa = torch.full((T, total_src), -1, dtype=torch.int32, device=dev)
+    da = torch.full((T, total_dst), -1, dtype=torch.int32, device=dev)
+    if max_dst > 4096:   # the kernel's taken bitmask holds 4096 destinations
+        for f in range(nframes):
+            s0, s1, d0, d1 = int(src_off[f]), int(src_off[f + 1]), int(dst_off[f]), int(dst_off[f + 1])
+            sa[:, s0:s1], da[:, d0:d1] = match_greedy(d[int(dist_off[f]):int(dist_off[f + 1])].view(s1 - s0, d1 - d0), scores[s0:s1], st[s0:s1],
+                                                      dt_[d0:d1], thr)
+    elif T and d.numel():
+        offs = torch.cat([src_off, dst_off, dist_off]).to(dev, non_blocking=True)   # one copy of the three offset arrays
+        os_, od_, odd = offs[:nframes + 1], offs[nframes + 1:2 * nframes + 2], offs[2 * nframes + 2:]
+        order = _frame_score_order(scores, os_, nframes)
+        with torch.cuda.device(dev):
+            stt = _c.match_greedy_batch(_c.ptr(d), _c.ptr(odd), _c.ptr(os_), _c.ptr(od_), nframes, max_dst, _c.ptr(order), _c.ptr(st), _c.ptr(dt_),
+                                        _c.ptr(thr), T, ncat, _c.ptr(sa), _c.ptr(da), _c.stream_ptr())
+        _c.check(stt, "match_greedy_batch")
+    if odev.type != "cuda" or numpy_in:
+        sa, da = sa.cpu(), da.cpu()
+    if numpy_in:
+        sa, da = sa.numpy(), da.numpy()
+    if not as_list:
+        return (sa[0], da[0]) if single else (sa, da)
+    out = []
+    for f in range(nframes):
+        a, b = sa[:, int(src_off[f]):int(src_off[f + 1])], da[:, int(dst_off[f]):int(dst_off[f + 1])]
+        out.append((a[0], b[0]) if single else (a, b))
+    return out

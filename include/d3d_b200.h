@@ -130,6 +130,35 @@ int d3d_iou3d_distance_f32(const float *boxes1, int64_t n, const float *boxes2, 
 int d3d_match_greedy_f32(const float *dist, int64_t n, int64_t m, int64_t ld, const int32_t *src_order, const int32_t *src_tag,
                          const int32_t *dst_tag, const float *thresholds, int32_t nsets, int32_t ncat, int32_t *src_assign,
                          int32_t *dst_assign, void *stream);
+/* Frame-batched evaluator distance matrix and matching (the detection evaluator runs both once per frame of a validation set).
+ * Frames are packed back to back: boxes1 f32[total1,7] / boxes2 f32[total2,7] with DEVICE offsets1 / offsets2 i64[nframes+1]
+ * (frame f owns rows [offsets[f], offsets[f+1]), n_f and m_f of them).  dist_offsets DEVICE i64[nframes+1]: frame f's block is the
+ * row-major [n_f, m_f] matrix at dist + dist_offsets[f] (leading dimension m_f); the caller chooses the layout, usually the running sum
+ * of n_f * m_f.  max_frame1 / max_frame2: HARD UPPER BOUNDS of n_f / m_f (0 = unknown, assume total1 / total2); they size the launch
+ * grid, and the part of a frame beyond them is not written.  Per frame, the block equals d3d_iou3d_distance_f32 on that frame bit for bit,
+ * for rotated != 0 and rotated == 0: the frames run the same tile body, reject test and clip.  One prep launch per box set and one
+ * distance launch for the whole batch (rotated == 0: one per 65535 rows of the largest frame).  nframes == 0 or an empty box set: no-op.
+ * Negative sizes: D3D_ERR_INVALID_ARGUMENT; workspace below d3d_iou3d_distance_batch_workspace_bytes: D3D_ERR_WORKSPACE;
+ * nframes > 2^31 - 1, rotated frames over 65535 tiles (64 rows / 128 columns) or axis-aligned frames over 65535 x 1024 columns:
+ * D3D_ERR_UNSUPPORTED. */
+size_t d3d_iou3d_distance_batch_workspace_bytes(int64_t total1, int64_t total2, int64_t nframes);
+int d3d_iou3d_distance_batch_f32(const float *boxes1, int64_t total1, const int64_t *offsets1, const float *boxes2, int64_t total2,
+                                 const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int rotated,
+                                 const int64_t *dist_offsets, float *dist, void *workspace, size_t workspace_bytes, void *stream);
+/* d3d_match_greedy_f32 on every frame of a packed batch in one launch: dist and dist_offsets as written by d3d_iou3d_distance_batch_f32,
+ * src_offsets / dst_offsets DEVICE i64[nframes+1] (total_src = src_offsets[nframes], total_dst = dst_offsets[nframes]).  src_order i32
+ * [total_src] holds, per frame, the FRAME-LOCAL source indices from the best score down; src_tag i32[total_src] / dst_tag i32[total_dst]
+ * are packed like the boxes; thresholds f32[nsets, ncat] are shared by all frames.  Outputs src_assign i32[nsets, total_src] /
+ * dst_assign i32[nsets, total_dst]: the frame-local partner index or -1.  Per frame and threshold set, the result equals
+ * d3d_match_greedy_f32 on the frame's block (d <= threshold, so a NaN distance never matches; equal distances go to the lower
+ * destination index; a source whose tag is outside [0, ncat) matches nothing).  One warp per (frame, threshold set) with its taken flags
+ * as a bitmask in shared memory.  max_frame_dst: HARD UPPER BOUND of the frames' destination counts; more than 4096:
+ * D3D_ERR_UNSUPPORTED (call d3d_match_greedy_f32 per frame); a frame over 4096 destinations despite the bound stays unmatched.
+ * Negative sizes or ncat < 1: D3D_ERR_INVALID_ARGUMENT; nframes == 0 or nsets == 0: no-op. */
+int d3d_match_greedy_batch_f32(const float *dist, const int64_t *dist_offsets, const int64_t *src_offsets, const int64_t *dst_offsets,
+                               int64_t nframes, int64_t max_frame_dst, const int32_t *src_order, const int32_t *src_tag,
+                               const int32_t *dst_tag, const float *thresholds, int32_t nsets, int32_t ncat, int32_t *src_assign,
+                               int32_t *dst_assign, void *stream);
 /* Point-in-rotated-box mask (SURVEY.md 8(f) row f4): mask u8[m boxes, n points] row-major, 1 where the point lies inside
  * the box.  points [n,2], boxes [m,5] (x, y, w, h, r).  Replaces crop_2dr (reference d3d/box/utils.h:45, utils.cpp:10-47,
  * bound at d3d/box/impl.cpp:26 and called by box2dr_crop / box3dp_crop, d3d/box/__init__.py:278-314); the reference
