@@ -327,8 +327,9 @@ def box3dp_crop(points, boxes, project_axis=2):
 
 class PDist2DR(torch.autograd.Function):
     """Differentiable signed distance from points to rotated boxes (reference d3d/box/__init__.py:149-166 over pdist2dr_forward /
-    pdist2dr_backward[_cuda], d3d/box/dist.h:7-23).  Returns T[M boxes, N points], positive inside -- the layout of the native function
-    (and of box2dr_crop).  The reference's wrapper hands (boxes, points) to a native function declared (points, boxes) and cannot run."""
+    pdist2dr_backward[_cuda], d3d/box/dist.h:7-23).  Returns T[M boxes, N points]: the signed Euclidean distance to the boundary of the
+    closed rectangle with half extents |w|/2, |h|/2 turned by r, positive inside -- the layout of the native function (and of
+    box2dr_crop).  The reference's wrapper hands (boxes, points) to a native function declared (points, boxes) and cannot run."""
     @staticmethod
     def forward(ctx, points, boxes):
         code = _c.dtype_code(points.dtype)
@@ -408,9 +409,13 @@ def box3dr_pdist(points, boxes, project_axis=2):
         raise ValueError("The projection axis can only be 0-x, 1-y and 2-z!")
     dist_2d = box2dr_pdist(points_2d, boxes_2d)
     dist_p = seg1d_pdist(points[:, project_axis], boxes[:, [project_axis, 3 + project_axis]]).to(dist_2d.device)
+    # on an edge of the prism (both terms 0) the square root has no derivative: take it of 1 there, so that its backward, which runs
+    # for every pair whichever branch is selected, multiplies by a finite number instead of 0 * inf = NaN
+    sq = dist_2d.square() + dist_p.square()
+    corner = torch.where(sq > 0, -torch.sqrt(torch.where(sq > 0, sq, torch.ones_like(sq))), torch.zeros_like(sq))
     return torch.where(dist_p > 0,
                        torch.where(dist_2d > 0, torch.min(dist_p, dist_2d), dist_2d),
-                       torch.where(dist_2d > 0, dist_p, -torch.sqrt(dist_2d.square() + dist_p.square())))
+                       torch.where(dist_2d > 0, dist_p, corner))
 
 
 def _dist3d_input(boxes):

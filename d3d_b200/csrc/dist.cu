@@ -1,86 +1,39 @@
 // dist.cu -- signed distance from points to rotated boxes (SURVEY.md 8(f) row f4, second half).
 //
 // Replaces pdist2dr_forward / pdist2dr_backward[_cuda] (reference d3d/box/dist.h:7-23, dist.cpp:11-110, dist_cuda.cu:9-81) behind
-// box2dr_pdist / box3dr_pdist (d3d/box/__init__.py:149-166, 330-381).  The value follows dgal operation by operation (vertices
-// geometry.hpp:417-429, line :331-336, projection parameter :372-380 with its three branches, segment distance :453-474, polygon
-// distance :482-497: positive inside, the first edge wins a tie), so fp64 results agree with the reference to rounding of hypot.
-// The backward is the analytic gradient of that value: along the edge normal when the closest feature is an edge, along the ray
-// to the vertex when it is a vertex; box gradients are reduced per box inside the CTA and leave with one atomic per field.
+// box2dr_pdist / box3dr_pdist (d3d/box/__init__.py:149-166, 330-381).  The value is the signed Euclidean distance to the box's boundary,
+// positive inside, computed in the box's own frame (dist.cuh) -- not dgal's line-by-line distance(Poly2, Point2), whose sign at points on
+// the line through an edge and whose projection at headings of pi / 2 are wrong (DESIGN.md section 2, deviation P1).  The backward is the
+// analytic gradient of that value; box gradients are reduced per box inside the CTA and leave with one atomic per field.
 #include "common.cuh"
-#include <math.h>
+#include "dist.cuh"
 
 namespace d3d {
 
-template <typename T> struct Quad { T vx[4], vy[4]; };
-
-template <typename T>
-__device__ __forceinline__ Quad<T> pd_quad(const T *b)
-{
-    const T x = b[0], y = b[1], w = b[2], h = b[3], r = b[4];
-    const T sr = sin(r), cr = cos(r);
-    const T dxsin = w * sr / 2, dxcos = w * cr / 2, dysin = h * sr / 2, dycos = h * cr / 2;
-    Quad<T> q;
-    q.vx[0] = x - dxcos + dysin; q.vy[0] = y - dxsin - dycos;
-    q.vx[1] = x + dxcos + dysin; q.vy[1] = y + dxsin - dycos;
-    q.vx[2] = x + dxcos - dysin; q.vy[2] = y + dxsin + dycos;
-    q.vx[3] = x - dxcos - dysin; q.vy[3] = y - dxsin + dycos;
-    return q;
-}
-
-template <typename T>
-__device__ __forceinline__ T pd_t(T a, T b, T c, T x, T y)
-{
-    if (b == 0) return (1 - y) / a;
-    else if (a == 0) return (x - 1) / b;
-    else return (b * x - a * y - a * (a + c) / b - b) / (a * a + b * b);
-}
-
-// signed distance to the segment (x1,y1)->(x2,y2); *feat: 0 interior of the edge, 1 the start vertex, 2 the end vertex
-template <typename T>
-__device__ __forceinline__ T pd_seg(T x1, T y1, T x2, T y2, T px, T py, int *feat)
-{
-    const T a = y2 - y1, b = x1 - x2, c = x2 * y1 - x1 * y2;
-    const T t = pd_t(a, b, c, px, py);
-    const T sign = a * px + b * py + c;
-    if (t < pd_t(a, b, c, x2, y2)) { const T d = hypot(px - x2, py - y2); *feat = 2; return sign > 0 ? d : -d; }
-    else if (t > pd_t(a, b, c, x1, y1)) { const T d = hypot(px - x1, py - y1); *feat = 1; return sign > 0 ? d : -d; }
-    *feat = 0;
-    return sign / hypot(a, b);
-}
-
-template <typename T>
-__device__ __forceinline__ T pd_poly(const Quad<T> &q, T px, T py, int *idx, int *feat)
-{
-    T dmin = -pd_seg(q.vx[3], q.vy[3], q.vx[0], q.vy[0], px, py, feat);
-    *idx = 3;
-#pragma unroll
-    for (int k = 1; k < 4; k++) {
-        int f;
-        const T dl = -pd_seg(q.vx[k - 1], q.vy[k - 1], q.vx[k], q.vy[k], px, py, &f);
-        if (fabs(dl) < fabs(dmin)) { dmin = dl; *idx = k - 1; *feat = f; }
-    }
-    return dmin;
-}
-
 constexpr int PD_THREADS = 256;
-constexpr int PD_BOXES = 8;   // boxes per CTA (their vertices live in shared memory)
+constexpr int PD_BOXES = 8;          // boxes per tile (their frames live in shared memory)
+constexpr int64_t PD_MAX_GY = 65535; // grid.y limit: larger box counts stride over their tiles
 
 template <typename T>
 __global__ void __launch_bounds__(PD_THREADS) pdist_fwd_kernel(const T *__restrict__ pts, int64_t n, const T *__restrict__ boxes, int64_t m, T *__restrict__ dist,
                                                                uint8_t *__restrict__ iedge)
 {
-    __shared__ Quad<T> sq[PD_BOXES];
-    const int64_t b0 = (int64_t)blockIdx.y * PD_BOXES;
-    if (threadIdx.x < PD_BOXES && b0 + threadIdx.x < m) sq[threadIdx.x] = pd_quad<T>(boxes + 5 * (b0 + threadIdx.x));
-    __syncthreads();
+    __shared__ PBox<T> sb[PD_BOXES];
     const int64_t j = (int64_t)blockIdx.x * PD_THREADS + threadIdx.x;
-    if (j >= n) return;
-    const T px = pts[2 * j], py = pts[2 * j + 1];
-    for (int k = 0; k < PD_BOXES && b0 + k < m; k++) {
-        int idx, feat;
-        const T d = pd_poly<T>(sq[k], px, py, &idx, &feat);
-        dist[(b0 + k) * n + j] = d;
-        if (iedge) iedge[(b0 + k) * n + j] = (uint8_t)idx;
+    const bool in = j < n;
+    const T px = in ? pts[2 * j] : T(0), py = in ? pts[2 * j + 1] : T(0);
+    for (int64_t b0 = (int64_t)blockIdx.y * PD_BOXES; b0 < m; b0 += (int64_t)gridDim.y * PD_BOXES) {
+        if (threadIdx.x < PD_BOXES && b0 + threadIdx.x < m) sb[threadIdx.x] = pd_box<T>(boxes + 5 * (b0 + threadIdx.x));
+        __syncthreads();
+        if (in) {
+            for (int k = 0; k < PD_BOXES && b0 + k < m; k++) {
+                int e;
+                const T d = pd_pair<T, false>(sb[k], px, py, &e, T(0), nullptr, nullptr);
+                dist[(b0 + k) * n + j] = d;
+                if (iedge) iedge[(b0 + k) * n + j] = (uint8_t)e;
+            }
+        }
+        __syncthreads();
     }
 }
 
@@ -91,76 +44,41 @@ template <typename T>
 __global__ void __launch_bounds__(PD_THREADS) pdist_bwd_kernel(const T *__restrict__ pts, int64_t n, const T *__restrict__ boxes, int64_t m, const T *__restrict__ grad,
                                                                T *__restrict__ grad_boxes, T *__restrict__ grad_pts)
 {
-    __shared__ Quad<T> sq[PD_BOXES];
-    __shared__ T sbox[PD_BOXES][5];
+    __shared__ PBox<T> sb[PD_BOXES];
     __shared__ T sacc[PD_BOXES][5];
-    const int64_t b0 = (int64_t)blockIdx.y * PD_BOXES;
-    if (threadIdx.x < PD_BOXES && b0 + threadIdx.x < m) {
-        sq[threadIdx.x] = pd_quad<T>(boxes + 5 * (b0 + threadIdx.x));
-        for (int k = 0; k < 5; k++) { sbox[threadIdx.x][k] = boxes[5 * (b0 + threadIdx.x) + k]; sacc[threadIdx.x][k] = T(0); }
-    }
-    __syncthreads();
     const int64_t j = (int64_t)blockIdx.x * PD_THREADS + threadIdx.x;
     const bool in = j < n;
     const T px = in ? pts[2 * j] : T(0), py = in ? pts[2 * j + 1] : T(0);
-    T gpx = 0, gpy = 0;
+    T gp[2] = {0, 0};
     const unsigned lane = threadIdx.x & 31u;
-    for (int k = 0; k < PD_BOXES && b0 + k < m; k++) {
-        T gb[5] = {0, 0, 0, 0, 0};
-        if (in) {
-            const Quad<T> &q = sq[k];
-            int idx, feat;
-            pd_poly<T>(q, px, py, &idx, &feat);
-            const T g = grad[(b0 + k) * n + j];
-            const int i1 = idx, i2 = (idx + 1) & 3;   // the edge i1 -> i2
-            const T x1 = q.vx[i1], y1 = q.vy[i1], x2 = q.vx[i2], y2 = q.vy[i2];
-            T gv[4][2] = {{0, 0}, {0, 0}, {0, 0}, {0, 0}};   // d(distance)/d(vertex)
-            T dpx, dpy;
-            if (feat == 0) {   // D = -s / L, s = a px + b py + c, L = |v2 - v1|
-                const T a = y2 - y1, b = x1 - x2, c = x2 * y1 - x1 * y2;
-                const T s = a * px + b * py + c, L = hypot(a, b), iL = 1 / L, iL2 = iL * iL;
-                dpx = -a * iL; dpy = -b * iL;
-                // ds/dv and dL/dv
-                const T sx1 = py - y2, sy1 = x2 - px, sx2 = y1 - py, sy2 = px - x1;
-                const T Lx1 = b * iL, Ly1 = -a * iL, Lx2 = -b * iL, Ly2 = a * iL;
-                gv[i1][0] = -(sx1 * L - s * Lx1) * iL2; gv[i1][1] = -(sy1 * L - s * Ly1) * iL2;
-                gv[i2][0] = -(sx2 * L - s * Lx2) * iL2; gv[i2][1] = -(sy2 * L - s * Ly2) * iL2;
-            } else {           // D = sigma |p - v|, sigma = -sign(s)
-                const T a = y2 - y1, b = x1 - x2, c = x2 * y1 - x1 * y2;
-                const T s = a * px + b * py + c;
-                const int iv = feat == 1 ? i1 : i2;
-                const T dx = px - q.vx[iv], dy = py - q.vy[iv], r = hypot(dx, dy);
-                const T sg = s > 0 ? T(-1) : T(1), ir = r > 0 ? sg / r : T(0);
-                dpx = dx * ir; dpy = dy * ir;
-                gv[iv][0] = -dpx; gv[iv][1] = -dpy;
+    for (int64_t b0 = (int64_t)blockIdx.y * PD_BOXES; b0 < m; b0 += (int64_t)gridDim.y * PD_BOXES) {
+        if (threadIdx.x < PD_BOXES && b0 + threadIdx.x < m) {
+            sb[threadIdx.x] = pd_box<T>(boxes + 5 * (b0 + threadIdx.x));
+            for (int f = 0; f < 5; f++) sacc[threadIdx.x][f] = T(0);
+        }
+        __syncthreads();
+        for (int k = 0; k < PD_BOXES && b0 + k < m; k++) {
+            T gb[5] = {0, 0, 0, 0, 0};
+            if (in) {
+                int e;
+                pd_pair<T, true>(sb[k], px, py, &e, grad[(b0 + k) * n + j], gp, gb);
             }
-            gpx += g * dpx; gpy += g * dpy;
-            // vertices -> (x, y, w, h, r): v_k = c + s_k (w/2) u + t_k (h/2) v, u = (cos r, sin r), v = (-sin r, cos r)
-            const T w = sbox[k][2], h = sbox[k][3], sr = sin(sbox[k][4]), cr = cos(sbox[k][4]);
-            const T sk[4] = {-1, 1, 1, -1}, tk[4] = {-1, -1, 1, 1};
 #pragma unroll
-            for (int v = 0; v < 4; v++) {
-                const T gx = g * gv[v][0], gy = g * gv[v][1];
-                gb[0] += gx; gb[1] += gy;
-                gb[2] += sk[v] * T(0.5) * (gx * cr + gy * sr);
-                gb[3] += tk[v] * T(0.5) * (-gx * sr + gy * cr);
-                gb[4] += gx * (-sk[v] * T(0.5) * w * sr - tk[v] * T(0.5) * h * cr) + gy * (sk[v] * T(0.5) * w * cr - tk[v] * T(0.5) * h * sr);
+            for (int f = 0; f < 5; f++) {
+                T v = gb[f];
+#pragma unroll
+                for (int d = 16; d; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+                if (lane == 0 && v != T(0)) pd_atomic_add(&sacc[k][f], v);
             }
         }
-#pragma unroll
-        for (int f = 0; f < 5; f++) {
-            T v = gb[f];
-#pragma unroll
-            for (int d = 16; d; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-            if (lane == 0 && v != T(0)) pd_atomic_add(&sacc[k][f], v);
+        __syncthreads();
+        if (threadIdx.x < PD_BOXES * 5) {
+            const int k = threadIdx.x / 5, f = threadIdx.x % 5;
+            if (b0 + k < m && sacc[k][f] != T(0)) pd_atomic_add(grad_boxes + 5 * (b0 + k) + f, sacc[k][f]);
         }
+        __syncthreads();
     }
-    if (in) { pd_atomic_add(grad_pts + 2 * j, gpx); pd_atomic_add(grad_pts + 2 * j + 1, gpy); }
-    __syncthreads();
-    if (threadIdx.x < PD_BOXES * 5) {
-        const int k = threadIdx.x / 5, f = threadIdx.x % 5;
-        if (b0 + k < m && sacc[k][f] != T(0)) pd_atomic_add(grad_boxes + 5 * (b0 + k) + f, sacc[k][f]);
-    }
+    if (in) { pd_atomic_add(grad_pts + 2 * j, gp[0]); pd_atomic_add(grad_pts + 2 * j + 1, gp[1]); }
 }
 
 template <typename T>
@@ -169,8 +87,7 @@ static int pdist_fwd(const T *pts, int64_t n, const T *boxes, int64_t m, T *dist
     if (n < 0 || m < 0) return D3D_ERR_INVALID_ARGUMENT;
     if (n == 0 || m == 0) return D3D_OK;
     if (!pts || !boxes || !dist) return D3D_ERR_INVALID_ARGUMENT;
-    const int64_t gy = cdiv(m, PD_BOXES);
-    if (gy > 65535) return D3D_ERR_INVALID_ARGUMENT;
+    const int64_t tiles = cdiv(m, PD_BOXES), gy = tiles < PD_MAX_GY ? tiles : PD_MAX_GY;
     pdist_fwd_kernel<T><<<dim3((unsigned)cdiv(n, PD_THREADS), (unsigned)gy), PD_THREADS, 0, st>>>(pts, n, boxes, m, dist, iedge);
     D3D_LAUNCHED();
     return D3D_OK;
@@ -182,8 +99,7 @@ static int pdist_bwd(const T *pts, int64_t n, const T *boxes, int64_t m, const T
     if (n < 0 || m < 0) return D3D_ERR_INVALID_ARGUMENT;
     if (n == 0 || m == 0) return D3D_OK;
     if (!pts || !boxes || !grad || !grad_boxes || !grad_pts) return D3D_ERR_INVALID_ARGUMENT;
-    const int64_t gy = cdiv(m, PD_BOXES);
-    if (gy > 65535) return D3D_ERR_INVALID_ARGUMENT;
+    const int64_t tiles = cdiv(m, PD_BOXES), gy = tiles < PD_MAX_GY ? tiles : PD_MAX_GY;
     pdist_bwd_kernel<T><<<dim3((unsigned)cdiv(n, PD_THREADS), (unsigned)gy), PD_THREADS, 0, st>>>(pts, n, boxes, m, grad, grad_boxes, grad_pts);
     D3D_LAUNCHED();
     return D3D_OK;

@@ -123,6 +123,84 @@ def box3dr_pdist(points, boxes, project_axis=2):
     return np.where(dp > 0, np.where(d2 > 0, np.minimum(dp, d2), d2), np.where(d2 > 0, dp, -np.sqrt(d2 * d2 + dp * dp))).astype(d2.dtype)
 
 
+def _pdist_frame(dx, dy, w, h, r, return_iedge=False):
+    """signed distance (positive inside) of the local offsets (dx, dy) = point - centre to the closed rectangle of half extents
+    |w| / 2, |h| / 2 turned by r, all float64 arrays that broadcast.  The offset is turned into the box's frame; the magnitude is the
+    least distance to its four edges as segments between the corners of pd_quad's order, (-w/2, -h/2), (w/2, -h/2), (w/2, h/2),
+    (-w/2, h/2); the sign comes from the containment test.  The edge index is the first minimum in the loop order 3, 0, 1, 2."""
+    c, s = np.cos(r), np.sin(r)
+    qx, qy = c * dx + s * dy, c * dy - s * dx
+    vx = [-w / 2, w / 2, w / 2, -w / 2]
+    vy = [-h / 2, -h / 2, h / 2, h / 2]
+    seg = []
+    for k in range(4):   # edge k: v_k -> v_k+1
+        ax, ay, bx, by = vx[k], vy[k], vx[(k + 1) % 4], vy[(k + 1) % 4]
+        ex, ey = bx - ax, by - ay
+        ll = ex * ex + ey * ey
+        with np.errstate(invalid="ignore", divide="ignore"):
+            t = np.where(ll > 0, np.clip(((qx - ax) * ex + (qy - ay) * ey) / np.where(ll > 0, ll, 1), 0, 1), 0)
+        cx, cy = np.where(t >= 1, bx, ax + t * ex), np.where(t >= 1, by, ay + t * ey)   # the corners exactly: ties at corners stay ties
+        seg.append(np.hypot(qx - cx, qy - cy))
+    order = (3, 0, 1, 2)
+    allseg = np.stack([seg[k] for k in order])
+    dmin = allseg.min(0)
+    inside = (np.abs(qx) <= np.abs(w) / 2) & (np.abs(qy) <= np.abs(h) / 2)
+    d = np.where(inside, dmin, -dmin)
+    if return_iedge:
+        return d, np.asarray(order, np.uint8)[allseg.argmin(0)]
+    return d
+
+
+def pdist2dr_local(points, boxes, return_iedge=False):
+    """Signed point-to-rotated-box distance T[M boxes, N points] (positive inside, zero on the boundary) in float64 with each pair moved
+    into its box's frame: p - c is taken in float64 (exact for widened float32 inputs, and for float64 points near their box) and turned
+    by -r.  The geometric truth that box2dr_pdist computes; pdist2dr above restates the reference, which differs from it on the lines
+    through edges, at headings of pi / 2 and far from the origin (SURVEY.md 8(c), P1).  With return_iedge, also the index k of the edge
+    v_k -> v_k+1 that realises the distance (ties: first of 3, 0, 1, 2)."""
+    p, b = np.asarray(points, np.float64), np.asarray(boxes, np.float64)
+    col = lambda k: b[:, k:k + 1]  # noqa: E731
+    return _pdist_frame(p[None, :, 0] - col(0), p[None, :, 1] - col(1), col(2), col(3), col(4), return_iedge)
+
+
+def pdist2dr_grad_local(points, boxes, h=1e-4, smooth_tol=1e-9):
+    """Per-pair derivatives of pdist2dr_local by five-point differences, taken in the box's frame: returns (value [M, N],
+    dp [M, N, 2] = d value / d points[j], db [M, N, 5] = d value / d boxes[i], smooth bool [M, N]).  A pair is smooth when the stencils at
+    h and h / 2 agree to `smooth_tol` in all seven derivatives; elsewhere (a tie between two edges inside, the boundary, a zero extent)
+    the value has a kink within the stencil and no derivative to compare with."""
+    p, b = np.asarray(points, np.float64), np.asarray(boxes, np.float64)
+    m, n = len(b), len(p)
+    dx, dy = p[None, :, 0] - b[:, 0:1], p[None, :, 1] - b[:, 1:2]
+    base = [dx, dy, np.zeros((m, 1)), np.zeros((m, 1)), b[:, 2:3], b[:, 3:4], b[:, 4:5]]   # point x, y, box x, y, w, h, r
+
+    def f(args):
+        return _pdist_frame(args[0] - args[2], args[1] - args[3], args[4], args[5], args[6])
+
+    val = f(base)
+    der, smooth = np.empty((m, n, 7)), np.ones((m, n), bool)
+    for k in range(7):
+        est = []
+        for hh in (h, h / 2):
+            fs = []
+            for s in (-2, -1, 1, 2):
+                a = list(base)
+                a[k] = a[k] + s * hh
+                fs.append(f(a))
+            est.append((fs[0] - 8 * fs[1] + 8 * fs[2] - fs[3]) / (12 * hh))
+        der[..., k] = est[0]
+        smooth &= np.abs(est[0] - est[1]) <= smooth_tol
+    return val, der[..., :2], der[..., 2:], smooth
+
+
+def box3dr_pdist_local(points, boxes, project_axis=2):
+    """box3dr_pdist in float64 from the local 2-D term (pdist2dr_local) and the signed distance along the projection axis: the signed
+    distance to the boundary of the prism, positive inside."""
+    p, b = np.asarray(points, np.float64), np.asarray(boxes, np.float64)
+    ax2 = {0: ([1, 2], [1, 2, 4, 5, 6]), 1: ([0, 2], [0, 2, 3, 5, 6]), 2: ([0, 1], [0, 1, 3, 4, 6])}[project_axis]
+    d2 = pdist2dr_local(p[:, ax2[0]], b[:, ax2[1]])
+    dp = np.abs(b[:, 3 + project_axis])[:, None] / 2 - np.abs(p[None, :, project_axis] - b[:, project_axis][:, None])
+    return np.where(dp > 0, np.where(d2 > 0, np.minimum(dp, d2), d2), np.where(d2 > 0, dp, -np.hypot(d2, dp)))
+
+
 def box3dp_crop(points, boxes, project_axis=2):
     """d3d/box/__init__.py:289-314: 2-D crop of the projection & the open interval test along the projection axis."""
     ax2 = {0: ([1, 2], [1, 2, 4, 5, 6]), 1: ([0, 2], [0, 2, 3, 5, 6]), 2: ([0, 1], [0, 1, 3, 4, 6])}[project_axis]

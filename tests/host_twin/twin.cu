@@ -1,7 +1,8 @@
-// twin.cu -- TEST INFRASTRUCTURE: compiles the product's clip math (d3d_b200/csrc/geom.cuh) and the pair math of the
-// differentiable IoU family (d3d_b200/csrc/iou_grad.cuh) as HOST code so the algorithm can be checked against the CPU
-// oracle on a machine without a GPU.  Nothing in the product loads this library.
+// twin.cu -- TEST INFRASTRUCTURE: compiles the product's clip math (d3d_b200/csrc/geom.cuh), the pair math of the
+// differentiable IoU family (d3d_b200/csrc/iou_grad.cuh) and of the point-to-box distance (d3d_b200/csrc/dist.cuh) as HOST
+// code so the algorithm can be checked against the CPU oracle on a machine without a GPU.  Nothing in the product loads this library.
 #include "../../d3d_b200/csrc/geom.cuh"
+#include "../../d3d_b200/csrc/dist.cuh"
 #include "../../d3d_b200/csrc/iou_grad.cuh"
 using namespace d3d;
 template <typename T> static void run(const T *b1, long n, const T *b2, long m, T *out, int aabb)
@@ -55,3 +56,25 @@ extern "C" void twin_iou_ex_f32(const float *b1, long n, const float *b2, long m
 { run_ex_type<float>(b1, n, b2, m, type, up, out, g1, g2); }
 extern "C" void twin_iou_ex_f64(const double *b1, long n, const double *b2, long m, int type, const double *up, double *out, double *g1, double *g2)
 { run_ex_type<double>(b1, n, b2, m, type, up, out, g1, g2); }
+
+// the point-to-box distance as dist.cu runs it: values and edge indices [m boxes, n points] as pdist_fwd_kernel computes them and, for
+// the upstream gradient `up` [m, n], the gradient sums gp [n, 2] and gb [m, 5] of pdist_bwd_kernel
+template <typename T> static void run_pd(const T *pts, long n, const T *boxes, long m, const T *up, T *out, unsigned char *edge, T *gp, T *gb)
+{
+    for (long j = 0; j < 2 * n; j++) gp[j] = T(0);
+    for (long i = 0; i < m; i++) {
+        const PBox<T> b = pd_box<T>(boxes + 5 * i);
+        T acc[5] = {0, 0, 0, 0, 0};
+        for (long j = 0; j < n; j++) {
+            int e;
+            out[i * n + j] = pd_pair<T, false>(b, pts[2 * j], pts[2 * j + 1], &e, T(0), nullptr, nullptr);
+            edge[i * n + j] = (unsigned char)e;
+            pd_pair<T, true>(b, pts[2 * j], pts[2 * j + 1], &e, up[i * n + j], gp + 2 * j, acc);
+        }
+        for (int k = 0; k < 5; k++) gb[5 * i + k] = acc[k];
+    }
+}
+extern "C" void twin_pdist_f32(const float *pts, long n, const float *boxes, long m, const float *up, float *out, unsigned char *edge, float *gp, float *gb)
+{ run_pd<float>(pts, n, boxes, m, up, out, edge, gp, gb); }
+extern "C" void twin_pdist_f64(const double *pts, long n, const double *boxes, long m, const double *up, double *out, unsigned char *edge, double *gp, double *gb)
+{ run_pd<double>(pts, n, boxes, m, up, out, edge, gp, gb); }
