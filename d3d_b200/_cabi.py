@@ -62,6 +62,12 @@ _pd_sig = [_vp, _i64, _vp, _i64, _vp, _vp, _vp]
 pdist2dr = {F32: _sig("d3d_pdist2dr_f32", C.c_int, _pd_sig), F64: _sig("d3d_pdist2dr_f64", C.c_int, _pd_sig)}
 _pdb_sig = [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp]
 pdist2dr_backward = {F32: _sig("d3d_pdist2dr_backward_f32", C.c_int, _pdb_sig), F64: _sig("d3d_pdist2dr_backward_f64", C.c_int, _pdb_sig)}
+crop_grid_min_pairs = _sig("d3d_crop2dr_grid_min_pairs", _i64, [])
+crop_batch_workspace_bytes = _sig("d3d_crop2dr_batch_workspace_bytes", _sz, [_i64, C.c_int])
+_pbb_sig = [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i64, _i64, C.c_int, _vp]   # packed points / boxes, offsets, bounds, axis, out offsets
+crop2dr_batch = {k: _sig(f"d3d_crop2dr_batch_{s}", C.c_int, _pbb_sig + [_vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+pdist2dr_batch = {k: _sig(f"d3d_pdist2dr_batch_{s}", C.c_int, _pbb_sig + [_vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+pdist2dr_batch_backward = {k: _sig(f"d3d_pdist2dr_batch_backward_{s}", C.c_int, _pbb_sig + [_vp, _vp, _vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 _iex_sig = [_vp, _i64, _vp, _i64, _vp, _i64, _vp]
 giou2dr = {F32: _sig("d3d_giou2dr_f32", C.c_int, _iex_sig), F64: _sig("d3d_giou2dr_f64", C.c_int, _iex_sig)}
 diou2dr = {F32: _sig("d3d_diou2dr_f32", C.c_int, _iex_sig), F64: _sig("d3d_diou2dr_f64", C.c_int, _iex_sig)}

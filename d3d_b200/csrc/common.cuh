@@ -42,6 +42,28 @@ struct Arena {
     bool ok() const { return off <= cap; }
 };
 
+// explicitly rounded arithmetic, never contracted into an FMA: results that must equal code compiled without contraction (the
+// reference's CPU code, torch's elementwise operators) bit for bit
+template <typename T> __device__ __forceinline__ T rn_mul(T a, T b);
+template <> __device__ __forceinline__ float rn_mul<float>(float a, float b) { return __fmul_rn(a, b); }
+template <> __device__ __forceinline__ double rn_mul<double>(double a, double b) { return __dmul_rn(a, b); }
+template <typename T> __device__ __forceinline__ T rn_sub(T a, T b);
+template <> __device__ __forceinline__ float rn_sub<float>(float a, float b) { return __fsub_rn(a, b); }
+template <> __device__ __forceinline__ double rn_sub<double>(double a, double b) { return __dsub_rn(a, b); }
+template <typename T> __device__ __forceinline__ T rn_add(T a, T b);
+template <> __device__ __forceinline__ float rn_add<float>(float a, float b) { return __fadd_rn(a, b); }
+template <> __device__ __forceinline__ double rn_add<double>(double a, double b) { return __dadd_rn(a, b); }
+template <typename T> __device__ __forceinline__ T rn_div2(T a);
+template <> __device__ __forceinline__ float rn_div2<float>(float a) { return __fmul_rn(a, 0.5f); }     // x / 2 is exact
+template <> __device__ __forceinline__ double rn_div2<double>(double a) { return __dmul_rn(a, 0.5); }
+template <typename T> __device__ __forceinline__ T rn_sqrt(T a);
+template <> __device__ __forceinline__ float rn_sqrt<float>(float a) { return __fsqrt_rn(a); }
+template <> __device__ __forceinline__ double rn_sqrt<double>(double a) { return __dsqrt_rn(a); }
+
+// projection of 3-D rows to an axis (box3dp_crop, box3dr_pdist): the plane of the two other axes is point columns (a, b) of [n, 3] and
+// box columns (a, b, 3 + a, 3 + b, 6) of [m, 7] (x, y, z, lx, ly, lz, r)
+__device__ __forceinline__ void proj_plane(int axis, int *a, int *b) { *a = axis == 0 ? 1 : 0; *b = axis == 2 ? 1 : 2; }
+
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31u; }
 __device__ __forceinline__ unsigned lanemask_lt() { unsigned m; asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m)); return m; }
 

@@ -20,25 +20,9 @@ namespace d3d {
 
 template <typename T> struct CropBox { T vx[4], vy[4], minx, maxx, miny, maxy; };
 
-template <typename T> __device__ __forceinline__ T rn_mul(T a, T b);
-template <> __device__ __forceinline__ float rn_mul<float>(float a, float b) { return __fmul_rn(a, b); }
-template <> __device__ __forceinline__ double rn_mul<double>(double a, double b) { return __dmul_rn(a, b); }
-template <typename T> __device__ __forceinline__ T rn_sub(T a, T b);
-template <> __device__ __forceinline__ float rn_sub<float>(float a, float b) { return __fsub_rn(a, b); }
-template <> __device__ __forceinline__ double rn_sub<double>(double a, double b) { return __dsub_rn(a, b); }
-template <typename T> __device__ __forceinline__ T rn_add(T a, T b);
-template <> __device__ __forceinline__ float rn_add<float>(float a, float b) { return __fadd_rn(a, b); }
-template <> __device__ __forceinline__ double rn_add<double>(double a, double b) { return __dadd_rn(a, b); }
-template <typename T> __device__ __forceinline__ T rn_div2(T a);
-template <> __device__ __forceinline__ float rn_div2<float>(float a) { return __fmul_rn(a, 0.5f); }     // x / 2 is exact
-template <> __device__ __forceinline__ double rn_div2<double>(double a) { return __dmul_rn(a, 0.5); }
-
 template <typename T>
-__global__ void __launch_bounds__(256) crop_prep_kernel(const T *__restrict__ boxes, int64_t m, CropBox<T> *__restrict__ recs)
+__device__ __forceinline__ CropBox<T> crop_prep_one(T x, T y, T w, T h, T r)
 {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= m) return;
-    const T x = boxes[5 * i], y = boxes[5 * i + 1], w = boxes[5 * i + 2], h = boxes[5 * i + 3], r = boxes[5 * i + 4];
     T sn, cs;
     if (sizeof(T) == 4) { sn = (T)sinf((float)r); cs = (T)cosf((float)r); } else { sn = (T)sin((double)r); cs = (T)cos((double)r); }
     const T dxsin = rn_div2(rn_mul(w, sn)), dxcos = rn_div2(rn_mul(w, cs)), dysin = rn_div2(rn_mul(h, sn)), dycos = rn_div2(rn_mul(h, cs));
@@ -53,7 +37,15 @@ __global__ void __launch_bounds__(256) crop_prep_kernel(const T *__restrict__ bo
         b.minx = b.vx[k] < b.minx ? b.vx[k] : b.minx; b.maxx = b.vx[k] > b.maxx ? b.vx[k] : b.maxx;
         b.miny = b.vy[k] < b.miny ? b.vy[k] : b.miny; b.maxy = b.vy[k] > b.maxy ? b.vy[k] : b.maxy;
     }
-    recs[i] = b;
+    return b;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) crop_prep_kernel(const T *__restrict__ boxes, int64_t m, CropBox<T> *__restrict__ recs)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    recs[i] = crop_prep_one<T>(boxes[5 * i], boxes[5 * i + 1], boxes[5 * i + 2], boxes[5 * i + 3], boxes[5 * i + 4]);
 }
 
 constexpr int CROP_THREADS = 256, CROP_PPT = 16, CROP_BT = 16;   // points per thread, boxes per CTA
@@ -433,6 +425,123 @@ static int crop_impl(const T *pts, int64_t n, const T *boxes, int64_t m, uint8_t
     return D3D_OK;
 }
 
+// ------------------------------------------------------------------ frame-batched mask
+// Frame f owns points [poff[f], poff[f+1]) and boxes [boff[f], boff[f+1]) of the packed inputs and writes its row-major [m_f, n_f] block
+// at mask + moff[f].  The box records of the whole batch are prepared by one launch; the tile kernel runs crop2dr_kernel's tiles with
+// frames on grid.x, so a frame costs no launch of its own, and decides a pair with crop_inside, the grid path's copy of crop2dr_kernel's
+// test (crop2dr_kernel keeps its own inline copy: calling crop_inside there changes its register allocation).  A frame of
+// CROP_GRID_MIN_PAIRS pairs or more is not written: the caller runs the single-frame entry point (its grid path) on it.
+// project_axis >= 0 (3-D rows): the records come from the plane of the two other axes, and a pair also needs box3dp_crop's test along
+// the axis, p - d / 2 < c < p + d / 2 with the box's centre c and extent d, rounded like torch's elementwise operators.
+template <typename T> struct CropZ { T c, hd; };
+
+template <typename T>
+__global__ void __launch_bounds__(256) crop_prep_batch_kernel(const T *__restrict__ boxes, int64_t m, int axis, CropBox<T> *__restrict__ recs,
+                                                              CropZ<T> *__restrict__ z)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    if (axis < 0) {
+        const T *b = boxes + 5 * i;
+        recs[i] = crop_prep_one<T>(b[0], b[1], b[2], b[3], b[4]);
+        return;
+    }
+    const T *b = boxes + 7 * i;
+    int pa, pb;
+    proj_plane(axis, &pa, &pb);
+    recs[i] = crop_prep_one<T>(b[pa], b[pb], b[3 + pa], b[3 + pb], b[6]);
+    CropZ<T> q;
+    q.c = b[axis]; q.hd = rn_div2(b[3 + axis]);
+    z[i] = q;
+}
+
+// frames on grid.x; 4096-point tiles on grid.y and 16-box tiles on grid.z, each striding over the frame's own tiles (tiles beyond the
+// frame's size exit at once)
+template <typename T, bool P3>
+__global__ void __launch_bounds__(CROP_THREADS) crop2dr_batch_kernel(const T *__restrict__ pts, const int64_t *__restrict__ poff, const CropBox<T> *__restrict__ recs,
+                                                                     const CropZ<T> *__restrict__ zr, const int64_t *__restrict__ boff, int axis,
+                                                                     const int64_t *__restrict__ moff, uint8_t *__restrict__ mask)
+{
+    __shared__ CropBox<T> sb[CROP_BT];
+    __shared__ CropZ<T> sz[P3 ? CROP_BT : 1];
+    const int64_t f = blockIdx.x, j0 = poff[f], n = poff[f + 1] - j0, i0 = boff[f], m = boff[f + 1] - i0;
+    if (n * m >= CROP_GRID_MIN_PAIRS) return;
+    const int64_t tiles_p = (n + CROP_THREADS * CROP_PPT - 1) / (CROP_THREADS * CROP_PPT), tiles_b = (m + CROP_BT - 1) / CROP_BT;
+    if ((int64_t)blockIdx.y >= tiles_p || (int64_t)blockIdx.z >= tiles_b) return;
+    int pa = 0, pb = 1;
+    if (P3) proj_plane(axis, &pa, &pb);
+    constexpr int PS = P3 ? 3 : 2;   // point row length
+    uint8_t *blk = mask + moff[f];
+    for (int64_t tb = blockIdx.z; tb < tiles_b; tb += gridDim.z) {
+        const int64_t box0 = tb * CROP_BT;
+        const int nb = (int)(m - box0 < CROP_BT ? m - box0 : CROP_BT);
+        __syncthreads();
+        for (int i = threadIdx.x; i < nb * (int)(sizeof(CropBox<T>) / sizeof(T)); i += CROP_THREADS)
+            reinterpret_cast<T *>(sb)[i] = reinterpret_cast<const T *>(recs + i0 + box0)[i];
+        if (P3 && threadIdx.x < nb) sz[threadIdx.x] = zr[i0 + box0 + threadIdx.x];
+        __syncthreads();
+        for (int64_t tp = blockIdx.y; tp < tiles_p; tp += gridDim.y) {
+            const int64_t p0 = (tp * CROP_THREADS + threadIdx.x) * CROP_PPT;
+            if (p0 >= n) continue;
+            T px[CROP_PPT], py[CROP_PPT], pz[P3 ? CROP_PPT : 1];
+            const bool full = p0 + CROP_PPT <= n;
+#pragma unroll
+            for (int k = 0; k < CROP_PPT; k++) {
+                const int64_t j = j0 + (p0 + k < n ? p0 + k : n - 1);
+                px[k] = pts[PS * j + pa]; py[k] = pts[PS * j + pb];
+                if (P3) pz[k] = pts[PS * j + axis];
+            }
+            for (int b = 0; b < nb; b++) {
+                const CropBox<T> B = sb[b];
+                uint32_t wds[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+                for (int k = 0; k < CROP_PPT; k++) {
+                    bool in = crop_inside<T>(B, px[k], py[k]);
+                    if (P3) in = in && rn_sub(pz[k], sz[b].hd) < sz[b].c && sz[b].c < rn_add(pz[k], sz[b].hd);
+                    wds[k >> 2] |= (in ? 1u : 0u) << ((k & 3) * 8);
+                }
+                uint8_t *row = blk + (box0 + b) * n + p0;
+                if (full && (reinterpret_cast<uintptr_t>(row) & 15) == 0) {   // frame blocks and rows start anywhere: decide per row
+                    __stcs(reinterpret_cast<uint4 *>(row), make_uint4(wds[0], wds[1], wds[2], wds[3]));
+                } else {
+                    for (int k = 0; k < CROP_PPT && p0 + k < n; k++) row[k] = (uint8_t)((wds[k >> 2] >> ((k & 3) * 8)) & 1u);
+                }
+            }
+        }
+    }
+}
+
+template <typename T> static size_t crop_batch_ws_bytes(int64_t total_boxes)
+{
+    const size_t m1 = (size_t)(total_boxes > 0 ? total_boxes : 1);
+    return 256 + align_up(m1 * sizeof(CropBox<T>)) + align_up(m1 * sizeof(CropZ<T>));
+}
+
+template <typename T>
+static int crop_batch_impl(const T *pts, int64_t total_pts, const int64_t *poff, const T *boxes, int64_t total_boxes, const int64_t *boff, int64_t nframes,
+                           int64_t max_pts, int64_t max_boxes, int axis, const int64_t *moff, uint8_t *mask, void *ws, size_t ws_bytes, cudaStream_t st)
+{
+    if (total_pts < 0 || total_boxes < 0 || nframes < 0 || max_pts < 0 || max_boxes < 0 || axis < -1 || axis > 2) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes == 0 || total_pts == 0 || total_boxes == 0) return D3D_OK;   // every block is empty
+    if (!pts || !poff || !boxes || !boff || !moff || !mask) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes > 0x7fffffffll) return D3D_ERR_UNSUPPORTED;
+    if (!ws || ws_bytes < crop_batch_ws_bytes<T>(total_boxes)) return D3D_ERR_WORKSPACE;
+    if (max_pts == 0) max_pts = total_pts;   // 0: bound unknown
+    if (max_boxes == 0) max_boxes = total_boxes;
+    Arena a(ws, ws_bytes);
+    a.take<char>(256);
+    CropBox<T> *recs = a.take<CropBox<T>>(total_boxes);
+    CropZ<T> *z = a.take<CropZ<T>>(total_boxes);
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    crop_prep_batch_kernel<T><<<(unsigned)cdiv(total_boxes, 256), 256, 0, st>>>(boxes, total_boxes, axis, recs, z); D3D_LAUNCHED();
+    const int64_t gy = cdiv(max_pts, (int64_t)CROP_THREADS * CROP_PPT), gz = cdiv(max_boxes, CROP_BT);
+    const dim3 grid((unsigned)nframes, (unsigned)(gy < 65535 ? gy : 65535), (unsigned)(gz < 65535 ? gz : 65535));
+    if (axis < 0) crop2dr_batch_kernel<T, false><<<grid, CROP_THREADS, 0, st>>>(pts, poff, recs, z, boff, axis, moff, mask);
+    else crop2dr_batch_kernel<T, true><<<grid, CROP_THREADS, 0, st>>>(pts, poff, recs, z, boff, axis, moff, mask);
+    D3D_LAUNCHED();
+    return D3D_OK;
+}
+
 }  // namespace d3d
 
 using namespace d3d;
@@ -441,3 +550,23 @@ extern "C" int d3d_crop2dr_f32(const float *points, int64_t n, const float *boxe
 { return crop_impl<float>(points, n, boxes, m, mask, ws, wsb, (cudaStream_t)stream); }
 extern "C" int d3d_crop2dr_f64(const double *points, int64_t n, const double *boxes, int64_t m, uint8_t *mask, void *ws, size_t wsb, void *stream)
 { return crop_impl<double>(points, n, boxes, m, mask, ws, wsb, (cudaStream_t)stream); }
+extern "C" int64_t d3d_crop2dr_grid_min_pairs(void) { return CROP_GRID_MIN_PAIRS; }
+extern "C" size_t d3d_crop2dr_batch_workspace_bytes(int64_t total_boxes, int dtype)
+{
+    if (total_boxes < 0) return 0;
+    return dtype == D3D_F64 ? crop_batch_ws_bytes<double>(total_boxes) : crop_batch_ws_bytes<float>(total_boxes);
+}
+extern "C" int d3d_crop2dr_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes, int64_t total_boxes,
+                                     const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                                     const int64_t *mask_offsets, uint8_t *mask, void *ws, size_t wsb, void *stream)
+{
+    return crop_batch_impl<float>(points, total_points, point_offsets, boxes, total_boxes, box_offsets, nframes, max_frame_points, max_frame_boxes,
+                                  project_axis, mask_offsets, mask, ws, wsb, (cudaStream_t)stream);
+}
+extern "C" int d3d_crop2dr_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes, int64_t total_boxes,
+                                     const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                                     const int64_t *mask_offsets, uint8_t *mask, void *ws, size_t wsb, void *stream)
+{
+    return crop_batch_impl<double>(points, total_points, point_offsets, boxes, total_boxes, box_offsets, nframes, max_frame_points, max_frame_boxes,
+                                   project_axis, mask_offsets, mask, ws, wsb, (cudaStream_t)stream);
+}

@@ -182,6 +182,47 @@ int d3d_pdist2dr_backward_f32(const float *points, int64_t n, const float *boxes
                               float *grad_points, void *stream);
 int d3d_pdist2dr_backward_f64(const double *points, int64_t n, const double *boxes, int64_t m, const double *grad, double *grad_boxes,
                               double *grad_points, void *stream);
+/* Frame-batched point-to-box mask and distance (a training batch or a dataset pass computes them once per frame).  Frames are packed back
+ * to back: points T[total_points, P] and boxes T[total_boxes, B] with DEVICE offsets point_offsets / box_offsets i64[nframes+1] (frame f
+ * owns rows [offsets[f], offsets[f+1]), n_f points and m_f boxes).  out_offsets DEVICE i64[nframes+1] (mask_offsets / dist_offsets): frame
+ * f's result is the row-major [m_f boxes, n_f points] block at out + out_offsets[f], usually at the running sum of m_f * n_f.
+ * project_axis -1: P = 2, B = 5 (x, y, w, h, r), per frame the result of d3d_crop2dr_* / d3d_pdist2dr_*.  project_axis 0, 1 or 2: P = 3,
+ * B = 7 (x, y, z, lx, ly, lz, r), projected to that axis like box3dp_crop / box3dr_pdist (d3d_b200.box): the 2-D operator runs on point
+ * columns (a, b) and box columns (a, b, 3 + a, 3 + b, 6), where a < b are the two other axes; the mask also requires
+ * p - d / 2 < c < p + d / 2 along the axis (point coordinate p, box centre c and extent d), the distance combines the 2-D distance d2 with
+ * the axial distance dp = min(c + d / 2 - p, p - c + d / 2) (the branch on p > c): min(d2, dp) inside the prism, d2 or dp where only one of
+ * them is positive, -sqrt(d2^2 + dp^2) outside both.  Every operation is rounded like torch's elementwise operators, so per frame the
+ * values equal the Python functions' bit for bit.
+ * max_frame_points / max_frame_boxes: HARD UPPER BOUNDS of n_f / m_f (0 = unknown, assume the totals); they size the launch grid.  No limit
+ * on nframes below 2^31.  Negative sizes or project_axis outside -1..2: D3D_ERR_INVALID_ARGUMENT; nframes == 0 or an empty side: no-op.
+ * d3d_crop2dr_batch_*: one box preparation and one mask launch.  A frame with n_f * m_f >= d3d_crop2dr_grid_min_pairs() is NOT written
+ * (neither are the bounds required to cover it): run d3d_crop2dr_* on it, whose grid path is faster there, then apply the axis test for
+ * project_axis >= 0.  Workspace below d3d_crop2dr_batch_workspace_bytes: D3D_ERR_WORKSPACE.
+ * d3d_pdist2dr_batch_*: one launch, no workspace, no iedge output.  The backward ACCUMULATES into grad_boxes T[total_boxes, B] and
+ * grad_points T[total_points, P] (caller zero-fills them); grad T has the layout of dist.  The 3-D gradient is the analytic gradient of the
+ * combination: where d2 == dp > 0 each gets half, and on the corner branch (d2, dp) get -(d2, dp) / sqrt(d2^2 + dp^2), 0 where both are 0. */
+int64_t d3d_crop2dr_grid_min_pairs(void);
+size_t d3d_crop2dr_batch_workspace_bytes(int64_t total_boxes, int dtype);
+int d3d_crop2dr_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes, int64_t total_boxes,
+                          const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                          const int64_t *mask_offsets, uint8_t *mask, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_crop2dr_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes, int64_t total_boxes,
+                          const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                          const int64_t *mask_offsets, uint8_t *mask, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_pdist2dr_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes, int64_t total_boxes,
+                           const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                           const int64_t *dist_offsets, float *dist, void *stream);
+int d3d_pdist2dr_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes, int64_t total_boxes,
+                           const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
+                           const int64_t *dist_offsets, double *dist, void *stream);
+int d3d_pdist2dr_batch_backward_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes,
+                                    int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                    int64_t max_frame_boxes, int project_axis, const int64_t *dist_offsets, const float *grad,
+                                    float *grad_boxes, float *grad_points, void *stream);
+int d3d_pdist2dr_batch_backward_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes,
+                                    int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                    int64_t max_frame_boxes, int project_axis, const int64_t *dist_offsets, const double *grad,
+                                    double *grad_boxes, double *grad_points, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * NMS, replaces nms2d[_cuda] (reference d3d/box/nms.h:6-10, nms.cpp:98-119, nms_cuda.cu:217-244).
