@@ -74,6 +74,10 @@ diou2dr = {F32: _sig("d3d_diou2dr_f32", C.c_int, _iex_sig), F64: _sig("d3d_diou2
 _ibw_sig = [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp]
 iou_backward = {name: {F32: _sig(f"d3d_{name}_backward_f32", C.c_int, _ibw_sig), F64: _sig(f"d3d_{name}_backward_f64", C.c_int, _ibw_sig)}
                 for name in ("iou2d", "iou2dr", "giou2dr", "diou2dr")}
+iou_batch_workspace_bytes = _sig("d3d_box2d_iou_batch_workspace_bytes", _sz, [_i64, _i64, _i64, C.c_int])
+_ib_sig = [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i64, _i64, C.c_int, _vp]   # packed boxes, offsets, bounds, iou type, out offsets
+iou_batch = {k: _sig(f"d3d_box2d_iou_batch_{s}", C.c_int, _ib_sig + [_vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+iou_batch_backward = {k: _sig(f"d3d_box2d_iou_batch_backward_{s}", C.c_int, _ib_sig + [_vp, _vp, _vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 match_greedy = _sig("d3d_match_greedy_f32", C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
 match_greedy_batch = _sig("d3d_match_greedy_batch_f32", C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
 iou_count_candidates = _sig("d3d_iou_count_candidates", C.c_int, [_vp, _i64, _vp, _i64, C.c_int, _vp, _vp, _sz, _vp])

@@ -188,6 +188,120 @@ def box2d_iou(boxes1, boxes2, method="box", precise=True):
     return result
 
 
+# rows x columns of the "rbox" tile (IouTile in csrc/iou.cu; keep both in step): a frame of more than 65535 tiles on an axis would make the
+# batch call return D3D_ERR_UNSUPPORTED, so it runs the single-frame kernel instead
+_IOU_TILE = {torch.float32: (64, 128), torch.float64: (64, 64)}
+
+
+class _IouBatch(torch.autograd.Function):
+    """packed IoU blocks of all frames: the forward is one launch sequence, the backward two launches, whatever the number of frames"""
+    @staticmethod
+    def forward(ctx, boxes1, boxes2, offsets, nframes, bounds, iou_type, total, big):
+        code = _c.dtype_code(boxes1.dtype)
+        out = torch.empty(total, dtype=boxes1.dtype, device=boxes1.device)
+        od1, od2, odo = offsets
+        fwd_max1, fwd_max2, max1, max2 = bounds
+        if fwd_max1 and fwd_max2:   # "rbox": the bounds of the frames that fit the tile grid, so the batch kernels skip the others
+            ws = None   # "grbox" / "drbox" need no workspace
+            if iou_type in (IouType.BOX, IouType.RBOX):
+                ws = _c.workspace(_c.iou_batch_workspace_bytes(len(boxes1), len(boxes2), nframes, code), boxes1.device)
+            with torch.cuda.device(boxes1.device):
+                st = _c.iou_batch[code](_c.ptr(boxes1), len(boxes1), _c.ptr(od1), _c.ptr(boxes2), len(boxes2), _c.ptr(od2), nframes, fwd_max1, fwd_max2,
+                                        int(iou_type), _c.ptr(odo), _c.ptr(out), _c.ptr(ws), ws.numel() if ws is not None else 0, _c.stream_ptr())
+            _c.check(st, "box2d_iou_batch")
+        for a0, a1, b0, b1, o0 in big:   # "rbox" frames past the batch kernel's tile grid: the single-frame kernel, into their block
+            _pairwise(boxes1[a0:a1], boxes2[b0:b1], _c.iou2dr, out=out[o0:o0 + (a1 - a0) * (b1 - b0)].view(a1 - a0, b1 - b0))
+        ctx.save_for_backward(boxes1, boxes2, *offsets)
+        ctx.args = (nframes, max1, max2, iou_type)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad):
+        boxes1, boxes2, od1, od2, odo = ctx.saved_tensors
+        nframes, max1, max2, iou_type = ctx.args
+        code = _c.dtype_code(boxes1.dtype)
+        grad = grad.contiguous()
+        g1, g2 = torch.empty_like(boxes1), torch.empty_like(boxes2)
+        with torch.cuda.device(boxes1.device):
+            st = _c.iou_batch_backward[code](_c.ptr(boxes1), len(boxes1), _c.ptr(od1), _c.ptr(boxes2), len(boxes2), _c.ptr(od2), nframes, max1, max2,
+                                             int(iou_type), _c.ptr(odo), _c.ptr(grad), _c.ptr(g1), _c.ptr(g2), _c.stream_ptr())
+        _c.check(st, "box2d_iou_batch backward")
+        return g1, g2, None, None, None, None, None, None
+
+
+def _check_iou2d(boxes1, boxes2):   # box2d_iou's checks
+    if len(boxes1.shape) != 2 or len(boxes2.shape) != 2:
+        raise ValueError("Input of rbox_2d_iou should be Nx2 tensors!")
+    if boxes1.shape[1] != 5 or boxes2.shape[1] != 5:
+        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+
+
+def box2d_iou_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", precise=True):
+    '''
+    :func:`box2d_iou` on a batch of frames (target assignment and IoU losses of a training batch); differentiable in both box sets.  Per
+    frame the values equal :func:`box2d_iou` on that frame bit for bit, and so do the gradients.  Two call forms, like
+    :func:`box3d_iou_distance_batch`: lists of per-frame ``boxes1`` [n_f, 5] / ``boxes2`` [m_f, 5] (returns the list of [n_f, m_f]
+    matrices, views into one packed buffer), or the frames packed back to back with ``offsets1`` / ``offsets2`` (int64 [nframes + 1], CPU)
+    (returns ``(iou_flat, iou_offsets)``: frame f's matrix is ``iou_flat[iou_offsets[f]:iou_offsets[f + 1]].view(n_f, m_f)``).  ``method``
+    and ``precise`` as in :func:`box2d_iou`.  numpy in -> numpy out, host tensors in -> host tensors out.  "rbox" frames of more than
+    65535 tiles (64 rows, or 128 fp32 / 64 fp64 columns) run the single-frame kernel, into their block; the batch kernels skip them,
+    though the workspace still has room for their records.
+    '''
+    as_list = isinstance(boxes1, (list, tuple))
+    if as_list:
+        if not isinstance(boxes2, (list, tuple)) or len(boxes1) != len(boxes2):
+            raise ValueError("boxes1 and boxes2 should hold the same number of frames")
+        if len(boxes1) == 0:
+            return []
+        numpy_in = isinstance(boxes1[0], np.ndarray)
+        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
+        l1, l2 = [tt(b) for b in boxes1], [tt(b) for b in boxes2]
+        for a, b in zip(l1, l2):
+            _check_iou2d(a, b)
+        if len({x.dtype for x in l1}) != 1 or len({x.dtype for x in l2}) != 1:
+            raise RuntimeError("the frames of a box set must have the same dtype")
+        off1, off2 = _frame_offsets(lens=[len(b) for b in l1]), _frame_offsets(lens=[len(b) for b in l2])
+        B1, B2 = torch.cat(l1), torch.cat(l2)
+    else:
+        numpy_in = isinstance(boxes1, np.ndarray)
+        if numpy_in:
+            assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
+            boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
+        if offsets1 is None or offsets2 is None:
+            raise ValueError("packed boxes need the frame offsets")
+        _check_iou2d(boxes1, boxes2)
+        off1, off2 = _frame_offsets(offsets1), _frame_offsets(offsets2)
+        B1, B2 = boxes1, boxes2
+    if off1.numel() != off2.numel() or int(off1[-1]) != len(B1) or int(off2[-1]) != len(B2):
+        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
+    iou_type = getattr(IouType, method.upper())
+    if iou_type not in (IouType.BOX, IouType.RBOX, IouType.GRBOX, IouType.DRBOX):
+        raise ValueError("Unrecognized iou type!")
+    otype, odev = B1.dtype, B1.device
+    b1, b2 = _c.to_device(B1), _c.to_device(B2)
+    if precise:
+        b1, b2 = b1.to(torch.float64), b2.to(torch.float64)
+    _c.dtype_code(b1.dtype)
+    if b2.dtype != b1.dtype:
+        raise RuntimeError("boxes1 and boxes2 must have the same dtype")
+    nframes = off1.numel() - 1
+    n_f, m_f = off1[1:] - off1[:-1], off2[1:] - off2[:-1]
+    blk = _block_offsets(off1, off2)
+    big = torch.zeros(nframes, dtype=torch.bool)
+    if iou_type == IouType.RBOX:
+        tr, tc = _IOU_TILE[b1.dtype]
+        big = (n_f > 65535 * tr) | (m_f > 65535 * tc)
+    small = (n_f * m_f > 0) & ~big
+    bounds = (int(n_f[small].max()) if bool(small.any()) else 0, int(m_f[small].max()) if bool(small.any()) else 0,
+              int(n_f.max()) if nframes else 0, int(m_f.max()) if nframes else 0)
+    big_frames = [(int(off1[f]), int(off1[f + 1]), int(off2[f]), int(off2[f + 1]), int(blk[f])) for f in torch.nonzero(big).flatten().tolist()]
+    offsets = _device_offsets(off1, off2, blk, b1.device)
+    flat = _IouBatch.apply(b1.contiguous(), b2.contiguous(), offsets, nframes, bounds, iou_type, int(blk[-1]), big_frames)
+    if precise:
+        flat = flat.to(otype)
+    return _point_box_outputs(flat, blk, off2, off1, as_list, numpy_in, odev)
+
+
 def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold=0, score_threshold=0, precise=True, offsets_dev=None,
                     supression_method="hard", supression_param=0):
     '''

@@ -30,6 +30,14 @@ void set_cuda_error(cudaError_t e);
 
 static inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 static inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
+// blocks on a grid axis (at most 65535) for `items` work items, per_block of them per block; kernels stride over the rest
+static inline unsigned stride_blocks(int64_t items, int64_t per_block)
+{
+    const int64_t b = items / per_block + (items % per_block != 0);
+    return (unsigned)(b < 1 ? 1 : b < 65535 ? b : 65535);
+}
+// n * m, saturating at INT64_MAX
+static inline int64_t pair_bound(int64_t n, int64_t m) { return n > 0 && m > INT64_MAX / n ? INT64_MAX : n * m; }
 
 // bump allocator over the caller's workspace
 struct Arena {

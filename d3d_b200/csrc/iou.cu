@@ -24,11 +24,10 @@ namespace d3d {
 // TILE > 0: field-major inside blocks of TILE boxes -- block t holds cx[TILE], cy[TILE], c, s, hw, hh, rho, area -- so that
 // a column tile is staged with one contiguous copy and a warp's shared-memory reads of one field of 32 different
 // columns of a 32-column chunk hit 32 different banks.
+// Box i of n; i >= n writes padding.
 template <typename T, int TILE>
-__global__ void __launch_bounds__(256) box_prep_kernel(const T *__restrict__ boxes, int64_t n, int64_t npad, BoxRec<T> *__restrict__ recs)
+__device__ __forceinline__ void box_prep_one(const T *__restrict__ boxes, int64_t n, int64_t i, BoxRec<T> *__restrict__ recs)
 {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= npad) return;
     BoxRec<T> r;
     if (i < n) {
         const T *b = boxes + 5 * i;
@@ -46,6 +45,14 @@ __global__ void __launch_bounds__(256) box_prep_kernel(const T *__restrict__ box
     }
 }
 
+template <typename T, int TILE>
+__global__ void __launch_bounds__(256) box_prep_kernel(const T *__restrict__ boxes, int64_t n, int64_t npad, BoxRec<T> *__restrict__ recs)
+{
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npad) return;
+    box_prep_one<T, TILE>(boxes, n, i, recs);
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) aabb_prep_kernel(const T *__restrict__ boxes, int64_t n, AABBRec<T> *__restrict__ recs)
 {
@@ -56,6 +63,8 @@ __global__ void __launch_bounds__(256) aabb_prep_kernel(const T *__restrict__ bo
 }
 
 // ------------------------------------------------------------------ rotated IoU tile kernel
+// box2d_iou_batch (d3d_b200/box/__init__.py, _IOU_TILE) repeats these shapes: it sends "rbox" frames of more than 65535 tiles on an axis
+// to the single-matrix kernel instead of the batch, so a change here must be made there too
 template <typename T> struct IouTile;
 template <> struct IouTile<float>  { static constexpr int TR = 64, TC = 128; };
 template <> struct IouTile<double> { static constexpr int TR = 64, TC = 64; };
@@ -242,6 +251,15 @@ iou2dr_tile_kernel(const BoxRec<T> *__restrict__ recA, int64_t n, const BoxRec<T
 }
 
 // ------------------------------------------------------------------ AABB IoU (method "box"): cheap, one thread per 4 columns
+// columns c0 .. c0+3 of the row at out + rowoff
+template <typename T>
+__device__ __forceinline__ void iou2d_cols(const AABBRec<T> a, const AABBRec<T> *__restrict__ recB, int64_t m, int64_t c0, T *__restrict__ out, int64_t rowoff)
+{
+#pragma unroll
+    for (int k = 0; k < 4; k++)
+        if (c0 + k < m) out[rowoff + c0 + k] = aabb_iou<T>(a, recB[c0 + k]);
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) iou2d_kernel(const AABBRec<T> *__restrict__ recA, int64_t n, const AABBRec<T> *__restrict__ recB, int64_t m,
                                                     T *__restrict__ out, int64_t ld)
@@ -249,10 +267,7 @@ __global__ void __launch_bounds__(256) iou2d_kernel(const AABBRec<T> *__restrict
     const int64_t row = blockIdx.y;
     const int64_t c0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (row >= n || c0 >= m) return;
-    const AABBRec<T> a = recA[row];
-#pragma unroll
-    for (int k = 0; k < 4; k++)
-        if (c0 + k < m) out[row * ld + c0 + k] = aabb_iou<T>(a, recB[c0 + k]);
+    iou2d_cols<T>(recA[row], recB, m, c0, out, row * ld);
 }
 
 // AABB variant of the matcher distance (DistanceTypes.IoU, d3d/dgal_wrap.h:70-91): 1 - iou(AABBs) * ziou.  Columns c0 .. c0+3 of the row at out + rowoff.
@@ -354,6 +369,51 @@ __global__ void __launch_bounds__(256) dist3d_aabb_batch_kernel(const AABBRec<fl
     if (row >= n || c0 >= m) return;
     const int64_t a = frame_rec_base(off1, f, 1) + row, b0 = frame_rec_base(off2, f, 1);
     dist3d_aabb_cols(recA[a], zA[a], recB + b0, zB + b0, m, c0, dist + dist_off[f], row * m);
+}
+
+// ------------------------------------------------------------------ frame-batched IoU matrix (box2d_iou_batch, methods "rbox" / "box")
+// Same layout as the distance matrix: frame f's n_f x m_f block (leading dimension m_f) at out + out_off[f], its records at
+// off[f] + f * pad.  Frames on grid.x, the frame's boxes strided over grid.y: box_prep_one over the frame, padded to a multiple of pad.
+// A frame of more than max_n boxes is skipped: the tile kernel skips it too (the caller runs the single-matrix kernel on it).
+template <typename T, int TILE>
+__global__ void __launch_bounds__(256) box_prep_batch_kernel(const T *__restrict__ boxes, const int64_t *__restrict__ off, int pad, int64_t max_n,
+                                                             BoxRec<T> *__restrict__ recs)
+{
+    const int64_t f = blockIdx.x, b0 = off[f], n = off[f + 1] - b0, npad = (n + pad - 1) / pad * pad;
+    if (n > max_n) return;
+    BoxRec<T> *r = recs + frame_rec_base(off, f, pad);
+    for (int64_t i = (int64_t)blockIdx.y * blockDim.x + threadIdx.x; i < npad; i += (int64_t)gridDim.y * blockDim.x)
+        box_prep_one<T, TILE>(boxes + 5 * b0, n, i, r);
+}
+
+// rotated: frames on grid.x, column tiles on grid.y, row tiles on grid.z; tiles beyond the frame's own size exit at once, and so does
+// every tile of a frame beyond the bounds max1 x max2 that size the grid
+template <typename T>
+__global__ void __launch_bounds__(IOU_THREADS, 3)
+iou2dr_batch_tile_kernel(const BoxRec<T> *__restrict__ recA, const int64_t *__restrict__ off1, const BoxRec<T> *__restrict__ recB,
+                         const int64_t *__restrict__ off2, int64_t max1, int64_t max2, const int64_t *__restrict__ out_off, T *__restrict__ out)
+{
+    constexpr int TR = IouTile<T>::TR, TC = IouTile<T>::TC;
+    const int64_t f = blockIdx.x, n = off1[f + 1] - off1[f], m = off2[f + 1] - off2[f];
+    const int64_t row0 = (int64_t)blockIdx.z * TR, col0 = (int64_t)blockIdx.y * TC;
+    if (row0 >= n || col0 >= m || n > max1 || m > max2) return;
+    iou2dr_tile<T, false>(recA + frame_rec_base(off1, f, TR), n, recB + frame_rec_base(off2, f, TC), m, out + out_off[f], m, nullptr, nullptr,
+                          row0, col0);
+}
+
+// axis-aligned: frames on grid.x; the threads of grid.y stride over the frame's (row, 4-column chunk) pairs, each running iou2d_kernel's
+// 4 columns of one row, so that a frame of a few dozen columns still fills its CTAs.  Records are the packed AABBs.
+template <typename T>
+__global__ void __launch_bounds__(256) iou2d_batch_kernel(const AABBRec<T> *__restrict__ recA, const int64_t *__restrict__ off1,
+                                                          const AABBRec<T> *__restrict__ recB, const int64_t *__restrict__ off2,
+                                                          const int64_t *__restrict__ out_off, T *__restrict__ out)
+{
+    const int64_t f = blockIdx.x, a0 = off1[f], b0 = off2[f], n = off1[f + 1] - a0, m = off2[f + 1] - b0, cm = (m + 3) / 4, nq = n * cm;
+    T *o = out + out_off[f];
+    for (int64_t q = (int64_t)blockIdx.y * blockDim.x + threadIdx.x; q < nq; q += (int64_t)gridDim.y * blockDim.x) {
+        const int64_t i = q / cm;
+        iou2d_cols<T>(recA[a0 + i], recB + b0, m, (q - i * cm) * 4, o, i * m);
+    }
 }
 
 // ------------------------------------------------------------------ candidate counter (measurement only; SURVEY.md 8(d) accounting)
@@ -545,6 +605,64 @@ static int dist3d_batch_impl(const float *b1, int64_t total1, const int64_t *off
     return D3D_OK;
 }
 
+template <typename T> static size_t iou_batch_ws_bytes(int64_t total1, int64_t total2, int64_t nframes)
+{
+    constexpr int TR = IouTile<T>::TR, TC = IouTile<T>::TC;
+    if (total1 < 0 || total2 < 0 || nframes < 0) return 0;
+    const size_t np = (size_t)(total1 + nframes * TR), mp = (size_t)(total2 + nframes * TC);
+    return 256 + align_up(np * sizeof(BoxRec<T>)) + align_up(mp * sizeof(BoxRec<T>));
+}
+
+// GIoU / DIoU forward of a packed batch (iou_grad.cu)
+template <typename T>
+int iou_ex_batch_fwd(const T *b1, const int64_t *off1, const T *b2, const int64_t *off2, int64_t nframes, int64_t max_pairs, int iou_type,
+                     const int64_t *out_off, T *out, cudaStream_t st);
+
+// every frame of a packed batch through the single-matrix per-pair code: "rbox" and "box" two prep launches and one IoU launch, "grbox" /
+// "drbox" one launch, whatever the number of frames
+template <typename T>
+static int iou_batch_impl(const T *b1, int64_t total1, const int64_t *off1, const T *b2, int64_t total2, const int64_t *off2, int64_t nframes,
+                          int64_t max1, int64_t max2, int iou_type, const int64_t *out_off, T *out, void *ws, size_t ws_bytes, cudaStream_t st)
+{
+    if (iou_type != D3D_IOU_BOX && iou_type != D3D_IOU_RBOX && iou_type != D3D_IOU_GRBOX && iou_type != D3D_IOU_DRBOX) return D3D_ERR_INVALID_ARGUMENT;
+    if (total1 < 0 || total2 < 0 || nframes < 0 || max1 < 0 || max2 < 0) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes == 0 || total1 == 0 || total2 == 0) return D3D_OK;   // every block is empty
+    if (!b1 || !b2 || !off1 || !off2 || !out_off || !out) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes > 0x7fffffffll) return D3D_ERR_UNSUPPORTED;
+    if (max1 == 0) max1 = total1;   // 0: bound unknown
+    if (max2 == 0) max2 = total2;
+    if (iou_type == D3D_IOU_GRBOX || iou_type == D3D_IOU_DRBOX)   // no records: the pair code reads the boxes
+        return iou_ex_batch_fwd<T>(b1, off1, b2, off2, nframes, pair_bound(max1, max2), iou_type, out_off, out, st);
+    constexpr int TR = IouTile<T>::TR, TC = IouTile<T>::TC;
+    const int64_t tiles_r = cdiv(max1, TR), tiles_c = cdiv(max2, TC);
+    if (iou_type == D3D_IOU_RBOX && (tiles_r > 65535 || tiles_c > 65535)) return D3D_ERR_UNSUPPORTED;
+    if (ws_bytes < iou_batch_ws_bytes<T>(total1, total2, nframes) || !ws) return D3D_ERR_WORKSPACE;
+    Arena a(ws, ws_bytes);
+    a.take<char>(256);
+    BoxRec<T> *ra = a.take<BoxRec<T>>(total1 + nframes * TR), *rb = a.take<BoxRec<T>>(total2 + nframes * TC);
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    const unsigned nf = (unsigned)nframes;
+    if (iou_type == D3D_IOU_BOX) {   // the AABB records need no frame padding: box i's record is record i
+        AABBRec<T> *aa = reinterpret_cast<AABBRec<T> *>(ra), *ab = reinterpret_cast<AABBRec<T> *>(rb);
+        aabb_prep_kernel<T><<<(unsigned)cdiv(total1, 256), 256, 0, st>>>(b1, total1, aa); D3D_LAUNCHED();
+        aabb_prep_kernel<T><<<(unsigned)cdiv(total2, 256), 256, 0, st>>>(b2, total2, ab); D3D_LAUNCHED();
+        iou2d_batch_kernel<T><<<dim3(nf, stride_blocks(pair_bound(max1, cdiv(max2, 4)), 256)), 256, 0, st>>>(aa, off1, ab, off2, out_off, out); D3D_LAUNCHED();
+        return D3D_OK;
+    }
+    box_prep_batch_kernel<T, 0><<<dim3(nf, stride_blocks(tiles_r * TR, 256)), 256, 0, st>>>(b1, off1, TR, max1, ra); D3D_LAUNCHED();
+    box_prep_batch_kernel<T, TC><<<dim3(nf, stride_blocks(tiles_c * TC, 256)), 256, 0, st>>>(b2, off2, TC, max2, rb); D3D_LAUNCHED();
+    static bool smem_opt_in[64] = {};   // per instantiation and per device
+    int dev = 0;
+    D3D_CUDA_TRY(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || !smem_opt_in[dev]) {
+        D3D_CUDA_TRY(cudaFuncSetAttribute(iou2dr_batch_tile_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IouSmem<T>)));
+        if (dev >= 0 && dev < 64) smem_opt_in[dev] = true;
+    }
+    iou2dr_batch_tile_kernel<T><<<dim3(nf, (unsigned)tiles_c, (unsigned)tiles_r), IOU_THREADS, sizeof(IouSmem<T>), st>>>(ra, off1, rb, off2, max1, max2, out_off, out);
+    D3D_LAUNCHED();
+    return D3D_OK;
+}
+
 template <typename T>
 static int count_cand_impl(const T *b1, int64_t n, const T *b2, int64_t m, unsigned long long *counters64, void *ws, size_t ws_bytes, cudaStream_t st)
 {
@@ -594,6 +712,20 @@ extern "C" int d3d_iou3d_distance_batch_f32(const float *boxes1, int64_t total1,
     return dist3d_batch_impl(boxes1, total1, offsets1, boxes2, total2, offsets2, nframes, max_frame1, max_frame2, rotated, dist_offsets, dist, ws, wsb,
                              (cudaStream_t)stream);
 }
+extern "C" size_t d3d_box2d_iou_batch_workspace_bytes(int64_t total1, int64_t total2, int64_t nframes, int dtype)
+{
+    return dtype == D3D_F64 ? iou_batch_ws_bytes<double>(total1, total2, nframes) : iou_batch_ws_bytes<float>(total1, total2, nframes);
+}
+#define D3D_IOU_BATCH_ENTRY(NAME, T)                                                                                                  \
+    extern "C" int NAME(const T *boxes1, int64_t total1, const int64_t *offsets1, const T *boxes2, int64_t total2, const int64_t *offsets2, \
+                        int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type, const int64_t *out_offsets, T *out,     \
+                        void *ws, size_t wsb, void *stream)                                                                           \
+    {                                                                                                                                 \
+        return iou_batch_impl<T>(boxes1, total1, offsets1, boxes2, total2, offsets2, nframes, max_frame1, max_frame2, iou_type,       \
+                                 out_offsets, out, ws, wsb, (cudaStream_t)stream);                                                    \
+    }
+D3D_IOU_BATCH_ENTRY(d3d_box2d_iou_batch_f32, float)
+D3D_IOU_BATCH_ENTRY(d3d_box2d_iou_batch_f64, double)
 extern "C" int d3d_iou_count_candidates(const void *b1, int64_t n, const void *b2, int64_t m, int dtype, uint64_t *counters64, void *ws, size_t wsb, void *stream)
 {
     return dtype == D3D_F64 ? count_cand_impl<double>((const double *)b1, n, (const double *)b2, m, (unsigned long long *)counters64, ws, wsb, (cudaStream_t)stream)

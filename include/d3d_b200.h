@@ -111,6 +111,36 @@ int d3d_diou2dr_backward_f32(const float *boxes1, int64_t n, const float *boxes2
                              float *grad_boxes2, void *stream);
 int d3d_diou2dr_backward_f64(const double *boxes1, int64_t n, const double *boxes2, int64_t m, const double *grad, int64_t ld, double *grad_boxes1,
                              double *grad_boxes2, void *stream);
+/* Frame-batched differentiable IoU family (a detector computes it once per frame of every training batch: target assignment, IoU / GIoU /
+ * DIoU losses).  Frames are packed back to back: boxes1 T[total1,5] / boxes2 T[total2,5] with DEVICE offsets1 / offsets2 i64[nframes+1]
+ * (frame f owns rows [offsets[f], offsets[f+1]), n_f and m_f of them).  out_offsets DEVICE i64[nframes+1]: frame f's block is the row-major
+ * [n_f, m_f] matrix at out + out_offsets[f] (leading dimension m_f), usually at the running sum of n_f * m_f.  iou_type: D3D_IOU_BOX (IoU of
+ * the axis-aligned bounding boxes), D3D_IOU_RBOX, D3D_IOU_GRBOX or D3D_IOU_DRBOX; anything else: D3D_ERR_INVALID_ARGUMENT.  Per frame, the
+ * block equals d3d_iou2d_* / d3d_iou2dr_* / d3d_giou2dr_* / d3d_diou2dr_* on that frame bit for bit, and the backward's gradients equal
+ * d3d_*_backward_* on that frame bit for bit: the frames run the same per-pair code, and the backward the same warp per owned box with the
+ * same summation order.  max_frame1 / max_frame2: HARD UPPER BOUNDS of n_f / m_f (0 = unknown, assume total1 / total2); they size the launch
+ * grid.  The RBOX forward skips a frame beyond them (n_f > max_frame1 or m_f > max_frame2): its block is not written, so a caller can pass
+ * the bounds of the frames that fit the tile grid and run d3d_iou2dr_* on the others.  Elsewhere a frame beyond them may be written only
+ * in part.  No limit on nframes below 2^31, nor on the frame sizes except for RBOX.
+ * Forward: "box" and "rbox" two box preparations and one IoU launch, "grbox" / "drbox" one launch and no workspace (may be NULL).  Workspace
+ * below d3d_box2d_iou_batch_workspace_bytes for BOX / RBOX: D3D_ERR_WORKSPACE.  RBOX frames over 65535 tiles of 64 rows or of 128 (fp32) /
+ * 64 (fp64) columns: D3D_ERR_UNSUPPORTED (call d3d_iou2dr_* on such frames).  Negative sizes: D3D_ERR_INVALID_ARGUMENT; nframes == 0 or an
+ * empty side: no-op.
+ * Backward: two launches, no workspace.  grad T has the layout of out; grad_boxes1 T[total1,5] / grad_boxes2 T[total2,5] are WRITTEN (not
+ * accumulated), every box included: the boxes of a frame whose other side is empty get exact zeros. */
+size_t d3d_box2d_iou_batch_workspace_bytes(int64_t total1, int64_t total2, int64_t nframes, int dtype);
+int d3d_box2d_iou_batch_f32(const float *boxes1, int64_t total1, const int64_t *offsets1, const float *boxes2, int64_t total2,
+                            const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type,
+                            const int64_t *out_offsets, float *out, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_box2d_iou_batch_f64(const double *boxes1, int64_t total1, const int64_t *offsets1, const double *boxes2, int64_t total2,
+                            const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type,
+                            const int64_t *out_offsets, double *out, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_box2d_iou_batch_backward_f32(const float *boxes1, int64_t total1, const int64_t *offsets1, const float *boxes2, int64_t total2,
+                                     const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type,
+                                     const int64_t *out_offsets, const float *grad, float *grad_boxes1, float *grad_boxes2, void *stream);
+int d3d_box2d_iou_batch_backward_f64(const double *boxes1, int64_t total1, const int64_t *offsets1, const double *boxes2, int64_t total2,
+                                     const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type,
+                                     const int64_t *out_offsets, const double *grad, double *grad_boxes1, double *grad_boxes2, void *stream);
 /* Detection-evaluation distance matrix (SURVEY.md 8(f) row f1): dist[i][j] = 1 - iou2d(BEV boxes) * ziou, fp32,
  * for 3-D boxes [n,7] / [m,7] with rows (x, y, z, lx, ly, lz, rz).  rotated != 0: rotated BEV IoU, replaces the pair
  * loop over box3dr_iou in ScoreMatcher.prepare_boxes (reference d3d/tracking/matcher.pyx:66-76, d3d/dgal_wrap.h:45-68);
