@@ -78,6 +78,9 @@ iou_batch_workspace_bytes = _sig("d3d_box2d_iou_batch_workspace_bytes", _sz, [_i
 _ib_sig = [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i64, _i64, C.c_int, _vp]   # packed boxes, offsets, bounds, iou type, out offsets
 iou_batch = {k: _sig(f"d3d_box2d_iou_batch_{s}", C.c_int, _ib_sig + [_vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 iou_batch_backward = {k: _sig(f"d3d_box2d_iou_batch_backward_{s}", C.c_int, _ib_sig + [_vp, _vp, _vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+iou_max_batch_workspace_bytes = _sig("d3d_box2d_iou_max_batch_workspace_bytes", _sz, [_i64, _i64, _i64, C.c_int])
+_imx_sig = _ib_sig[:-1] + [C.c_int, _vp, _vp, _vp, _vp, _vp, _sz, _vp]   # ... iou type, out dtype, max1, idx1, max2, idx2, workspace
+iou_max_batch = {k: _sig(f"d3d_box2d_iou_max_batch_{s}", C.c_int, _imx_sig) for k, s in ((F32, "f32"), (F64, "f64"))}
 match_greedy = _sig("d3d_match_greedy_f32", C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
 match_greedy_batch = _sig("d3d_match_greedy_batch_f32", C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp])
 iou_count_candidates = _sig("d3d_iou_count_candidates", C.c_int, [_vp, _i64, _vp, _i64, C.c_int, _vp, _vp, _sz, _vp])

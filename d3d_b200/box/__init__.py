@@ -302,6 +302,109 @@ def box2d_iou_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", 
     return _point_box_outputs(flat, blk, off2, off1, as_list, numpy_in, odev)
 
 
+def _iou_max_packed(B1, B2, off1, off2, method, precise):
+    """(max1, idx1, max2, idx2) of packed frames on the device, frame-local indices"""
+    iou_type = getattr(IouType, method.upper())
+    if iou_type not in (IouType.BOX, IouType.RBOX):
+        raise ValueError("Unsupported iou type!")
+    otype = B1.dtype
+    b1, b2 = _c.to_device(B1.detach()), _c.to_device(B2.detach())
+    if precise:
+        b1, b2 = b1.to(torch.float64), b2.to(torch.float64)
+    code = _c.dtype_code(b1.dtype)
+    if b2.dtype != b1.dtype:
+        raise RuntimeError("boxes1 and boxes2 must have the same dtype")
+    ocode = _c.dtype_code(otype)
+    dev, total1, total2, nframes = b1.device, len(b1), len(b2), off1.numel() - 1
+    max1, max2 = torch.empty(total1, dtype=otype, device=dev), torch.empty(total2, dtype=otype, device=dev)
+    idx1, idx2 = torch.empty(total1, dtype=torch.int64, device=dev), torch.empty(total2, dtype=torch.int64, device=dev)
+    if nframes and total1 + total2:
+        b1, b2 = b1.contiguous(), b2.contiguous()
+        n_f, m_f = off1[1:] - off1[:-1], off2[1:] - off2[:-1]
+        offs = torch.cat([off1, off2]).to(dev, non_blocking=True)   # one copy of both offset arrays
+        ws = _c.workspace(_c.iou_max_batch_workspace_bytes(total1, total2, nframes, code), dev)
+        with torch.cuda.device(dev):
+            st = _c.iou_max_batch[code](_c.ptr(b1), total1, _c.ptr(offs[:nframes + 1]), _c.ptr(b2), total2, _c.ptr(offs[nframes + 1:]), nframes,
+                                        int(n_f.max()), int(m_f.max()), int(iou_type), ocode, _c.ptr(max1), _c.ptr(idx1), _c.ptr(max2), _c.ptr(idx2),
+                                        _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        _c.check(st, "box2d_iou_max_batch")
+    return max1, idx1, max2, idx2
+
+
+def _iou_max_outputs(outs, odev, numpy_in):
+    if odev.type != "cuda" or numpy_in:
+        outs = tuple(x.cpu() for x in outs)
+    return tuple(x.numpy() for x in outs) if numpy_in else tuple(outs)
+
+
+def box2d_iou_max(boxes1, boxes2, method="box", precise=True):
+    '''
+    Best overlap of every box with the other set, without the IoU matrix (target assignment: each anchor's best ground truth and each
+    ground truth's best anchor).  Returns ``(max1, idx1, max2, idx2)``: ``max1`` / ``idx1`` [N] are the values and int64 indices that
+    ``torch.max(box2d_iou(boxes1, boxes2, method, precise), dim=1)`` returns, ``max2`` / ``idx2`` [M] those of ``dim=0``, bit for bit:
+    the comparison is made on the values in the output dtype (with ``precise``, computed in float64 and rounded to the input dtype), ties
+    go to the lower index, and NaN is the maximum, at the first NaN's index.  Where torch would raise because the other set is empty,
+    the value is 0 and the index -1.  The outputs do not require grad: they are assignment targets, not a differentiable IoU.
+    numpy in -> numpy out, host tensors in -> host tensors out.
+
+    :param boxes1: Input boxes, shape is N x 5 (x,y,w,h,r)
+    :param boxes2: Input boxes, shape is M x 5 (x,y,w,h,r)
+    :param method: 'box' - axis-aligned box, 'rbox' - rotated box
+    :param precise: force using double precision to calculate iou
+    '''
+    numpy_in = isinstance(boxes1, np.ndarray)
+    if numpy_in:
+        assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
+        boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
+    _check_iou2d(boxes1, boxes2)
+    off1, off2 = _frame_offsets(lens=[len(boxes1)]), _frame_offsets(lens=[len(boxes2)])
+    return _iou_max_outputs(_iou_max_packed(boxes1, boxes2, off1, off2, method, precise), boxes1.device, numpy_in)
+
+
+def box2d_iou_max_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", precise=True):
+    '''
+    :func:`box2d_iou_max` on a batch of frames in one launch sequence; per frame the outputs equal :func:`box2d_iou_max` on that frame
+    bit for bit.  Two call forms, like :func:`box2d_iou_batch`: lists of per-frame ``boxes1`` [n_f, 5] / ``boxes2`` [m_f, 5] (returns the
+    list of per-frame ``(max1, idx1, max2, idx2)`` tuples), or the frames packed back to back with ``offsets1`` / ``offsets2`` (int64
+    [nframes + 1], CPU) (returns the packed ``(max1 [total1], idx1 [total1], max2 [total2], idx2 [total2])`` with FRAME-LOCAL indices, as
+    :func:`match_greedy_batch` gives them).  A box whose frame's other side is empty gets value 0 and index -1.  ``method`` ('box' or
+    'rbox') and ``precise`` as in :func:`box2d_iou_max`.  The outputs do not require grad.  numpy in -> numpy out, host tensors in -> host
+    tensors out.
+    '''
+    as_list = isinstance(boxes1, (list, tuple))
+    if as_list:
+        if not isinstance(boxes2, (list, tuple)) or len(boxes1) != len(boxes2):
+            raise ValueError("boxes1 and boxes2 should hold the same number of frames")
+        if len(boxes1) == 0:
+            return []
+        numpy_in = isinstance(boxes1[0], np.ndarray)
+        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
+        l1, l2 = [tt(b) for b in boxes1], [tt(b) for b in boxes2]
+        for a, b in zip(l1, l2):
+            _check_iou2d(a, b)
+        if len({x.dtype for x in l1}) != 1 or len({x.dtype for x in l2}) != 1:
+            raise RuntimeError("the frames of a box set must have the same dtype")
+        off1, off2 = _frame_offsets(lens=[len(b) for b in l1]), _frame_offsets(lens=[len(b) for b in l2])
+        B1, B2 = torch.cat(l1), torch.cat(l2)
+    else:
+        numpy_in = isinstance(boxes1, np.ndarray)
+        if numpy_in:
+            assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
+            boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
+        if offsets1 is None or offsets2 is None:
+            raise ValueError("packed boxes need the frame offsets")
+        _check_iou2d(boxes1, boxes2)
+        off1, off2 = _frame_offsets(offsets1), _frame_offsets(offsets2)
+        B1, B2 = boxes1, boxes2
+    if off1.numel() != off2.numel() or int(off1[-1]) != len(B1) or int(off2[-1]) != len(B2):
+        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
+    m1, i1, m2, i2 = _iou_max_outputs(_iou_max_packed(B1, B2, off1, off2, method, precise), B1.device, numpy_in)
+    if not as_list:
+        return m1, i1, m2, i2
+    return [(m1[int(off1[f]):int(off1[f + 1])], i1[int(off1[f]):int(off1[f + 1])], m2[int(off2[f]):int(off2[f + 1])], i2[int(off2[f]):int(off2[f + 1])])
+            for f in range(off1.numel() - 1)]
+
+
 def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold=0, score_threshold=0, precise=True, offsets_dev=None,
                     supression_method="hard", supression_param=0):
     '''

@@ -100,11 +100,13 @@ __device__ __forceinline__ float z_iou(const ZRange &a, const ZRange &b)
 // pair), so the detection-evaluation matrix costs little more than the IoU matrix.
 // One CTA computes the TR x TC tile at (row0, col0) of the n x m matrix `out` (leading dimension ld); row0 < n and col0 < m.
 // recA / zA hold n rows padded to a multiple of TR, recB / zB m columns padded to a multiple of TC (field-major in blocks of TC).
-// The single-matrix kernel and the frame-batched kernel both run this body, so a pair gets the same reject test and clip in both.
+// The single-matrix kernel, the frame-batched kernel and the max-IoU reduction all run iou2dr_tile_fill, so a pair gets the same reject
+// test and clip in all of them.  It leaves the tile's values in sm.tile: a warp's own rows are complete after __syncwarp (fp32) or
+// __syncthreads (fp64); the whole tile after a __syncthreads.  Every value is +0 (rejected pairs, padding rows and columns), positive
+// or NaN (rbox_iou: ai >= +0 and au > 0, so never negative and never -0).
 template <typename T, bool ZD>
-__device__ __forceinline__ void iou2dr_tile(const BoxRec<T> *__restrict__ recA, int64_t n, const BoxRec<T> *__restrict__ recB, int64_t m,
-                                            T *__restrict__ out, int64_t ld, const ZRange *__restrict__ zA, const ZRange *__restrict__ zB,
-                                            const int64_t row0, const int64_t col0)
+__device__ __forceinline__ void iou2dr_tile_fill(const BoxRec<T> *__restrict__ recA, const BoxRec<T> *__restrict__ recB, const ZRange *__restrict__ zA,
+                                                 const ZRange *__restrict__ zB, const int64_t row0, const int64_t col0)
 {
     using S = IouSmem<T>;
     constexpr int TR = S::TR, TC = S::TC, RW = S::RW, KC = S::KC;
@@ -215,6 +217,20 @@ __device__ __forceinline__ void iou2dr_tile(const BoxRec<T> *__restrict__ recA, 
     }
     if constexpr (CTAQ) __syncthreads();   // other warps clipped candidates of this warp's rows
     else __syncwarp();
+}
+
+template <typename T, bool ZD>
+__device__ __forceinline__ void iou2dr_tile(const BoxRec<T> *__restrict__ recA, int64_t n, const BoxRec<T> *__restrict__ recB, int64_t m,
+                                            T *__restrict__ out, int64_t ld, const ZRange *__restrict__ zA, const ZRange *__restrict__ zB,
+                                            const int64_t row0, const int64_t col0)
+{
+    using S = IouSmem<T>;
+    constexpr int TC = S::TC, RW = S::RW;
+    constexpr int V = 16 / sizeof(T);    // elements per 16-byte vector
+    extern __shared__ __align__(16) unsigned char iou_smem_raw[];
+    S &sm = *reinterpret_cast<S *>(iou_smem_raw);
+    const unsigned lane = lane_id(), w = threadIdx.x >> 5;
+    iou2dr_tile_fill<T, ZD>(recA, recB, zA, zB, row0, col0);
 
     // stream this warp's rows to HBM: full-line 16-byte stores when the row pointers are 16-byte aligned
     const int64_t wrow0 = row0 + w * RW;
@@ -413,6 +429,246 @@ __global__ void __launch_bounds__(256) iou2d_batch_kernel(const AABBRec<T> *__re
     for (int64_t q = (int64_t)blockIdx.y * blockDim.x + threadIdx.x; q < nq; q += (int64_t)gridDim.y * blockDim.x) {
         const int64_t i = q / cm;
         iou2d_cols<T>(recA[a0 + i], recB + b0, m, (q - i * cm) * 4, o, i * m);
+    }
+}
+
+// ------------------------------------------------------------------ fused max-IoU reduction (box2d_iou_max_batch, methods "rbox" / "box")
+// Per box of either set, the largest IoU over the other set of its frame and the frame-local index that attains it, with torch.max's
+// rules on the output dtype O: ties (+0 against -0 included) go to the lower index, NaN is the maximum at the first NaN's index.
+// Tiles reduce their rows and columns to (value, index) keys and combine them across tiles with atomics on an order-preserving key:
+//   hi: the value's bits mapped so that unsigned order is value order (sign flip for >= 0, complement for < 0; -0 maps like +0,
+//       every NaN to the top), lo: the complement of the index, so that a larger key is a larger value or, on a tie, a lower index.
+// fp32 keys pack (hi << 32 | lo) into one 64-bit atomicMax; fp64 keys are 16 bytes, combined by a 16-byte atomicCAS loop (sm_90+).
+// A CAS loop costs retries under contention, but no value is below +0 and keys start at (+0, index 0), so a row or column whose tile
+// maximum is +0 commits nothing: on sparse frames almost every tile, and the loop runs rarely.  The initial key is also the answer
+// of a row whose every value is +0.  EMPTY (key 0, unreachable from a value) marks a box whose frame's other side is empty: (0, -1).
+template <typename O> struct MaxKey;
+template <> struct MaxKey<float> {
+    using K = unsigned long long;
+    static __device__ __forceinline__ K make(float v, int64_t i)
+    {
+        const unsigned b = __float_as_uint(v);
+        const unsigned o = v != v ? 0xffffffffu : v == 0.f ? 0x80000000u : (b >> 31) ? ~b : b | 0x80000000u;
+        return (K)o << 32 | (0xffffffffu - (unsigned)i);
+    }
+    static __device__ __forceinline__ K init() { return 0x80000000ull << 32 | 0xffffffffull; }
+    static __device__ __forceinline__ K empty() { return 0; }
+    static __device__ __forceinline__ bool above(K a, K b) { return a > b; }
+    static __device__ __forceinline__ void commit(K *p, K k) { atomicMax(p, k); }
+    static __device__ __forceinline__ void decode(K k, float *v, int64_t *i)
+    {
+        const unsigned o = (unsigned)(k >> 32);
+        if (o == 0) { *v = 0.f; *i = -1; return; }
+        *v = o == 0xffffffffu ? __uint_as_float(0x7fffffffu) : __uint_as_float((o >> 31) ? o & 0x7fffffffu : ~o);
+        *i = (int64_t)(0xffffffffu - (unsigned)k);
+    }
+};
+struct __align__(16) Key128 { unsigned long long lo, hi; };
+template <> struct MaxKey<double> {
+    using K = Key128;
+    static __device__ __forceinline__ K make(double v, int64_t i)
+    {
+        const unsigned long long b = (unsigned long long)__double_as_longlong(v), sign = 1ull << 63;
+        K k;
+        k.hi = v != v ? ~0ull : v == 0.0 ? sign : (b >> 63) ? ~b : b | sign;
+        k.lo = ~(unsigned long long)i;
+        return k;
+    }
+    static __device__ __forceinline__ K init() { K k; k.hi = 1ull << 63; k.lo = ~0ull; return k; }
+    static __device__ __forceinline__ K empty() { K k; k.hi = 0; k.lo = 0; return k; }
+    static __device__ __forceinline__ bool above(K a, K b) { return a.hi > b.hi || (a.hi == b.hi && a.lo > b.lo); }
+    static __device__ __forceinline__ void commit(K *p, K k)
+    {
+        K old = *p;   // possibly stale: keys only grow, so a stale key is below the current one and the CAS corrects it
+        while (above(k, old)) {
+            const K prev = atomicCAS(p, old, k);
+            if (prev.hi == old.hi && prev.lo == old.lo) break;
+            old = prev;
+        }
+    }
+    static __device__ __forceinline__ void decode(K k, double *v, int64_t *i)
+    {
+        if (k.hi == 0) { *v = 0.0; *i = -1; return; }
+        const unsigned long long sign = 1ull << 63;
+        *v = k.hi == ~0ull ? __longlong_as_double(0x7ff8000000000000ll) : __longlong_as_double((long long)((k.hi & sign) ? k.hi & ~sign : ~k.hi));
+        *i = (int64_t)~k.lo;
+    }
+};
+template <typename O> __device__ __forceinline__ typename MaxKey<O>::K key_max(typename MaxKey<O>::K a, typename MaxKey<O>::K b)
+{
+    return MaxKey<O>::above(b, a) ? b : a;
+}
+
+// every box's key: init(), or empty() when its frame's other side is empty.  Frames on grid.x, the frame's boxes of both sets strided over grid.y.
+template <typename O>
+__global__ void __launch_bounds__(256) iou_max_init_kernel(const int64_t *__restrict__ off1, const int64_t *__restrict__ off2, typename MaxKey<O>::K *__restrict__ key1,
+                                                           typename MaxKey<O>::K *__restrict__ key2)
+{
+    const int64_t f = blockIdx.x, a0 = off1[f], b0 = off2[f], n = off1[f + 1] - a0, m = off2[f + 1] - b0;
+    for (int64_t i = (int64_t)blockIdx.y * blockDim.x + threadIdx.x; i < n + m; i += (int64_t)gridDim.y * blockDim.x) {
+        if (i < n) key1[a0 + i] = m ? MaxKey<O>::init() : MaxKey<O>::empty();
+        else key2[b0 + i - n] = n ? MaxKey<O>::init() : MaxKey<O>::empty();
+    }
+}
+
+// keys -> values and int64 indices, both sets in one flat pass
+template <typename O>
+__global__ void __launch_bounds__(256) iou_max_finalise_kernel(const typename MaxKey<O>::K *__restrict__ key1, int64_t total1, const typename MaxKey<O>::K *__restrict__ key2,
+                                                               int64_t total2, O *__restrict__ max1, int64_t *__restrict__ idx1, O *__restrict__ max2,
+                                                               int64_t *__restrict__ idx2)
+{
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total1 + total2; i += (int64_t)gridDim.x * blockDim.x) {
+        if (i < total1) MaxKey<O>::decode(key1[i], max1 + i, idx1 + i);
+        else MaxKey<O>::decode(key2[i - total1], max2 + i - total1, idx2 + i - total1);
+    }
+}
+
+// Inside a tile the values are compared as their bits in O: every value is +0, positive or NaN (iou2dr_tile_fill, aabb_iou), so with
+// NaN canonicalised the unsigned order of the bits is the value order, +0 is 0 and ties are equal bits.  Keys are built only for commits.
+template <typename O> struct OBits;
+template <> struct OBits<float> {
+    using U = unsigned;
+    static __device__ __forceinline__ U canon(float v) { const U u = __float_as_uint(v); return u > 0x7f800000u ? 0x7fffffffu : u; }
+    static __device__ __forceinline__ float value(U u) { return __uint_as_float(u); }
+};
+template <> struct OBits<double> {
+    using U = unsigned long long;
+    static __device__ __forceinline__ U canon(double v)
+    {
+        const U u = (U)__double_as_longlong(v);
+        return u > 0x7ff0000000000000ull ? 0x7fffffffffffffffull : u;
+    }
+    static __device__ __forceinline__ double value(U u) { return __longlong_as_double((long long)u); }
+};
+
+// rotated: iou2dr_tile_fill's tile, then its row and column maxima instead of the stores.  Frames on grid.x, column tiles ct0 + grid.y,
+// row tiles rt0 + grid.z (slabs of 65535 tiles for larger frames: the keys combine across slabs as across tiles).  Records as for the matrix.
+template <typename T, typename O>
+__global__ void __launch_bounds__(IOU_THREADS, 3)
+iou2dr_max_batch_tile_kernel(const BoxRec<T> *__restrict__ recA, const int64_t *__restrict__ off1, const BoxRec<T> *__restrict__ recB,
+                             const int64_t *__restrict__ off2, int64_t rt0, int64_t ct0, typename MaxKey<O>::K *__restrict__ key1,
+                             typename MaxKey<O>::K *__restrict__ key2)
+{
+    using S = IouSmem<T>;
+    using KT = MaxKey<O>;
+    using K = typename KT::K;
+    using B = OBits<O>;
+    using U = typename B::U;
+    constexpr int TR = S::TR, TC = S::TC, RW = S::RW, KC = S::KC;
+    const int64_t f = blockIdx.x, n = off1[f + 1] - off1[f], m = off2[f + 1] - off2[f];
+    const int64_t row0 = (rt0 + blockIdx.z) * TR, col0 = (ct0 + blockIdx.y) * TC;
+    if (row0 >= n || col0 >= m) return;
+    iou2dr_tile_fill<T, false>(recA + frame_rec_base(off1, f, TR), recB + frame_rec_base(off2, f, TC), nullptr, nullptr, row0, col0);
+    __syncthreads();   // the column maxima read every warp's rows
+    extern __shared__ __align__(16) unsigned char iou_smem_raw[];
+    S &sm = *reinterpret_cast<S *>(iou_smem_raw);
+    const unsigned lane = lane_id(), w = threadIdx.x >> 5;
+    K *krow = key1 + off1[f], *kcol = key2 + off2[f];
+    // rows: warp w owns rows w*RW .. w*RW+RW-1, lane the KC adjacent columns lane*KC ..; the warp's maximum, then the lowest column
+    // holding it.  A row whose maximum is +0 commits nothing (the initial key).  Padding columns hold +0.
+    static_assert(KC * sizeof(T) == 16, "one 16-byte load per lane and row");
+#pragma unroll
+    for (int r = 0; r < RW; r++) {
+        const int row = w * RW + r;
+        T v[KC];
+        *reinterpret_cast<float4 *>(v) = *reinterpret_cast<const float4 *>(&sm.tile[row][lane * KC]);
+        U bu = B::canon((O)v[0]);
+        int bc = 0;
+#pragma unroll
+        for (int c = 1; c < KC; c++) { const U u = B::canon((O)v[c]); if (u > bu) { bu = u; bc = c; } }
+        U mx = bu;
+#pragma unroll
+        for (int d = 16; d; d >>= 1) { const U t = __shfl_xor_sync(0xffffffffu, mx, d); mx = t > mx ? t : mx; }
+        if (mx == 0) continue;
+        int col = bu == mx ? (int)lane * KC + bc : TC;
+#pragma unroll
+        for (int d = 16; d; d >>= 1) col = min(col, __shfl_xor_sync(0xffffffffu, col, d));
+        if (lane == 0 && row0 + row < n) KT::commit(krow + row0 + row, KT::make(B::value(mx), col0 + col));
+    }
+    // columns: PARTS threads per column, RP rows each, combined through the candidate queue's shared memory (free after the clip)
+    constexpr int PARTS = IOU_THREADS / TC, RP = TR / PARTS;
+    static_assert(sizeof(sm.queue) >= IOU_THREADS * sizeof(K), "column partials fit the queue");
+    K *part = reinterpret_cast<K *>(&sm.queue[0][0]);
+    const int c = threadIdx.x % TC, p = threadIdx.x / TC;
+    U bu = B::canon((O)sm.tile[p * RP][c]);
+    int br = 0;
+#pragma unroll 8
+    for (int r = 1; r < RP; r++) { const U u = B::canon((O)sm.tile[p * RP + r][c]); if (u > bu) { bu = u; br = r; } }
+    part[threadIdx.x] = KT::make(B::value(bu), row0 + p * RP + br);
+    __syncthreads();
+    if (threadIdx.x < TC) {
+        K k = part[threadIdx.x];
+#pragma unroll
+        for (int q = 1; q < PARTS; q++) k = key_max<O>(k, part[q * TC + threadIdx.x]);
+        if (col0 + c < m && KT::above(k, KT::init())) KT::commit(kcol + col0 + c, k);
+    }
+}
+
+// axis-aligned: a CTA owns a BR x BC tile of a frame.  Its threads fill the tile in shared memory with iou2d_cols, called as
+// iou2d_batch_kernel calls it (the row record by value, 4 columns from the records): FMA contraction of aabb_iou<T> depends on how the
+// code around it reuses the row's extents, and this shape rounds as the matrix does.  Then rows reduce across the warp and columns
+// across the threads of a column, as in the rotated tile.  Frames on grid.x, row tiles rt0 + grid.y, column tiles ct0 + grid.z.
+// Records are the packed AABBs.
+constexpr int IOU_MAX_BOX_BR = 32, IOU_MAX_BOX_BC = 128;
+template <typename T, typename O>
+__global__ void __launch_bounds__(256) iou2d_max_batch_kernel(const AABBRec<T> *__restrict__ recA, const int64_t *__restrict__ off1,
+                                                              const AABBRec<T> *__restrict__ recB, const int64_t *__restrict__ off2, int64_t rt0,
+                                                              int64_t ct0, typename MaxKey<O>::K *__restrict__ key1, typename MaxKey<O>::K *__restrict__ key2)
+{
+    using KT = MaxKey<O>;
+    using K = typename KT::K;
+    using B = OBits<O>;
+    using U = typename B::U;
+    constexpr int BR = IOU_MAX_BOX_BR, BC = IOU_MAX_BOX_BC, RW = BR / 8, PARTS = 256 / BC, RP = BR / PARTS;
+    __shared__ __align__(16) T tile[BR][BC];
+    __shared__ K part[256];
+    const int64_t f = blockIdx.x, a0 = off1[f], b0 = off2[f], n = off1[f + 1] - a0, m = off2[f + 1] - b0;
+    const int64_t row0 = (rt0 + blockIdx.y) * BR, col0 = (ct0 + blockIdx.z) * BC;
+    if (row0 >= n || col0 >= m) return;
+    const int nr = (int)(n - row0 < BR ? n - row0 : BR), nc = (int)(m - col0 < BC ? m - col0 : BC);
+    for (int q = threadIdx.x; q < BR * (BC / 4); q += 256) {
+        const int r = q / (BC / 4), c4 = q % (BC / 4);
+        if (r < nr) iou2d_cols<T>(recA[a0 + row0 + r], recB + b0 + col0, nc, c4 * 4, &tile[0][0], r * BC);
+    }
+    __syncthreads();
+    const unsigned lane = lane_id(), w = threadIdx.x >> 5;
+    // rows: warp w owns rows w*RW ..; lane the 4 adjacent columns lane*4 ..
+#pragma unroll
+    for (int rr = 0; rr < RW; rr++) {
+        const int r = w * RW + rr;
+        U bu = 0;
+        int bc = 0;
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const int col = (int)lane * 4 + c;
+            const U u = r < nr && col < nc ? B::canon((O)tile[r][col]) : U(0);
+            if (u > bu) { bu = u; bc = col; }
+        }
+        U mx = bu;
+#pragma unroll
+        for (int d = 16; d; d >>= 1) { const U t = __shfl_xor_sync(0xffffffffu, mx, d); mx = t > mx ? t : mx; }
+        if (mx == 0) continue;
+        int col = bu == mx ? bc : BC;
+#pragma unroll
+        for (int d = 16; d; d >>= 1) col = min(col, __shfl_xor_sync(0xffffffffu, col, d));
+        if (lane == 0) KT::commit(key1 + a0 + row0 + r, KT::make(B::value(mx), col0 + col));
+    }
+    // columns: PARTS threads per column, RP rows each
+    const int c = threadIdx.x % BC, p = threadIdx.x / BC;
+    U bu = 0;
+    int br = 0;
+#pragma unroll 4
+    for (int r = 0; r < RP; r++) {
+        const U u = p * RP + r < nr && c < nc ? B::canon((O)tile[p * RP + r][c]) : U(0);
+        if (u > bu) { bu = u; br = r; }
+    }
+    part[threadIdx.x] = bu ? KT::make(B::value(bu), row0 + p * RP + br) : KT::init();
+    __syncthreads();
+    if ((int)threadIdx.x < nc) {
+        K k = part[threadIdx.x];
+#pragma unroll
+        for (int q = 1; q < PARTS; q++) k = key_max<O>(k, part[q * BC + threadIdx.x]);
+        if (KT::above(k, KT::init())) KT::commit(key2 + b0 + col0 + threadIdx.x, k);
     }
 }
 
@@ -663,6 +919,87 @@ static int iou_batch_impl(const T *b1, int64_t total1, const int64_t *off1, cons
     return D3D_OK;
 }
 
+// the records of iou_batch_ws_bytes, then one key per box of each set (sized for the larger fp64 key when the inputs are fp64)
+template <typename T> static size_t iou_max_batch_ws_bytes(int64_t total1, int64_t total2, int64_t nframes)
+{
+    if (total1 < 0 || total2 < 0 || nframes < 0) return 0;
+    return iou_batch_ws_bytes<T>(total1, total2, nframes) + align_up((size_t)total1 * sizeof(typename MaxKey<T>::K)) +
+           align_up((size_t)total2 * sizeof(typename MaxKey<T>::K));
+}
+
+template <typename T, typename O>
+static int iou_max_batch_run(const T *b1, int64_t total1, const int64_t *off1, const T *b2, int64_t total2, const int64_t *off2, int64_t nframes,
+                             int64_t max1, int64_t max2, int iou_type, O *max1o, int64_t *idx1, O *max2o, int64_t *idx2, void *ws, size_t ws_bytes,
+                             cudaStream_t st)
+{
+    using K = typename MaxKey<O>::K;
+    constexpr int TR = IouTile<T>::TR, TC = IouTile<T>::TC;
+    if (sizeof(O) == 4 && (max1 > 0xffffffffll || max2 > 0xffffffffll)) return D3D_ERR_UNSUPPORTED;   // the fp32 key holds a 32-bit index
+    Arena a(ws, ws_bytes);
+    a.take<char>(256);
+    BoxRec<T> *ra = a.take<BoxRec<T>>(total1 + nframes * TR), *rb = a.take<BoxRec<T>>(total2 + nframes * TC);
+    K *k1 = reinterpret_cast<K *>(a.take<typename MaxKey<T>::K>(total1)), *k2 = reinterpret_cast<K *>(a.take<typename MaxKey<T>::K>(total2));
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    const unsigned nf = (unsigned)nframes;
+    iou_max_init_kernel<O><<<dim3(nf, stride_blocks(max1 + max2, 256)), 256, 0, st>>>(off1, off2, k1, k2); D3D_LAUNCHED();
+    if (total1 > 0 && total2 > 0) {
+        if (iou_type == D3D_IOU_BOX) {
+            AABBRec<T> *aa = reinterpret_cast<AABBRec<T> *>(ra), *ab = reinterpret_cast<AABBRec<T> *>(rb);
+            aabb_prep_kernel<T><<<(unsigned)cdiv(total1, 256), 256, 0, st>>>(b1, total1, aa); D3D_LAUNCHED();
+            aabb_prep_kernel<T><<<(unsigned)cdiv(total2, 256), 256, 0, st>>>(b2, total2, ab); D3D_LAUNCHED();
+            const int64_t tr = cdiv(max1, IOU_MAX_BOX_BR), tc = cdiv(max2, IOU_MAX_BOX_BC);
+            for (int64_t r0 = 0; r0 < tr; r0 += 65535)
+                for (int64_t c0 = 0; c0 < tc; c0 += 65535) {
+                    const dim3 grid(nf, (unsigned)(tr - r0 < 65535 ? tr - r0 : 65535), (unsigned)(tc - c0 < 65535 ? tc - c0 : 65535));
+                    iou2d_max_batch_kernel<T, O><<<grid, 256, 0, st>>>(aa, off1, ab, off2, r0, c0, k1, k2); D3D_LAUNCHED();
+                }
+        } else {
+            const int64_t tr = cdiv(max1, TR), tc = cdiv(max2, TC);
+            box_prep_batch_kernel<T, 0><<<dim3(nf, stride_blocks(tr * TR, 256)), 256, 0, st>>>(b1, off1, TR, max1, ra); D3D_LAUNCHED();
+            box_prep_batch_kernel<T, TC><<<dim3(nf, stride_blocks(tc * TC, 256)), 256, 0, st>>>(b2, off2, TC, max2, rb); D3D_LAUNCHED();
+            static bool smem_opt_in[64] = {};   // per instantiation and per device
+            int dev = 0;
+            D3D_CUDA_TRY(cudaGetDevice(&dev));
+            if (dev < 0 || dev >= 64 || !smem_opt_in[dev]) {
+                D3D_CUDA_TRY(cudaFuncSetAttribute(iou2dr_max_batch_tile_kernel<T, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IouSmem<T>)));
+                if (dev >= 0 && dev < 64) smem_opt_in[dev] = true;
+            }
+            for (int64_t r0 = 0; r0 < tr; r0 += 65535)
+                for (int64_t c0 = 0; c0 < tc; c0 += 65535) {
+                    const dim3 grid(nf, (unsigned)(tc - c0 < 65535 ? tc - c0 : 65535), (unsigned)(tr - r0 < 65535 ? tr - r0 : 65535));
+                    iou2dr_max_batch_tile_kernel<T, O><<<grid, IOU_THREADS, sizeof(IouSmem<T>), st>>>(ra, off1, rb, off2, r0, c0, k1, k2); D3D_LAUNCHED();
+                }
+        }
+    }
+    iou_max_finalise_kernel<O><<<stride_blocks(total1 + total2, 256), 256, 0, st>>>(k1, total1, k2, total2, max1o, idx1, max2o, idx2); D3D_LAUNCHED();
+    return D3D_OK;
+}
+
+// per box of a packed batch, the maximum IoU over the other set of its frame and its index: an init, two preparations, the tile
+// launches (one per slab of 65535 x 65535 tiles) and a finalise, whatever the number of frames
+template <typename T>
+static int iou_max_batch_impl(const T *b1, int64_t total1, const int64_t *off1, const T *b2, int64_t total2, const int64_t *off2, int64_t nframes,
+                              int64_t max1, int64_t max2, int iou_type, int out_dtype, void *max1o, int64_t *idx1, void *max2o, int64_t *idx2,
+                              void *ws, size_t ws_bytes, cudaStream_t st)
+{
+    if (iou_type != D3D_IOU_BOX && iou_type != D3D_IOU_RBOX) return D3D_ERR_INVALID_ARGUMENT;
+    if (out_dtype != D3D_F32 && !(sizeof(T) == 8 && out_dtype == D3D_F64)) return D3D_ERR_INVALID_ARGUMENT;
+    if (total1 < 0 || total2 < 0 || nframes < 0 || max1 < 0 || max2 < 0) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes == 0 || total1 + total2 == 0) return D3D_OK;   // no box
+    if (!off1 || !off2 || (total1 && (!b1 || !max1o || !idx1)) || (total2 && (!b2 || !max2o || !idx2))) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes > 0x7fffffffll) return D3D_ERR_UNSUPPORTED;
+    if (ws_bytes < iou_max_batch_ws_bytes<T>(total1, total2, nframes) || !ws) return D3D_ERR_WORKSPACE;
+    if (max1 == 0) max1 = total1;   // 0: bound unknown
+    if (max2 == 0) max2 = total2;
+    if constexpr (sizeof(T) == 8) {
+        if (out_dtype == D3D_F64)
+            return iou_max_batch_run<T, double>(b1, total1, off1, b2, total2, off2, nframes, max1, max2, iou_type, (double *)max1o, idx1, (double *)max2o,
+                                                idx2, ws, ws_bytes, st);
+    }
+    return iou_max_batch_run<T, float>(b1, total1, off1, b2, total2, off2, nframes, max1, max2, iou_type, (float *)max1o, idx1, (float *)max2o, idx2,
+                                       ws, ws_bytes, st);
+}
+
 template <typename T>
 static int count_cand_impl(const T *b1, int64_t n, const T *b2, int64_t m, unsigned long long *counters64, void *ws, size_t ws_bytes, cudaStream_t st)
 {
@@ -726,6 +1063,20 @@ extern "C" size_t d3d_box2d_iou_batch_workspace_bytes(int64_t total1, int64_t to
     }
 D3D_IOU_BATCH_ENTRY(d3d_box2d_iou_batch_f32, float)
 D3D_IOU_BATCH_ENTRY(d3d_box2d_iou_batch_f64, double)
+extern "C" size_t d3d_box2d_iou_max_batch_workspace_bytes(int64_t total1, int64_t total2, int64_t nframes, int dtype)
+{
+    return dtype == D3D_F64 ? iou_max_batch_ws_bytes<double>(total1, total2, nframes) : iou_max_batch_ws_bytes<float>(total1, total2, nframes);
+}
+#define D3D_IOU_MAX_BATCH_ENTRY(NAME, T)                                                                                                   \
+    extern "C" int NAME(const T *boxes1, int64_t total1, const int64_t *offsets1, const T *boxes2, int64_t total2, const int64_t *offsets2,  \
+                        int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type, int out_dtype, void *max1, int64_t *idx1,      \
+                        void *max2, int64_t *idx2, void *ws, size_t wsb, void *stream)                                                     \
+    {                                                                                                                                  \
+        return iou_max_batch_impl<T>(boxes1, total1, offsets1, boxes2, total2, offsets2, nframes, max_frame1, max_frame2, iou_type,    \
+                                     out_dtype, max1, idx1, max2, idx2, ws, wsb, (cudaStream_t)stream);                                \
+    }
+D3D_IOU_MAX_BATCH_ENTRY(d3d_box2d_iou_max_batch_f32, float)
+D3D_IOU_MAX_BATCH_ENTRY(d3d_box2d_iou_max_batch_f64, double)
 extern "C" int d3d_iou_count_candidates(const void *b1, int64_t n, const void *b2, int64_t m, int dtype, uint64_t *counters64, void *ws, size_t wsb, void *stream)
 {
     return dtype == D3D_F64 ? count_cand_impl<double>((const double *)b1, n, (const double *)b2, m, (unsigned long long *)counters64, ws, wsb, (cudaStream_t)stream)

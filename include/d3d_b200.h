@@ -141,6 +141,27 @@ int d3d_box2d_iou_batch_backward_f32(const float *boxes1, int64_t total1, const 
 int d3d_box2d_iou_batch_backward_f64(const double *boxes1, int64_t total1, const int64_t *offsets1, const double *boxes2, int64_t total2,
                                      const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type,
                                      const int64_t *out_offsets, const double *grad, double *grad_boxes1, double *grad_boxes2, void *stream);
+/* Fused max-IoU reduction (target assignment: each anchor / proposal's best ground truth and each ground truth's best anchor), without
+ * the IoU matrix.  Boxes, offsets, max_frame1 / max_frame2 and iou_type as for d3d_box2d_iou_batch_*, except that iou_type is D3D_IOU_BOX
+ * or D3D_IOU_RBOX only.  Outputs: max1 [total1] / idx1 i64[total1] and max2 [total2] / idx2 i64[total2] (DEVICE), of dtype out_dtype:
+ * D3D_F32, or D3D_F64 for the f64 entry (fp32 boxes computed in fp64 and rounded to fp32: pass fp64 boxes and D3D_F32).  For box i of
+ * frame f, max1[i] / idx1[i] are the value and FRAME-LOCAL column index that torch.max(block, dim=1) returns for frame f's block of
+ * d3d_box2d_iou_batch_* rounded to out_dtype; max2 / idx2 those of dim=0.  So ties (+0 against -0 included) go to the lower index, and
+ * NaN is the maximum, at the first NaN's index.  A box whose frame's other side is empty gets (0, -1).  Rows and columns reduce inside
+ * the tiles and combine across tiles through atomics on an order-preserving (value, index) key; the result does not depend on the
+ * schedule.  Every frame size works: frames of more than 65535 tiles on an axis take more than one tile launch.  An init, two box
+ * preparations, the tile launches (one per 65535 x 65535 tiles of the largest frame) and a finalise, whatever the number of frames.
+ * max_frame1 / max_frame2 are HARD UPPER BOUNDS (0 = unknown, assume total1 / total2); a frame beyond them has undefined results.
+ * Invalid iou_type or out_dtype, or negative sizes: D3D_ERR_INVALID_ARGUMENT; workspace below d3d_box2d_iou_max_batch_workspace_bytes
+ * (dtype = the boxes' dtype): D3D_ERR_WORKSPACE; nframes > 2^31 - 1, or a D3D_F32 output with a frame of 2^32 boxes or more:
+ * D3D_ERR_UNSUPPORTED.  nframes == 0 or no box: no-op. */
+size_t d3d_box2d_iou_max_batch_workspace_bytes(int64_t total1, int64_t total2, int64_t nframes, int dtype);
+int d3d_box2d_iou_max_batch_f32(const float *boxes1, int64_t total1, const int64_t *offsets1, const float *boxes2, int64_t total2,
+                                const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type, int out_dtype,
+                                void *max1, int64_t *idx1, void *max2, int64_t *idx2, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_box2d_iou_max_batch_f64(const double *boxes1, int64_t total1, const int64_t *offsets1, const double *boxes2, int64_t total2,
+                                const int64_t *offsets2, int64_t nframes, int64_t max_frame1, int64_t max_frame2, int iou_type, int out_dtype,
+                                void *max1, int64_t *idx1, void *max2, int64_t *idx2, void *workspace, size_t workspace_bytes, void *stream);
 /* Detection-evaluation distance matrix (SURVEY.md 8(f) row f1): dist[i][j] = 1 - iou2d(BEV boxes) * ziou, fp32,
  * for 3-D boxes [n,7] / [m,7] with rows (x, y, z, lx, ly, lz, rz).  rotated != 0: rotated BEV IoU, replaces the pair
  * loop over box3dr_iou in ScoreMatcher.prepare_boxes (reference d3d/tracking/matcher.pyx:66-76, d3d/dgal_wrap.h:45-68);
