@@ -66,6 +66,10 @@ crop_grid_min_pairs = _sig("d3d_crop2dr_grid_min_pairs", _i64, [])
 crop_batch_workspace_bytes = _sig("d3d_crop2dr_batch_workspace_bytes", _sz, [_i64, C.c_int])
 _pbb_sig = [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i64, _i64, C.c_int, _vp]   # packed points / boxes, offsets, bounds, axis, out offsets
 crop2dr_batch = {k: _sig(f"d3d_crop2dr_batch_{s}", C.c_int, _pbb_sig + [_vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+crop_assign_workspace_bytes = _sig("d3d_crop2dr_assign_workspace_bytes", _sz, [_i64, _i64, C.c_int])
+crop2dr_assign = {k: _sig(f"d3d_crop2dr_assign_{s}", C.c_int, [_vp, _i64, _vp, _i64, C.c_int, _vp, _vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
+crop_assign_batch_workspace_bytes = _sig("d3d_crop2dr_assign_batch_workspace_bytes", _sz, [_i64, C.c_int])
+crop2dr_assign_batch = {k: _sig(f"d3d_crop2dr_assign_batch_{s}", C.c_int, _pbb_sig[:-1] + [_vp, _vp, _vp, _sz, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 pdist2dr_batch = {k: _sig(f"d3d_pdist2dr_batch_{s}", C.c_int, _pbb_sig + [_vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 pdist2dr_batch_backward = {k: _sig(f"d3d_pdist2dr_batch_backward_{s}", C.c_int, _pbb_sig + [_vp, _vp, _vp, _vp]) for k, s in ((F32, "f32"), (F64, "f64"))}
 _iex_sig = [_vp, _i64, _vp, _i64, _vp, _i64, _vp]

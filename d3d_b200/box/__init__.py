@@ -331,7 +331,8 @@ def _iou_max_packed(B1, B2, off1, off2, method, precise):
     return max1, idx1, max2, idx2
 
 
-def _iou_max_outputs(outs, odev, numpy_in):
+def _reduction_outputs(outs, odev, numpy_in):
+    """device outputs of a fused reduction on the inputs' side (numpy, host or device)"""
     if odev.type != "cuda" or numpy_in:
         outs = tuple(x.cpu() for x in outs)
     return tuple(x.numpy() for x in outs) if numpy_in else tuple(outs)
@@ -358,7 +359,7 @@ def box2d_iou_max(boxes1, boxes2, method="box", precise=True):
         boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
     _check_iou2d(boxes1, boxes2)
     off1, off2 = _frame_offsets(lens=[len(boxes1)]), _frame_offsets(lens=[len(boxes2)])
-    return _iou_max_outputs(_iou_max_packed(boxes1, boxes2, off1, off2, method, precise), boxes1.device, numpy_in)
+    return _reduction_outputs(_iou_max_packed(boxes1, boxes2, off1, off2, method, precise), boxes1.device, numpy_in)
 
 
 def box2d_iou_max_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", precise=True):
@@ -398,7 +399,7 @@ def box2d_iou_max_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="bo
         B1, B2 = boxes1, boxes2
     if off1.numel() != off2.numel() or int(off1[-1]) != len(B1) or int(off2[-1]) != len(B2):
         raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
-    m1, i1, m2, i2 = _iou_max_outputs(_iou_max_packed(B1, B2, off1, off2, method, precise), B1.device, numpy_in)
+    m1, i1, m2, i2 = _reduction_outputs(_iou_max_packed(B1, B2, off1, off2, method, precise), B1.device, numpy_in)
     if not as_list:
         return m1, i1, m2, i2
     return [(m1[int(off1[f]):int(off1[f + 1])], i1[int(off1[f]):int(off1[f + 1])], m2[int(off2[f]):int(off2[f + 1])], i2[int(off2[f]):int(off2[f + 1])])
@@ -781,6 +782,115 @@ def box3dp_crop_batch(points, boxes, point_offsets=None, box_offsets=None, proje
     if isinstance(points, (list, tuple)) and len(points) == 0:
         return []
     return _crop_batch(points, boxes, point_offsets, box_offsets, project_axis)
+
+
+def _crop_assign_frame(p, b, project_axis, point_box, box_npoints):
+    """one frame's reductions on the device, written into the given int64 slices (the single-frame entry: grid path on large frames)"""
+    code = _c.dtype_code(p.dtype)
+    n, m = len(p), len(b)
+    if n or m:
+        ws = _c.workspace(_c.crop_assign_workspace_bytes(n, m, code) if n and m else 0, p.device)
+        with torch.cuda.device(p.device):
+            st = _c.crop2dr_assign[code](_c.ptr(p), n, _c.ptr(b), m, project_axis, _c.ptr(point_box), _c.ptr(box_npoints), _c.ptr(ws), ws.numel(),
+                                         _c.stream_ptr())
+        _c.check(st, "box2dr_crop_assign" if project_axis < 0 else "box3dp_crop_assign")
+
+
+def _crop_assign(points, boxes, project_axis):
+    check = _check_crop2d if project_axis < 0 else _check_3d
+    numpy_in = isinstance(points, np.ndarray)
+    if numpy_in:
+        assert isinstance(boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
+        points, boxes = torch.from_numpy(points), torch.from_numpy(boxes)
+    check(points, boxes)
+    _c.dtype_code(points.dtype)
+    if boxes.dtype != points.dtype:
+        raise RuntimeError("points and boxes must have the same dtype")
+    odev = points.device
+    P, B = _c.to_device(points.detach()), _c.to_device(boxes.detach())
+    point_box = torch.empty(len(P), dtype=torch.int64, device=P.device)
+    box_npoints = torch.empty(len(B), dtype=torch.int64, device=P.device)
+    _crop_assign_frame(P, B, project_axis, point_box, box_npoints)
+    return _reduction_outputs((point_box, box_npoints), odev, numpy_in)
+
+
+def box2dr_crop_assign(points, boxes):
+    '''
+    The two reductions of :func:`box2dr_crop`'s mask that point labels and box filters use, without the mask.  Returns
+    ``(point_box, box_npoints)``: ``point_box`` int64 [N] is the lowest index of a box containing each point, or -1 if there is none
+    (``torch.where(mask.any(0), mask.to(torch.uint8).argmax(0), -1)``), and ``box_npoints`` int64 [M] the number of points inside each box
+    (``mask.sum(1)``), both exactly equal to those of the mask.  The outputs carry no grad.  numpy in -> numpy out, host tensors in -> host
+    tensors out.
+
+    :param points: The input points, shape: N x 2
+    :param boxes: Input boxes array, shape: M x 5
+    '''
+    return _crop_assign(points, boxes, -1)
+
+
+def box3dp_crop_assign(points, boxes, project_axis=2):
+    '''
+    :func:`box2dr_crop_assign` for :func:`box3dp_crop`'s mask: points [N, 3], boxes [M, 7] projected to ``project_axis``.
+
+    :param points: The input points, shape: N x 3
+    :param boxes: Input boxes array, shape: M x 7
+    :param project_axis: Axis for the box to be projected to. {0: x, 1: y, 2: z}
+    '''
+    _check_axis(project_axis)
+    return _crop_assign(points, boxes, project_axis)
+
+
+def _crop_assign_batch(points, boxes, point_offsets, box_offsets, project_axis):
+    check = _check_crop2d if project_axis < 0 else _check_3d
+    P, B, poff, boff, as_list, numpy_in, odev = _point_box_inputs(points, boxes, point_offsets, box_offsets, check)
+    P, B = P.detach().contiguous(), B.detach().contiguous()
+    code = _c.dtype_code(P.dtype)
+    nframes = poff.numel() - 1
+    n_f, m_f = poff[1:] - poff[:-1], boff[1:] - boff[:-1]
+    point_box = torch.empty(len(P), dtype=torch.int64, device=P.device)
+    box_npoints = torch.empty(len(B), dtype=torch.int64, device=P.device)
+    big = n_f * m_f >= int(_c.crop_grid_min_pairs())   # the single-frame entry (grid path) computes these
+    small = (n_f * m_f > 0) & ~big
+    if nframes and len(P) + len(B):
+        offs = torch.cat([poff, boff]).to(P.device, non_blocking=True)   # one copy of both offset arrays
+        ws = _c.workspace(_c.crop_assign_batch_workspace_bytes(len(B), code), P.device)
+        any_small = bool(small.any())
+        with torch.cuda.device(P.device):
+            st = _c.crop2dr_assign_batch[code](_c.ptr(P), len(P), _c.ptr(offs[:nframes + 1]), _c.ptr(B), len(B), _c.ptr(offs[nframes + 1:]), nframes,
+                                               int(n_f[small].max()) if any_small else 1, int(m_f[small].max()) if any_small else 1, project_axis,
+                                               _c.ptr(point_box), _c.ptr(box_npoints), _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        _c.check(st, "box2dr_crop_assign_batch" if project_axis < 0 else "box3dp_crop_assign_batch")
+    for f in torch.nonzero(big).flatten().tolist():   # after the batch call, which initialises every slice
+        p0, p1, b0, b1 = int(poff[f]), int(poff[f + 1]), int(boff[f]), int(boff[f + 1])
+        _crop_assign_frame(P[p0:p1], B[b0:b1], project_axis, point_box[p0:p1], box_npoints[b0:b1])
+    pb, bn = _reduction_outputs((point_box, box_npoints), odev, numpy_in)
+    if not as_list:
+        return pb, bn
+    return [(pb[int(poff[f]):int(poff[f + 1])], bn[int(boff[f]):int(boff[f + 1])]) for f in range(nframes)]
+
+
+def box2dr_crop_assign_batch(points, boxes, point_offsets=None, box_offsets=None):
+    '''
+    :func:`box2dr_crop_assign` on a batch of frames in one launch sequence; per frame the outputs equal :func:`box2dr_crop_assign` on that
+    frame exactly.  Two call forms, like :func:`box2dr_crop_batch`: lists of per-frame ``points`` [N_f, 2] / ``boxes`` [M_f, 5] (returns the
+    list of per-frame ``(point_box, box_npoints)`` tuples), or the frames packed back to back with ``point_offsets`` / ``box_offsets``
+    (int64 [nframes + 1], CPU) (returns the packed ``(point_box [total_points], box_npoints [total_boxes])``, with FRAME-LOCAL box indices
+    as :func:`box2d_iou_max_batch` gives them).  The outputs carry no grad.  numpy in -> numpy out, host tensors in -> host tensors out.
+    '''
+    if isinstance(points, (list, tuple)) and len(points) == 0:
+        return []
+    return _crop_assign_batch(points, boxes, point_offsets, box_offsets, -1)
+
+
+def box3dp_crop_assign_batch(points, boxes, point_offsets=None, box_offsets=None, project_axis=2):
+    '''
+    :func:`box3dp_crop_assign` on a batch of frames: points [N_f, 3], boxes [M_f, 7]; call forms and outputs as
+    :func:`box2dr_crop_assign_batch`, and per frame the outputs equal :func:`box3dp_crop_assign` on that frame exactly.
+    '''
+    _check_axis(project_axis)
+    if isinstance(points, (list, tuple)) and len(points) == 0:
+        return []
+    return _crop_assign_batch(points, boxes, point_offsets, box_offsets, project_axis)
 
 
 class _PDistBatch(torch.autograd.Function):

@@ -241,10 +241,17 @@ __device__ __forceinline__ void crop_cells(const CropBox<T> &B, const CropGrid &
     *y0 = crop_cell(ly, G.miny, G.invy); *y1 = crop_cell(hy, G.miny, G.invy);
 }
 
-// all 32 lanes of a warp call this with the same box; thread-private: first (its first candidate) -- candidates first, first + stride, ... are its own
-template <typename T>
+// the mask's hit action: a 1 in the box's row
+template <typename T> struct CropMaskHit {
+    uint8_t *__restrict__ row;
+    __device__ __forceinline__ void operator()(const CropPt<T> &p) const { row[p.idx] = 1; }
+};
+
+// all 32 lanes of a warp call this with the same box; thread-private: first (its first candidate) -- candidates first, first + stride, ... are its own.
+// hit(p) runs for every candidate p inside the box.
+template <typename T, typename Hit>
 __device__ __forceinline__ void crop_walk(const CropBox<T> &B, int x0, int x1, int y0, int y1, const CropPt<T> *__restrict__ sorted,
-                                          const uint32_t *__restrict__ cellptr, uint8_t *__restrict__ row, uint32_t first, uint32_t stride)
+                                          const uint32_t *__restrict__ cellptr, Hit &hit, uint32_t first, uint32_t stride)
 {
     const unsigned lane = threadIdx.x & 31;
     for (int yb = y0; yb <= y1; yb += 32) {
@@ -271,7 +278,7 @@ __device__ __forceinline__ void crop_walk(const CropBox<T> &B, int x0, int x1, i
 #pragma unroll
             for (int u = 0; u < 4; u++) if (ok[u]) p[u] = sorted[k[u]];
 #pragma unroll
-            for (int u = 0; u < 4; u++) if (ok[u] && crop_inside<T>(B, p[u].x, p[u].y)) row[p[u].idx] = 1;
+            for (int u = 0; u < 4; u++) if (ok[u] && crop_inside<T>(B, p[u].x, p[u].y)) hit(p[u]);
         }
     }
 }
@@ -304,7 +311,8 @@ __global__ void __launch_bounds__(256) crop_hits_kernel(const CropPt<T> *__restr
         if (lane < ns) heavy_item[base + lane] = make_uint2((uint32_t)i, lane | (ns << 16));
         return;
     }
-    crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, mask + i * n, lane, 32u);
+    CropMaskHit<T> hit{mask + i * n};
+    crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, hit, lane, 32u);
 }
 
 template <typename T>
@@ -322,7 +330,8 @@ __global__ void __launch_bounds__(CROP_HT) crop_heavy_kernel(const CropPt<T> *__
         const CropBox<T> B = recs[i];
         int x0, x1, y0, y1;
         crop_cells<T>(B, G, &x0, &x1, &y0, &y1);
-        crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, mask + i * n, j * CROP_HT + threadIdx.x, ns * CROP_HT);
+        CropMaskHit<T> hit{mask + i * n};
+        crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, hit, j * CROP_HT + threadIdx.x, ns * CROP_HT);
     }
 }
 
@@ -542,6 +551,276 @@ static int crop_batch_impl(const T *pts, int64_t total_pts, const int64_t *poff,
     return D3D_OK;
 }
 
+// ------------------------------------------------------------------ fused reductions of the mask
+// point_box[j] = the lowest frame-local index of a box whose mask entry for point j is 1, or -1; box_npoints[i] = the number of points
+// in box i.  Nothing of the mask is stored.  The outputs are handled as unsigned 64-bit words: -1 is the all-ones word, so the per-point
+// result is an unsigned atomicMin into an output filled with 0xff bytes (no finalise pass), and the counts are atomicAdds into a zeroed
+// output.  The decision per pair is the mask's: crop_inside, and for 3-D rows the same rounded test along the axis.
+typedef unsigned long long u64;
+
+// crop2dr_batch_kernel's tiles and frame mapping (frames on grid.x; poff == nullptr: one frame of n1 points and m1 boxes).  A thread
+// decides its 16 points against each box of the tile as a 16-bit word; hits are rare, so a warp votes first and only a warp with a hit
+// reduces: its count goes to a shared counter per box (one global atomic per box and CTA at the end of the box tile), and each point
+// not already claimed by a lower box of the tile takes an atomicMin.  Frames of skip_pairs pairs or more are left to the grid path.
+template <typename T, bool P3>
+__global__ void __launch_bounds__(CROP_THREADS) crop_assign_tile_kernel(const T *__restrict__ pts, const int64_t *__restrict__ poff, int64_t n1,
+                                                                        const CropBox<T> *__restrict__ recs, const CropZ<T> *__restrict__ zr,
+                                                                        const int64_t *__restrict__ boff, int64_t m1, int axis, int64_t skip_pairs,
+                                                                        const CropGrid *__restrict__ skip_if_grid, u64 *__restrict__ point_box,
+                                                                        u64 *__restrict__ box_npoints)
+{
+    if (skip_if_grid && crop_grid_ok(skip_if_grid)) return;   // the grid path produced the outputs
+    __shared__ CropBox<T> sb[CROP_BT];
+    __shared__ CropZ<T> sz[P3 ? CROP_BT : 1];
+    __shared__ uint32_t scnt[CROP_BT];
+    const int64_t f = blockIdx.x;
+    const int64_t j0 = poff ? poff[f] : 0, n = poff ? poff[f + 1] - j0 : n1, i0 = boff ? boff[f] : 0, m = boff ? boff[f + 1] - i0 : m1;
+    if (n * m >= skip_pairs) return;
+    const int64_t tiles_p = (n + CROP_THREADS * CROP_PPT - 1) / (CROP_THREADS * CROP_PPT), tiles_b = (m + CROP_BT - 1) / CROP_BT;
+    if ((int64_t)blockIdx.y >= tiles_p || (int64_t)blockIdx.z >= tiles_b) return;
+    int pa = 0, pb = 1;
+    if (P3) proj_plane(axis, &pa, &pb);
+    constexpr int PS = P3 ? 3 : 2;   // point row length
+    const unsigned lane = threadIdx.x & 31;
+    for (int64_t tb = blockIdx.z; tb < tiles_b; tb += gridDim.z) {
+        const int64_t box0 = tb * CROP_BT;
+        const int nb = (int)(m - box0 < CROP_BT ? m - box0 : CROP_BT);
+        __syncthreads();
+        for (int i = threadIdx.x; i < nb * (int)(sizeof(CropBox<T>) / sizeof(T)); i += CROP_THREADS)
+            reinterpret_cast<T *>(sb)[i] = reinterpret_cast<const T *>(recs + i0 + box0)[i];
+        if (P3 && threadIdx.x < nb) sz[threadIdx.x] = zr[i0 + box0 + threadIdx.x];
+        if (threadIdx.x < CROP_BT) scnt[threadIdx.x] = 0u;
+        __syncthreads();
+        for (int64_t tp = blockIdx.y; tp < tiles_p; tp += gridDim.y) {
+            const int64_t p0 = (tp * CROP_THREADS + threadIdx.x) * CROP_PPT;
+            // threads past the frame's end stay for the warp votes, with no valid point
+            const int np = p0 >= n ? 0 : (n - p0 < CROP_PPT ? (int)(n - p0) : CROP_PPT);
+            const uint32_t valid = (1u << np) - 1u;
+            T px[CROP_PPT], py[CROP_PPT], pz[P3 ? CROP_PPT : 1];
+#pragma unroll
+            for (int k = 0; k < CROP_PPT; k++) {
+                const int64_t j = j0 + (p0 + k < n ? p0 + k : n - 1);
+                px[k] = pts[PS * j + pa]; py[k] = pts[PS * j + pb];
+                if (P3) pz[k] = pts[PS * j + axis];
+            }
+            uint32_t seen = 0u;   // points already claimed by a lower box of this tile
+            for (int b = 0; b < nb; b++) {
+                const CropBox<T> B = sb[b];
+                uint32_t hb = 0u;
+#pragma unroll
+                for (int k = 0; k < CROP_PPT; k++) {
+                    bool in = crop_inside<T>(B, px[k], py[k]);
+                    if (P3) in = in && rn_sub(pz[k], sz[b].hd) < sz[b].c && sz[b].c < rn_add(pz[k], sz[b].hd);
+                    hb |= (in ? 1u : 0u) << k;
+                }
+                hb &= valid;
+                if (__any_sync(0xffffffffu, hb != 0u)) {
+                    const uint32_t c = __reduce_add_sync(0xffffffffu, (uint32_t)__popc(hb));
+                    if (lane == 0) atomicAdd(scnt + b, c);
+                    for (uint32_t fresh = hb & ~seen; fresh; fresh &= fresh - 1u)
+                        atomicMin(point_box + j0 + p0 + (__ffs(fresh) - 1), (u64)(box0 + b));
+                    seen |= hb;
+                }
+            }
+        }
+        __syncthreads();
+        if (threadIdx.x < nb && scnt[threadIdx.x]) atomicAdd(box_npoints + i0 + box0 + threadIdx.x, (u64)scnt[threadIdx.x]);
+    }
+}
+
+// the grid path's hit action: the point's atomicMin and the walker's count; for 3-D rows the test along the axis comes first (the
+// sorted records hold the plane coordinates, the axis coordinate is read through the point's index)
+template <typename T, bool P3> struct CropAssignHit {
+    const T *__restrict__ pts;
+    int axis;
+    CropZ<T> z;
+    int64_t box;
+    u64 *__restrict__ point_box;
+    uint32_t count;
+    __device__ __forceinline__ void operator()(const CropPt<T> &p)
+    {
+        if (P3) {
+            const T c = pts[3 * (int64_t)p.idx + axis];
+            if (!(rn_sub(c, z.hd) < z.c && z.c < rn_add(c, z.hd))) return;
+        }
+        atomicMin(point_box + p.idx, (u64)box);
+        count++;
+    }
+};
+
+// crop_hits_kernel / crop_heavy_kernel with the reducing hit action: a warp's count is one atomicAdd
+template <typename T, bool P3>
+__global__ void __launch_bounds__(256) crop_assign_hits_kernel(const CropPt<T> *__restrict__ sorted, const T *__restrict__ pts, int axis,
+                                                               const CropBox<T> *__restrict__ recs, const CropZ<T> *__restrict__ zr, int64_t m,
+                                                               const CropGrid *__restrict__ g, const uint32_t *__restrict__ cellptr,
+                                                               u64 *__restrict__ point_box, u64 *__restrict__ box_npoints,
+                                                               uint32_t *__restrict__ heavy_count, uint2 *__restrict__ heavy_item)
+{
+    const unsigned lane = threadIdx.x & 31;
+    const int64_t i = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (i >= m) return;
+    const CropGrid G = *g;
+    const CropBox<T> B = recs[i];
+    if (!G.ok) return;                                      // no grid: the tile kernel that follows computes the outputs
+    if (!(B.minx < B.maxx) || !(B.miny < B.maxy)) return;   // empty or NaN box: no point passes the open AABB test
+    int x0, x1, y0, y1;
+    crop_cells<T>(B, G, &x0, &x1, &y0, &y1);
+    uint32_t total = 0;
+    for (int yb = y0; yb <= y1; yb += 32) {
+        uint32_t c = 0;
+        if (yb + (int)lane <= y1) c = cellptr[(yb + (int)lane) * CG + x1 + 1] - cellptr[(yb + (int)lane) * CG + x0];
+        total += __reduce_add_sync(0xffffffffu, c);
+    }
+    if (total > (uint32_t)CROP_LIGHT) {   // at most CROP_HSLICES items per box
+        const uint32_t ns = min((uint32_t)CROP_HSLICES, (total + CROP_ITEM - 1) / CROP_ITEM);
+        uint32_t base = 0;
+        if (lane == 0) base = atomicAdd(heavy_count, ns);
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (lane < ns) heavy_item[base + lane] = make_uint2((uint32_t)i, lane | (ns << 16));
+        return;
+    }
+    CropAssignHit<T, P3> hit{pts, axis, P3 ? zr[i] : CropZ<T>{}, i, point_box, 0u};
+    crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, hit, lane, 32u);
+    const uint32_t c = __reduce_add_sync(0xffffffffu, hit.count);
+    if (lane == 0 && c) atomicAdd(box_npoints + i, (u64)c);
+}
+
+template <typename T, bool P3>
+__global__ void __launch_bounds__(CROP_HT) crop_assign_heavy_kernel(const CropPt<T> *__restrict__ sorted, const T *__restrict__ pts, int axis,
+                                                                    const CropBox<T> *__restrict__ recs, const CropZ<T> *__restrict__ zr,
+                                                                    const CropGrid *__restrict__ g, const uint32_t *__restrict__ cellptr,
+                                                                    u64 *__restrict__ point_box, u64 *__restrict__ box_npoints,
+                                                                    const uint32_t *__restrict__ heavy_count, const uint2 *__restrict__ heavy_item)
+{
+    const CropGrid G = *g;
+    if (!G.ok) return;
+    const uint32_t items = *heavy_count;
+    for (uint32_t w = blockIdx.x; w < items; w += gridDim.x) {
+        const uint2 it = heavy_item[w];
+        const int64_t i = it.x;
+        const uint32_t j = it.y & 0xffffu, ns = it.y >> 16;
+        const CropBox<T> B = recs[i];
+        int x0, x1, y0, y1;
+        crop_cells<T>(B, G, &x0, &x1, &y0, &y1);
+        CropAssignHit<T, P3> hit{pts, axis, P3 ? zr[i] : CropZ<T>{}, i, point_box, 0u};
+        crop_walk<T>(B, x0, x1, y0, y1, sorted, cellptr, hit, j * CROP_HT + threadIdx.x, ns * CROP_HT);
+        const uint32_t c = __reduce_add_sync(0xffffffffu, hit.count);
+        if ((threadIdx.x & 31) == 0 && c) atomicAdd(box_npoints + i, (u64)c);
+    }
+}
+
+// 3-D rows on the grid path: the two plane columns, packed as the 2-D rows the binning kernels read
+template <typename T>
+__global__ void __launch_bounds__(256) crop_plane_kernel(const T *__restrict__ pts, int64_t n, int axis, T *__restrict__ plane)
+{
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    int pa, pb;
+    proj_plane(axis, &pa, &pb);
+    plane[2 * j] = pts[3 * j + pa]; plane[2 * j + 1] = pts[3 * j + pb];
+}
+
+template <typename T> static size_t crop_assign_ws_bytes(int64_t m, int64_t n)
+{
+    const size_t n1 = (size_t)(n > 0 ? n : 1), m1 = (size_t)(m > 0 ? m : 1);
+    return align_up(m1 * sizeof(CropBox<T>)) + align_up(m1 * sizeof(CropZ<T>)) + align_up(n1 * 2 * sizeof(T)) + crop_grid_ws_bytes<T>(m, n);
+}
+
+template <typename T>
+static int crop_assign_impl(const T *pts, int64_t n, const T *boxes, int64_t m, int axis, int64_t *point_box, int64_t *box_npoints, void *ws,
+                            size_t ws_bytes, cudaStream_t st)
+{
+    if (n < 0 || m < 0 || axis < -1 || axis > 2) return D3D_ERR_INVALID_ARGUMENT;
+    if (n == 0 && m == 0) return D3D_OK;
+    if ((n && (!pts || !point_box)) || (m && (!boxes || !box_npoints))) return D3D_ERR_INVALID_ARGUMENT;
+    if (n >= (1ll << 32) || m > 0x7fffffffll) return D3D_ERR_INVALID_ARGUMENT;
+    if (n && m && (!ws || ws_bytes < crop_assign_ws_bytes<T>(m, n))) return D3D_ERR_WORKSPACE;
+    if (n) D3D_CUDA_TRY(cudaMemsetAsync(point_box, 0xff, (size_t)n * sizeof(int64_t), st));
+    if (m) D3D_CUDA_TRY(cudaMemsetAsync(box_npoints, 0, (size_t)m * sizeof(int64_t), st));
+    if (!n || !m) return D3D_OK;
+    Arena a(ws, ws_bytes);
+    CropBox<T> *recs = a.take<CropBox<T>>(m);
+    CropZ<T> *z = a.take<CropZ<T>>(m);
+    T *plane = a.take<T>((size_t)n * 2);
+    u64 *pbox = reinterpret_cast<u64 *>(point_box), *bcnt = reinterpret_cast<u64 *>(box_npoints);
+    int mode = 0;   // D3D_B200_CROP_PATH=brute | grid, as for the mask
+    if (const int t = tuning(D3D_TUNE_CROP_PATH, 0)) mode = t;
+    const bool grid = mode == 2 || (mode == 0 && m * n >= CROP_GRID_MIN_PAIRS);
+    crop_prep_batch_kernel<T><<<(unsigned)cdiv(m, 256), 256, 0, st>>>(boxes, m, axis, recs, z); D3D_LAUNCHED();
+    const int64_t gy = cdiv(n, (int64_t)CROP_THREADS * CROP_PPT), gz = cdiv(m, CROP_BT);
+    if (!grid) {
+        const dim3 tg(1u, (unsigned)(gy < 65535 ? gy : 65535), (unsigned)(gz < 65535 ? gz : 65535));
+        if (axis < 0) crop_assign_tile_kernel<T, false><<<tg, CROP_THREADS, 0, st>>>(pts, nullptr, n, recs, z, nullptr, m, axis, INT64_MAX, nullptr, pbox, bcnt);
+        else crop_assign_tile_kernel<T, true><<<tg, CROP_THREADS, 0, st>>>(pts, nullptr, n, recs, z, nullptr, m, axis, INT64_MAX, nullptr, pbox, bcnt);
+        D3D_LAUNCHED();
+        return D3D_OK;
+    }
+    uint32_t *acc = a.take<uint32_t>(16);
+    CropGrid *g = a.take<CropGrid>(1);
+    uint32_t *cellcnt = a.take<uint32_t>((size_t)(CG_CELLS + 1));
+    uint32_t *cellptr = a.take<uint32_t>((size_t)(CG_CELLS + 1));
+    CropPt<T> *sorted = a.take<CropPt<T>>(n);
+    uint2 *cellrank = a.take<uint2>(n);
+    uint2 *heavy_item = a.take<uint2>((size_t)m * CROP_HSLICES);
+    void *scan_ws = a.take<char>(scan_workspace_bytes(CG_CELLS + 1));
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    uint32_t *heavy_count = acc + 5;
+    const uint32_t init[6] = {0xffffffffu, 0u, 0xffffffffu, 0u, 0u, 0u};
+    const unsigned gb = (unsigned)cdiv(n, 256);
+    const T *p2 = pts;   // the 2-D rows the grid is built from
+    if (axis >= 0) { crop_plane_kernel<T><<<gb, 256, 0, st>>>(pts, n, axis, plane); D3D_LAUNCHED(); p2 = plane; }
+    D3D_CUDA_TRY(cudaMemcpyAsync(acc, init, sizeof(init), cudaMemcpyHostToDevice, st));
+    D3D_CUDA_TRY(cudaMemsetAsync(cellcnt, 0, (size_t)(CG_CELLS + 1) * 4, st));
+    crop_bounds_kernel<T><<<gb < 592 ? gb : 592, 256, 0, st>>>(p2, n, acc); D3D_LAUNCHED();
+    crop_grid_kernel<<<1, 1, 0, st>>>(acc, g); D3D_LAUNCHED();
+    crop_bin_kernel<T, 0><<<gb, 256, 0, st>>>(p2, n, g, cellcnt, nullptr, cellrank, nullptr); D3D_LAUNCHED();
+    const int rc = exclusive_scan_u32(cellcnt, cellptr, CG_CELLS + 1, nullptr, scan_ws, st);
+    if (rc) return rc;
+    crop_bin_kernel<T, 1><<<gb, 256, 0, st>>>(p2, n, g, nullptr, cellptr, cellrank, sorted); D3D_LAUNCHED();
+    // geometry that admits no grid (non-finite points, all points identical): the tile kernel runs instead (it leaves at once otherwise)
+    const dim3 fg(1u, (unsigned)(gy < 74 ? gy : 74), (unsigned)(gz < 16 ? gz : 16));
+    if (axis < 0) {
+        crop_assign_hits_kernel<T, false><<<(unsigned)cdiv(m, 8), 256, 0, st>>>(sorted, pts, axis, recs, z, m, g, cellptr, pbox, bcnt, heavy_count, heavy_item); D3D_LAUNCHED();
+        crop_assign_heavy_kernel<T, false><<<1184, CROP_HT, 0, st>>>(sorted, pts, axis, recs, z, g, cellptr, pbox, bcnt, heavy_count, heavy_item); D3D_LAUNCHED();
+        crop_assign_tile_kernel<T, false><<<fg, CROP_THREADS, 0, st>>>(pts, nullptr, n, recs, z, nullptr, m, axis, INT64_MAX, g, pbox, bcnt); D3D_LAUNCHED();
+    } else {
+        crop_assign_hits_kernel<T, true><<<(unsigned)cdiv(m, 8), 256, 0, st>>>(sorted, pts, axis, recs, z, m, g, cellptr, pbox, bcnt, heavy_count, heavy_item); D3D_LAUNCHED();
+        crop_assign_heavy_kernel<T, true><<<1184, CROP_HT, 0, st>>>(sorted, pts, axis, recs, z, g, cellptr, pbox, bcnt, heavy_count, heavy_item); D3D_LAUNCHED();
+        crop_assign_tile_kernel<T, true><<<fg, CROP_THREADS, 0, st>>>(pts, nullptr, n, recs, z, nullptr, m, axis, INT64_MAX, g, pbox, bcnt); D3D_LAUNCHED();
+    }
+    return D3D_OK;
+}
+
+template <typename T>
+static int crop_assign_batch_impl(const T *pts, int64_t total_pts, const int64_t *poff, const T *boxes, int64_t total_boxes, const int64_t *boff,
+                                  int64_t nframes, int64_t max_pts, int64_t max_boxes, int axis, int64_t *point_box, int64_t *box_npoints, void *ws,
+                                  size_t ws_bytes, cudaStream_t st)
+{
+    if (total_pts < 0 || total_boxes < 0 || nframes < 0 || max_pts < 0 || max_boxes < 0 || axis < -1 || axis > 2) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes == 0 || (total_pts == 0 && total_boxes == 0)) return D3D_OK;
+    if (!poff || !boff || (total_pts && (!pts || !point_box)) || (total_boxes && (!boxes || !box_npoints))) return D3D_ERR_INVALID_ARGUMENT;
+    if (nframes > 0x7fffffffll) return D3D_ERR_UNSUPPORTED;
+    if (total_pts && total_boxes && (!ws || ws_bytes < crop_batch_ws_bytes<T>(total_boxes))) return D3D_ERR_WORKSPACE;
+    if (total_pts) D3D_CUDA_TRY(cudaMemsetAsync(point_box, 0xff, (size_t)total_pts * sizeof(int64_t), st));
+    if (total_boxes) D3D_CUDA_TRY(cudaMemsetAsync(box_npoints, 0, (size_t)total_boxes * sizeof(int64_t), st));
+    if (!total_pts || !total_boxes) return D3D_OK;
+    if (max_pts == 0) max_pts = total_pts;   // 0: bound unknown
+    if (max_boxes == 0) max_boxes = total_boxes;
+    Arena a(ws, ws_bytes);
+    a.take<char>(256);
+    CropBox<T> *recs = a.take<CropBox<T>>(total_boxes);
+    CropZ<T> *z = a.take<CropZ<T>>(total_boxes);
+    if (!a.ok()) return D3D_ERR_WORKSPACE;
+    u64 *pbox = reinterpret_cast<u64 *>(point_box), *bcnt = reinterpret_cast<u64 *>(box_npoints);
+    crop_prep_batch_kernel<T><<<(unsigned)cdiv(total_boxes, 256), 256, 0, st>>>(boxes, total_boxes, axis, recs, z); D3D_LAUNCHED();
+    const int64_t gy = cdiv(max_pts, (int64_t)CROP_THREADS * CROP_PPT), gz = cdiv(max_boxes, CROP_BT);
+    const dim3 grid((unsigned)nframes, (unsigned)(gy < 65535 ? gy : 65535), (unsigned)(gz < 65535 ? gz : 65535));
+    if (axis < 0) crop_assign_tile_kernel<T, false><<<grid, CROP_THREADS, 0, st>>>(pts, poff, 0, recs, z, boff, 0, axis, CROP_GRID_MIN_PAIRS, nullptr, pbox, bcnt);
+    else crop_assign_tile_kernel<T, true><<<grid, CROP_THREADS, 0, st>>>(pts, poff, 0, recs, z, boff, 0, axis, CROP_GRID_MIN_PAIRS, nullptr, pbox, bcnt);
+    D3D_LAUNCHED();
+    return D3D_OK;
+}
+
 }  // namespace d3d
 
 using namespace d3d;
@@ -569,4 +848,36 @@ extern "C" int d3d_crop2dr_batch_f64(const double *points, int64_t total_points,
 {
     return crop_batch_impl<double>(points, total_points, point_offsets, boxes, total_boxes, box_offsets, nframes, max_frame_points, max_frame_boxes,
                                    project_axis, mask_offsets, mask, ws, wsb, (cudaStream_t)stream);
+}
+extern "C" size_t d3d_crop2dr_assign_workspace_bytes(int64_t n, int64_t m, int dtype)
+{
+    if (n < 0 || m < 0) return 0;
+    return dtype == D3D_F64 ? crop_assign_ws_bytes<double>(m, n) : crop_assign_ws_bytes<float>(m, n);
+}
+extern "C" int d3d_crop2dr_assign_f32(const float *points, int64_t n, const float *boxes, int64_t m, int project_axis, int64_t *point_box,
+                                      int64_t *box_npoints, void *ws, size_t wsb, void *stream)
+{ return crop_assign_impl<float>(points, n, boxes, m, project_axis, point_box, box_npoints, ws, wsb, (cudaStream_t)stream); }
+extern "C" int d3d_crop2dr_assign_f64(const double *points, int64_t n, const double *boxes, int64_t m, int project_axis, int64_t *point_box,
+                                      int64_t *box_npoints, void *ws, size_t wsb, void *stream)
+{ return crop_assign_impl<double>(points, n, boxes, m, project_axis, point_box, box_npoints, ws, wsb, (cudaStream_t)stream); }
+extern "C" size_t d3d_crop2dr_assign_batch_workspace_bytes(int64_t total_boxes, int dtype)
+{
+    if (total_boxes < 0) return 0;
+    return dtype == D3D_F64 ? crop_batch_ws_bytes<double>(total_boxes) : crop_batch_ws_bytes<float>(total_boxes);
+}
+extern "C" int d3d_crop2dr_assign_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes,
+                                            int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                            int64_t max_frame_boxes, int project_axis, int64_t *point_box, int64_t *box_npoints, void *ws, size_t wsb,
+                                            void *stream)
+{
+    return crop_assign_batch_impl<float>(points, total_points, point_offsets, boxes, total_boxes, box_offsets, nframes, max_frame_points,
+                                         max_frame_boxes, project_axis, point_box, box_npoints, ws, wsb, (cudaStream_t)stream);
+}
+extern "C" int d3d_crop2dr_assign_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes,
+                                            int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                            int64_t max_frame_boxes, int project_axis, int64_t *point_box, int64_t *box_npoints, void *ws, size_t wsb,
+                                            void *stream)
+{
+    return crop_assign_batch_impl<double>(points, total_points, point_offsets, boxes, total_boxes, box_offsets, nframes, max_frame_points,
+                                          max_frame_boxes, project_axis, point_box, box_npoints, ws, wsb, (cudaStream_t)stream);
 }

@@ -260,6 +260,37 @@ int d3d_crop2dr_batch_f32(const float *points, int64_t total_points, const int64
 int d3d_crop2dr_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes, int64_t total_boxes,
                           const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
                           const int64_t *mask_offsets, uint8_t *mask, void *workspace, size_t workspace_bytes, void *stream);
+/* Fused reductions of the point-in-box mask, without the mask: point_box i64[points] is the lowest FRAME-LOCAL index of a box whose mask
+ * entry for the point is 1, or -1 if there is none; box_npoints i64[boxes] is the number of points inside each box.  The decision per pair
+ * is that of d3d_crop2dr_* / d3d_crop2dr_batch_* (same points, boxes and project_axis convention), so per frame the outputs equal
+ * where(mask.any(0), mask.argmax(0), -1) and mask.sum(1) exactly.
+ * d3d_crop2dr_assign_*: one frame, n points, m boxes (project_axis -1: rows [n,2] / [m,5]; 0, 1, 2: rows [n,3] / [m,7]).  It initialises
+ * point_box[0, n) and box_npoints[0, m) itself and then computes them; like d3d_crop2dr_* it bins the points into a grid when
+ * n * m >= d3d_crop2dr_grid_min_pairs() (D3D_B200_CROP_PATH=brute | grid forces a back end); the result does not depend on the back end.
+ * Workspace below d3d_crop2dr_assign_workspace_bytes (needed when n and m are both positive): D3D_ERR_WORKSPACE; n >= 2^32 or m >= 2^31:
+ * D3D_ERR_INVALID_ARGUMENT.
+ * d3d_crop2dr_assign_batch_*: the arguments of d3d_crop2dr_batch_* with the two outputs in place of mask_offsets and mask.  It initialises
+ * ALL of point_box [total_points] (to -1) and box_npoints [total_boxes] (to 0), including the slices of the frames it skips, then makes
+ * one box preparation and one tile launch, whatever the number of frames.  Like the mask batch entry, it does not compute a frame with
+ * n_f * m_f >= d3d_crop2dr_grid_min_pairs() (the bounds need not cover it): call d3d_crop2dr_assign_* on that frame's slices AFTER the batch
+ * call on the same stream, which would otherwise overwrite them.  Workspace below d3d_crop2dr_assign_batch_workspace_bytes:
+ * D3D_ERR_WORKSPACE; nframes > 2^31 - 1: D3D_ERR_UNSUPPORTED.
+ * Both: negative sizes or project_axis outside -1..2: D3D_ERR_INVALID_ARGUMENT; no point and no box (or nframes == 0): no-op.  A null
+ * pointer is allowed only for an empty side.  Argument errors return before any CUDA call. */
+size_t d3d_crop2dr_assign_workspace_bytes(int64_t n, int64_t m, int dtype);
+int d3d_crop2dr_assign_f32(const float *points, int64_t n, const float *boxes, int64_t m, int project_axis, int64_t *point_box,
+                           int64_t *box_npoints, void *workspace, size_t workspace_bytes, void *stream);
+int d3d_crop2dr_assign_f64(const double *points, int64_t n, const double *boxes, int64_t m, int project_axis, int64_t *point_box,
+                           int64_t *box_npoints, void *workspace, size_t workspace_bytes, void *stream);
+size_t d3d_crop2dr_assign_batch_workspace_bytes(int64_t total_boxes, int dtype);
+int d3d_crop2dr_assign_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes,
+                                 int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                 int64_t max_frame_boxes, int project_axis, int64_t *point_box, int64_t *box_npoints, void *workspace,
+                                 size_t workspace_bytes, void *stream);
+int d3d_crop2dr_assign_batch_f64(const double *points, int64_t total_points, const int64_t *point_offsets, const double *boxes,
+                                 int64_t total_boxes, const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points,
+                                 int64_t max_frame_boxes, int project_axis, int64_t *point_box, int64_t *box_npoints, void *workspace,
+                                 size_t workspace_bytes, void *stream);
 int d3d_pdist2dr_batch_f32(const float *points, int64_t total_points, const int64_t *point_offsets, const float *boxes, int64_t total_boxes,
                            const int64_t *box_offsets, int64_t nframes, int64_t max_frame_points, int64_t max_frame_boxes, int project_axis,
                            const int64_t *dist_offsets, float *dist, void *stream);
