@@ -6,6 +6,7 @@ import numpy as np
 import torch
 
 from .. import _cabi as _c
+from . import _frames
 
 
 class IouType(enum.IntEnum):   # d3d/box/common.h:5-9
@@ -139,6 +140,13 @@ DIou2DR = _make_iou_function("diou2dr", "Differentiable rotated DIoU function fo
 DIou2DR.__name__ = DIou2DR.__qualname__ = "DIou2DR"
 
 
+def _check_iou2d(boxes1, boxes2):   # box2d_iou's checks
+    if len(boxes1.shape) != 2 or len(boxes2.shape) != 2:
+        raise ValueError("Input of rbox_2d_iou should be Nx2 tensors!")
+    if boxes1.shape[1] != 5 or boxes2.shape[1] != 5:
+        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+
+
 def box2d_iou(boxes1, boxes2, method="box", precise=True):
     '''
     Differentiable IoU on axis-aligned or rotated 2D boxes (reference d3d/box/__init__.py:180-224)
@@ -158,10 +166,7 @@ def box2d_iou(boxes1, boxes2, method="box", precise=True):
 
     otype = boxes1.dtype
     odev = boxes1.device
-    if len(boxes1.shape) != 2 or len(boxes2.shape) != 2:
-        raise ValueError("Input of rbox_2d_iou should be Nx2 tensors!")
-    if boxes1.shape[1] != 5 or boxes2.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+    _check_iou2d(boxes1, boxes2)
 
     iou_type = getattr(IouType, method.upper())
     if iou_type == IouType.BOX:
@@ -209,8 +214,8 @@ class _IouBatch(torch.autograd.Function):
                 st = _c.iou_batch[code](_c.ptr(boxes1), len(boxes1), _c.ptr(od1), _c.ptr(boxes2), len(boxes2), _c.ptr(od2), nframes, fwd_max1, fwd_max2,
                                         int(iou_type), _c.ptr(odo), _c.ptr(out), _c.ptr(ws), ws.numel() if ws is not None else 0, _c.stream_ptr())
             _c.check(st, "box2d_iou_batch")
-        for a0, a1, b0, b1, o0 in big:   # "rbox" frames past the batch kernel's tile grid: the single-frame kernel, into their block
-            _pairwise(boxes1[a0:a1], boxes2[b0:b1], _c.iou2dr, out=out[o0:o0 + (a1 - a0) * (b1 - b0)].view(a1 - a0, b1 - b0))
+        for _, r, c, k in big:   # "rbox" frames past the batch kernel's tile grid: the single-frame kernel, into their block
+            _pairwise(boxes1[r], boxes2[c], _c.iou2dr, out=out[k].view(r.stop - r.start, c.stop - c.start))
         ctx.save_for_backward(boxes1, boxes2, *offsets)
         ctx.args = (nframes, max1, max2, iou_type)
         return out
@@ -229,11 +234,14 @@ class _IouBatch(torch.autograd.Function):
         return g1, g2, None, None, None, None, None, None
 
 
-def _check_iou2d(boxes1, boxes2):   # box2d_iou's checks
-    if len(boxes1.shape) != 2 or len(boxes2.shape) != 2:
-        raise ValueError("Input of rbox_2d_iou should be Nx2 tensors!")
-    if boxes1.shape[1] != 5 or boxes2.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+def _iou_pair(b1, b2, precise):
+    """both packed box sets on the device, in float64 with `precise`; their dtypes are checked before any device work"""
+    if not precise:
+        _c.dtype_code(b1.dtype)
+        if b2.dtype != b1.dtype:
+            raise RuntimeError("boxes1 and boxes2 must have the same dtype")
+    b1, b2 = _c.to_device(b1), _c.to_device(b2)
+    return (b1.to(torch.float64), b2.to(torch.float64)) if precise else (b1, b2)
 
 
 def box2d_iou_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", precise=True):
@@ -247,95 +255,45 @@ def box2d_iou_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", 
     65535 tiles (64 rows, or 128 fp32 / 64 fp64 columns) run the single-frame kernel, into their block; the batch kernels skip them,
     though the workspace still has room for their records.
     '''
-    as_list = isinstance(boxes1, (list, tuple))
-    if as_list:
-        if not isinstance(boxes2, (list, tuple)) or len(boxes1) != len(boxes2):
-            raise ValueError("boxes1 and boxes2 should hold the same number of frames")
-        if len(boxes1) == 0:
-            return []
-        numpy_in = isinstance(boxes1[0], np.ndarray)
-        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
-        l1, l2 = [tt(b) for b in boxes1], [tt(b) for b in boxes2]
-        for a, b in zip(l1, l2):
-            _check_iou2d(a, b)
-        if len({x.dtype for x in l1}) != 1 or len({x.dtype for x in l2}) != 1:
-            raise RuntimeError("the frames of a box set must have the same dtype")
-        off1, off2 = _frame_offsets(lens=[len(b) for b in l1]), _frame_offsets(lens=[len(b) for b in l2])
-        B1, B2 = torch.cat(l1), torch.cat(l2)
-    else:
-        numpy_in = isinstance(boxes1, np.ndarray)
-        if numpy_in:
-            assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
-            boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
-        if offsets1 is None or offsets2 is None:
-            raise ValueError("packed boxes need the frame offsets")
-        _check_iou2d(boxes1, boxes2)
-        off1, off2 = _frame_offsets(offsets1), _frame_offsets(offsets2)
-        B1, B2 = boxes1, boxes2
-    if off1.numel() != off2.numel() or int(off1[-1]) != len(B1) or int(off2[-1]) != len(B2):
-        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
+    if _frames.empty(boxes1, boxes2):
+        return []
+    B1, B2, fr = _frames.inputs(boxes1, boxes2, offsets1, offsets2, _check_iou2d, ("boxes1", "boxes2"))
     iou_type = getattr(IouType, method.upper())
     if iou_type not in (IouType.BOX, IouType.RBOX, IouType.GRBOX, IouType.DRBOX):
         raise ValueError("Unrecognized iou type!")
-    otype, odev = B1.dtype, B1.device
-    b1, b2 = _c.to_device(B1), _c.to_device(B2)
-    if precise:
-        b1, b2 = b1.to(torch.float64), b2.to(torch.float64)
-    _c.dtype_code(b1.dtype)
-    if b2.dtype != b1.dtype:
-        raise RuntimeError("boxes1 and boxes2 must have the same dtype")
-    nframes = off1.numel() - 1
-    n_f, m_f = off1[1:] - off1[:-1], off2[1:] - off2[:-1]
-    blk = _block_offsets(off1, off2)
-    big = torch.zeros(nframes, dtype=torch.bool)
+    b1, b2 = _iou_pair(B1, B2, precise)
+    n_f, m_f = fr.lengths()
+    big = torch.zeros(fr.nframes, dtype=torch.bool)
     if iou_type == IouType.RBOX:
         tr, tc = _IOU_TILE[b1.dtype]
         big = (n_f > 65535 * tr) | (m_f > 65535 * tc)
-    small = (n_f * m_f > 0) & ~big
-    bounds = (int(n_f[small].max()) if bool(small.any()) else 0, int(m_f[small].max()) if bool(small.any()) else 0,
-              int(n_f.max()) if nframes else 0, int(m_f.max()) if nframes else 0)
-    big_frames = [(int(off1[f]), int(off1[f + 1]), int(off2[f]), int(off2[f + 1]), int(blk[f])) for f in torch.nonzero(big).flatten().tolist()]
-    offsets = _device_offsets(off1, off2, blk, b1.device)
-    flat = _IouBatch.apply(b1.contiguous(), b2.contiguous(), offsets, nframes, bounds, iou_type, int(blk[-1]), big_frames)
-    if precise:
-        flat = flat.to(otype)
-    return _point_box_outputs(flat, blk, off2, off1, as_list, numpy_in, odev)
+    bounds = fr.bounds((n_f * m_f > 0) & ~big) + fr.bounds()
+    offsets = _frames.to_device(b1.device, fr.rows, fr.cols, fr.blocks)
+    flat = _IouBatch.apply(b1.contiguous(), b2.contiguous(), offsets, fr.nframes, bounds, iou_type, int(fr.blocks[-1]), list(fr.each(big)))
+    return fr.matrices(flat.to(B1.dtype) if precise else flat)
 
 
-def _iou_max_packed(B1, B2, off1, off2, method, precise):
-    """(max1, idx1, max2, idx2) of packed frames on the device, frame-local indices"""
+def _iou_max(B1, B2, fr, method, precise):
+    """(max1, idx1, max2, idx2) of the frames `fr` of the packed box sets, frame-local indices, on the caller's side"""
     iou_type = getattr(IouType, method.upper())
     if iou_type not in (IouType.BOX, IouType.RBOX):
         raise ValueError("Unsupported iou type!")
     otype = B1.dtype
-    b1, b2 = _c.to_device(B1.detach()), _c.to_device(B2.detach())
-    if precise:
-        b1, b2 = b1.to(torch.float64), b2.to(torch.float64)
-    code = _c.dtype_code(b1.dtype)
-    if b2.dtype != b1.dtype:
-        raise RuntimeError("boxes1 and boxes2 must have the same dtype")
     ocode = _c.dtype_code(otype)
-    dev, total1, total2, nframes = b1.device, len(b1), len(b2), off1.numel() - 1
+    b1, b2 = _iou_pair(B1.detach(), B2.detach(), precise)
+    code = _c.dtype_code(b1.dtype)
+    dev, total1, total2 = b1.device, len(b1), len(b2)
     max1, max2 = torch.empty(total1, dtype=otype, device=dev), torch.empty(total2, dtype=otype, device=dev)
     idx1, idx2 = torch.empty(total1, dtype=torch.int64, device=dev), torch.empty(total2, dtype=torch.int64, device=dev)
-    if nframes and total1 + total2:
+    if fr.nframes and total1 + total2:
         b1, b2 = b1.contiguous(), b2.contiguous()
-        n_f, m_f = off1[1:] - off1[:-1], off2[1:] - off2[:-1]
-        offs = torch.cat([off1, off2]).to(dev, non_blocking=True)   # one copy of both offset arrays
-        ws = _c.workspace(_c.iou_max_batch_workspace_bytes(total1, total2, nframes, code), dev)
+        od1, od2 = _frames.to_device(dev, fr.rows, fr.cols)
+        ws = _c.workspace(_c.iou_max_batch_workspace_bytes(total1, total2, fr.nframes, code), dev)
         with torch.cuda.device(dev):
-            st = _c.iou_max_batch[code](_c.ptr(b1), total1, _c.ptr(offs[:nframes + 1]), _c.ptr(b2), total2, _c.ptr(offs[nframes + 1:]), nframes,
-                                        int(n_f.max()), int(m_f.max()), int(iou_type), ocode, _c.ptr(max1), _c.ptr(idx1), _c.ptr(max2), _c.ptr(idx2),
-                                        _c.ptr(ws), ws.numel(), _c.stream_ptr())
+            st = _c.iou_max_batch[code](_c.ptr(b1), total1, _c.ptr(od1), _c.ptr(b2), total2, _c.ptr(od2), fr.nframes, *fr.bounds(), int(iou_type),
+                                        ocode, _c.ptr(max1), _c.ptr(idx1), _c.ptr(max2), _c.ptr(idx2), _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box2d_iou_max_batch")
-    return max1, idx1, max2, idx2
-
-
-def _reduction_outputs(outs, odev, numpy_in):
-    """device outputs of a fused reduction on the inputs' side (numpy, host or device)"""
-    if odev.type != "cuda" or numpy_in:
-        outs = tuple(x.cpu() for x in outs)
-    return tuple(x.numpy() for x in outs) if numpy_in else tuple(outs)
+    return fr.outputs(rows=(max1, idx1), cols=(max2, idx2))
 
 
 def box2d_iou_max(boxes1, boxes2, method="box", precise=True):
@@ -358,8 +316,7 @@ def box2d_iou_max(boxes1, boxes2, method="box", precise=True):
         assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
         boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
     _check_iou2d(boxes1, boxes2)
-    off1, off2 = _frame_offsets(lens=[len(boxes1)]), _frame_offsets(lens=[len(boxes2)])
-    return _reduction_outputs(_iou_max_packed(boxes1, boxes2, off1, off2, method, precise), boxes1.device, numpy_in)
+    return _iou_max(boxes1, boxes2, _frames.Frames([0, len(boxes1)], [0, len(boxes2)], False, numpy_in, boxes1.device), method, precise)
 
 
 def box2d_iou_max_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="box", precise=True):
@@ -372,38 +329,9 @@ def box2d_iou_max_batch(boxes1, boxes2, offsets1=None, offsets2=None, method="bo
     'rbox') and ``precise`` as in :func:`box2d_iou_max`.  The outputs do not require grad.  numpy in -> numpy out, host tensors in -> host
     tensors out.
     '''
-    as_list = isinstance(boxes1, (list, tuple))
-    if as_list:
-        if not isinstance(boxes2, (list, tuple)) or len(boxes1) != len(boxes2):
-            raise ValueError("boxes1 and boxes2 should hold the same number of frames")
-        if len(boxes1) == 0:
-            return []
-        numpy_in = isinstance(boxes1[0], np.ndarray)
-        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
-        l1, l2 = [tt(b) for b in boxes1], [tt(b) for b in boxes2]
-        for a, b in zip(l1, l2):
-            _check_iou2d(a, b)
-        if len({x.dtype for x in l1}) != 1 or len({x.dtype for x in l2}) != 1:
-            raise RuntimeError("the frames of a box set must have the same dtype")
-        off1, off2 = _frame_offsets(lens=[len(b) for b in l1]), _frame_offsets(lens=[len(b) for b in l2])
-        B1, B2 = torch.cat(l1), torch.cat(l2)
-    else:
-        numpy_in = isinstance(boxes1, np.ndarray)
-        if numpy_in:
-            assert isinstance(boxes2, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
-            boxes1, boxes2 = torch.from_numpy(boxes1), torch.from_numpy(boxes2)
-        if offsets1 is None or offsets2 is None:
-            raise ValueError("packed boxes need the frame offsets")
-        _check_iou2d(boxes1, boxes2)
-        off1, off2 = _frame_offsets(offsets1), _frame_offsets(offsets2)
-        B1, B2 = boxes1, boxes2
-    if off1.numel() != off2.numel() or int(off1[-1]) != len(B1) or int(off2[-1]) != len(B2):
-        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
-    m1, i1, m2, i2 = _reduction_outputs(_iou_max_packed(B1, B2, off1, off2, method, precise), B1.device, numpy_in)
-    if not as_list:
-        return m1, i1, m2, i2
-    return [(m1[int(off1[f]):int(off1[f + 1])], i1[int(off1[f]):int(off1[f + 1])], m2[int(off2[f]):int(off2[f + 1])], i2[int(off2[f]):int(off2[f + 1])])
-            for f in range(off1.numel() - 1)]
+    if _frames.empty(boxes1, boxes2):
+        return []
+    return _iou_max(*_frames.inputs(boxes1, boxes2, offsets1, offsets2, _check_iou2d, ("boxes1", "boxes2")), method, precise)
 
 
 def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold=0, score_threshold=0, precise=True, offsets_dev=None,
@@ -420,52 +348,45 @@ def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold
     :param supression_method: 'hard', or 'linear' / 'gaussian' (soft-NMS: one CTA walks each frame, the frames run side by side)
     :param supression_param: parameter of the soft decay, as in :func:`box2d_nms`
     '''
-    as_list = isinstance(boxes, (list, tuple))
-    if as_list:
+    if isinstance(boxes, (list, tuple)):
         if len(boxes) != len(scores):
             raise ValueError("Numbers of boxes and scores are inconsistent!")
         if len(boxes) == 0:
             return []
-        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x
-        numpy_in = isinstance(boxes[0], np.ndarray)
-        blist, slist = [tt(b) for b in boxes], [tt(s_) for s_ in scores]
-        odev = blist[0].device
-        lens = [int(b.shape[0]) for b in blist]
-        offsets = torch.zeros(len(lens) + 1, dtype=torch.int64)
-        offsets[1:] = torch.tensor(lens).cumsum(0)
-        boxes = torch.cat([_c.to_device(b).reshape(-1, 5) for b in blist], 0)
-        scores = torch.cat([_c.to_device(s_).reshape(-1) for s_ in slist], 0)
+        blist, slist = [_frames.host(b) for b in boxes], [_frames.host(s_) for s_ in scores]
+        fr = _frames.Frames(_frames.offsets_of(len(b) for b in blist), None, True, isinstance(boxes[0], np.ndarray), blist[0].device)
+        counts = sum(b.numel() // 5 for b in blist), sum(s_.numel() for s_ in slist)   # boxes: the rows of 5 that the copies below hold
     else:
         numpy_in = isinstance(boxes, np.ndarray)
         if numpy_in:
             boxes, scores = torch.from_numpy(boxes), torch.from_numpy(scores)
-        odev = boxes.device
         if offsets is None:
             raise ValueError("packed boxes need the frame offsets")
-        offsets = torch.as_tensor(offsets).to(torch.int64).cpu()
-    if len(boxes) != len(scores) or int(offsets[-1]) != len(boxes):
-        raise ValueError("Numbers of boxes and scores are inconsistent!")
+        fr = _frames.Frames(offsets, None, False, numpy_in, boxes.device)
+        counts = len(boxes), len(scores)
+    fr.expect(*counts, "boxes, scores")
     iou_type = getattr(IouType, iou_method.upper())
     if iou_type not in (IouType.BOX, IouType.RBOX):
         raise ValueError("Unsupported iou type!")
     sup_type = getattr(SupressionType, supression_method.upper())
+    if fr.as_list:   # frame by frame to the device (asynchronous copies from pinned host memory), concatenated there
+        boxes = torch.cat([_c.to_device(b).reshape(-1, 5) for b in blist], 0)
+        scores = torch.cat([_c.to_device(s_).reshape(-1) for s_ in slist], 0)
     b, s_ = _c.to_device(boxes), _c.to_device(scores)
     if precise:
         b, s_ = b.to(torch.float64), s_.to(torch.float64)
     elif s_.dtype != b.dtype:
         s_ = s_.to(b.dtype)
     b, s_ = b.contiguous(), s_.contiguous()
-    total, nframes = int(b.shape[0]), int(offsets.numel()) - 1
-    max_frame = int((offsets[1:] - offsets[:-1]).max()) if nframes > 0 else 0
+    total, nframes = int(b.shape[0]), fr.nframes
+    max_frame = fr.bounds()[0]
     suppressed = torch.zeros(total, dtype=torch.uint8, device=b.device)
     if total > 0 and max_frame > 8192:
-        for f in range(nframes):
-            lo, hi = int(offsets[f]), int(offsets[f + 1])
-            if hi > lo:
-                suppressed[lo:hi] = nms2d_cuda(b[lo:hi], s_[lo:hi], iou_type, sup_type, iou_threshold, score_threshold, supression_param).view(torch.uint8)
+        for _, r, _, _ in fr.each(fr.lengths()[0] > 0):
+            suppressed[r] = nms2d_cuda(b[r], s_[r], iou_type, sup_type, iou_threshold, score_threshold, supression_param).view(torch.uint8)
     elif total > 0:
         code = _c.dtype_code(b.dtype)
-        od = offsets.to(b.device, non_blocking=True) if offsets_dev is None else offsets_dev
+        od = _frames.to_device(b.device, fr.rows)[0] if offsets_dev is None else offsets_dev
         if sup_type == SupressionType.HARD:
             ws = _c.workspace(_c.nms_batch_workspace_bytes(total, nframes, max_frame, code), b.device)
             with torch.cuda.device(b.device):
@@ -478,13 +399,55 @@ def box2d_nms_batch(boxes, scores, offsets=None, iou_method="box", iou_threshold
                                                float(iou_threshold), float(score_threshold), float(supression_param), _c.ptr(suppressed),
                                                _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box2d_nms_batch")
-    keep = ~suppressed.view(torch.bool)
-    if odev.type != "cuda":
-        keep = keep.cpu()
-    if as_list:
-        out = [keep[int(offsets[f]):int(offsets[f + 1])] for f in range(nframes)]
-        return [k.cpu().numpy() for k in out] if numpy_in else out
-    return keep.cpu().numpy() if numpy_in else keep
+    keep = fr.outputs(rows=(~suppressed.view(torch.bool),))
+    return [k for k, in keep] if fr.as_list else keep[0]
+
+
+_PLANE = {0: ([1, 2], [1, 2, 4, 5, 6]), 1: ([0, 2], [0, 2, 3, 5, 6]), 2: ([0, 1], [0, 1, 3, 4, 6])}   # box3dp_crop / box3dr_pdist's columns
+
+
+def _check_axis(project_axis):
+    if project_axis not in (0, 1, 2):
+        raise ValueError("The projection axis can only be 0-x, 1-y and 2-z!")
+
+
+def _check_crop2d(points, boxes):   # box2dr_crop's checks
+    if len(points.shape) != 2 or points.shape[1] != 2:
+        raise ValueError("Input points should be Nx2 tensors!")
+    if len(boxes.shape) != 2 or boxes.shape[1] != 5:
+        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+
+
+def _check_pdist2d(points, boxes):   # box2dr_pdist's checks
+    if len(boxes.shape) != 2:
+        raise ValueError("Input boxes should be Nx2 tensors!")
+    if boxes.shape[1] != 5:
+        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+    if len(points.shape) != 2 or points.shape[1] != 2:
+        raise ValueError("Input points should be Nx2 tensors!")
+
+
+def _check_3d(points, boxes):
+    if len(points.shape) != 2 or points.shape[1] != 3:
+        raise ValueError("Input points should be Nx3 tensors!")
+    if len(boxes.shape) != 2 or boxes.shape[1] != 7:
+        raise ValueError("Input boxes should have 7 fields: x, y, z, lx, ly, lz, r")
+
+
+def _crop_axis_mask(points, boxes, project_axis):
+    """box3dp_crop's test along the projected axis, [M, N]"""
+    points_p = points[:, [project_axis]].t()
+    boxes_p = boxes[:, [project_axis]]
+    boxes_pd = boxes[:, [3 + project_axis]] / 2
+    return (points_p - boxes_pd < boxes_p) & (boxes_p < points_p + boxes_pd)
+
+
+def _point_box_pair(points, boxes):
+    """points and boxes on the device; their dtypes are checked first"""
+    _c.dtype_code(points.dtype)
+    if boxes.dtype != points.dtype:
+        raise RuntimeError("points and boxes must have the same dtype")
+    return _c.to_device(points), _c.to_device(boxes)
 
 
 def crop_2dr_cuda(points, boxes, out=None):
@@ -511,10 +474,7 @@ def box2dr_crop(points, boxes):
     :param points: The input point points, shape: N x 2
     :param boxes: Input boxes array, shape: M x 5
     '''
-    if len(points.shape) != 2 or points.shape[1] != 2:
-        raise ValueError("Input points should be Nx2 tensors!")
-    if len(boxes.shape) != 2 or boxes.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
+    _check_crop2d(points, boxes)
     odev = points.device
     r = crop_2dr_cuda(_c.to_device(points).contiguous(), _c.to_device(boxes).contiguous())
     return r if odev.type == "cuda" else r.cpu()
@@ -528,20 +488,10 @@ def box3dp_crop(points, boxes, project_axis=2):
     :param boxes: Input boxes array, shape: M x 7
     :param project_axis: Axis for the box to be projected to. {0: x, 1: y, 2: z}
     '''
-    if project_axis == 0:
-        points_2d, boxes_2d = points[:, [1, 2]], boxes[:, [1, 2, 4, 5, 6]]
-    elif project_axis == 1:
-        points_2d, boxes_2d = points[:, [0, 2]], boxes[:, [0, 2, 3, 5, 6]]
-    elif project_axis == 2:
-        points_2d, boxes_2d = points[:, [0, 1]], boxes[:, [0, 1, 3, 4, 6]]
-    else:
-        raise ValueError("The projection axis can only be 0-x, 1-y and 2-z!")
-    mask_2d = box2dr_crop(points_2d, boxes_2d)
-    points_p = points[:, [project_axis]].t()
-    boxes_p = boxes[:, [project_axis]]
-    boxes_pd = boxes[:, [3 + project_axis]] / 2
-    mask_p = (points_p - boxes_pd < boxes_p) & (boxes_p < points_p + boxes_pd)
-    return mask_2d & mask_p.to(mask_2d.device)
+    _check_axis(project_axis)
+    pc, bc = _PLANE[project_axis]
+    mask_2d = box2dr_crop(points[:, pc], boxes[:, bc])
+    return mask_2d & _crop_axis_mask(points, boxes, project_axis).to(mask_2d.device)
 
 
 class PDist2DR(torch.autograd.Function):
@@ -596,12 +546,7 @@ def box2dr_pdist(points, boxes, method="rbox"):
     :param method: 'rbox' - rotated box
     :return: M x N
     '''
-    if len(boxes.shape) != 2:
-        raise ValueError("Input boxes should be Nx2 tensors!")
-    if boxes.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
-    if len(points.shape) != 2 or points.shape[1] != 2:
-        raise ValueError("Input points should be Nx2 tensors!")
+    _check_pdist2d(points, boxes)
     if method != "rbox":
         raise ValueError("Only supported rotated boxes by now!")
     odev = points.device
@@ -618,15 +563,9 @@ def box3dr_pdist(points, boxes, project_axis=2):
     :param project_axis: Axis for the box to be projected to. {0: x, 1: y, 2: z}
     :return: M x N
     '''
-    if project_axis == 0:
-        points_2d, boxes_2d = points[:, [1, 2]], boxes[:, [1, 2, 4, 5, 6]]
-    elif project_axis == 1:
-        points_2d, boxes_2d = points[:, [0, 2]], boxes[:, [0, 2, 3, 5, 6]]
-    elif project_axis == 2:
-        points_2d, boxes_2d = points[:, [0, 1]], boxes[:, [0, 1, 3, 4, 6]]
-    else:
-        raise ValueError("The projection axis can only be 0-x, 1-y and 2-z!")
-    dist_2d = box2dr_pdist(points_2d, boxes_2d)
+    _check_axis(project_axis)
+    pc, bc = _PLANE[project_axis]
+    dist_2d = box2dr_pdist(points[:, pc], boxes[:, bc])
     dist_p = seg1d_pdist(points[:, project_axis], boxes[:, [project_axis, 3 + project_axis]]).to(dist_2d.device)
     # on an edge of the prism (both terms 0) the square root has no derivative: take it of 1 there, so that its backward, which runs
     # for every pair whichever branch is selected, multiplies by a finite number instead of 0 * inf = NaN
@@ -638,125 +577,35 @@ def box3dr_pdist(points, boxes, project_axis=2):
 
 
 # ------------------------------------------------------------------ frame-batched point <-> box operators
-_PLANE = {0: ([1, 2], [1, 2, 4, 5, 6]), 1: ([0, 2], [0, 2, 3, 5, 6]), 2: ([0, 1], [0, 1, 3, 4, 6])}   # box3dp_crop / box3dr_pdist's columns
-
-
-def _check_axis(project_axis):
-    if project_axis not in (0, 1, 2):
-        raise ValueError("The projection axis can only be 0-x, 1-y and 2-z!")
-
-
-def _check_crop2d(points, boxes):   # box2dr_crop's checks
-    if len(points.shape) != 2 or points.shape[1] != 2:
-        raise ValueError("Input points should be Nx2 tensors!")
-    if len(boxes.shape) != 2 or boxes.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
-
-
-def _check_pdist2d(points, boxes):   # box2dr_pdist's checks
-    if len(boxes.shape) != 2:
-        raise ValueError("Input boxes should be Nx2 tensors!")
-    if boxes.shape[1] != 5:
-        raise ValueError("Input boxes should have 5 fields: x, y, w, h, r")
-    if len(points.shape) != 2 or points.shape[1] != 2:
-        raise ValueError("Input points should be Nx2 tensors!")
-
-
-def _check_3d(points, boxes):
-    if len(points.shape) != 2 or points.shape[1] != 3:
-        raise ValueError("Input points should be Nx3 tensors!")
-    if len(boxes.shape) != 2 or boxes.shape[1] != 7:
-        raise ValueError("Input boxes should have 7 fields: x, y, z, lx, ly, lz, r")
-
-
-def _point_box_inputs(points, boxes, point_offsets, box_offsets, check):
-    """(points, boxes on the device, CPU point / box offsets, list form?, numpy in?, device of the inputs) of a batch call.  The list
-    form is concatenated with torch.cat, so autograd reaches every per-frame tensor."""
-    as_list = isinstance(points, (list, tuple))
-    if as_list:
-        if not isinstance(boxes, (list, tuple)) or len(points) != len(boxes):
-            raise ValueError("points and boxes should hold the same number of frames")
-        numpy_in = isinstance(points[0], np.ndarray)
-        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
-        pl, bl = [tt(p) for p in points], [tt(b) for b in boxes]
-        for p, b in zip(pl, bl):
-            check(p, b)
-        if len({x.dtype for x in pl + bl}) != 1:
-            raise RuntimeError("points and boxes must have the same dtype")
-        poff, boff = _frame_offsets(lens=[len(p) for p in pl]), _frame_offsets(lens=[len(b) for b in bl])
-        P, B = torch.cat(pl), torch.cat(bl)
-    else:
-        numpy_in = isinstance(points, np.ndarray)
-        if numpy_in:
-            assert isinstance(boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
-            points, boxes = torch.from_numpy(points), torch.from_numpy(boxes)
-        if point_offsets is None or box_offsets is None:
-            raise ValueError("packed points and boxes need the frame offsets")
-        check(points, boxes)
-        poff, boff = _frame_offsets(point_offsets), _frame_offsets(box_offsets)
-        P, B = points, boxes
-    if poff.numel() != boff.numel() or int(poff[-1]) != len(P) or int(boff[-1]) != len(B):
-        raise ValueError("Numbers of points, boxes and frame offsets are inconsistent!")
-    _c.dtype_code(P.dtype)
-    if B.dtype != P.dtype:
-        raise RuntimeError("points and boxes must have the same dtype")
-    return _c.to_device(P), _c.to_device(B), poff, boff, as_list, numpy_in, P.device
-
-
-def _point_box_outputs(flat, blk, poff, boff, as_list, numpy_in, odev):
-    """packed (flat, block offsets) or the list of per-frame [M_f, N_f] views, on the inputs' side (numpy, host or device)"""
-    if odev.type != "cuda" or numpy_in:
-        flat = flat.cpu()
-    if numpy_in:
-        flat, blk = flat.detach().numpy(), blk.numpy()
-    if not as_list:
-        return flat, blk
-    return [flat[int(blk[f]):int(blk[f + 1])].reshape(int(boff[f + 1] - boff[f]), int(poff[f + 1] - poff[f])) for f in range(len(poff) - 1)]
-
-
-def _device_offsets(poff, boff, blk, dev):
-    """the three offset arrays on the device with one copy"""
-    nf = poff.numel() - 1
-    offs = torch.cat([poff, boff, blk]).to(dev, non_blocking=True)
-    return offs[:nf + 1], offs[nf + 1:2 * nf + 2], offs[2 * nf + 2:]
-
-
-def _crop_axis_mask(points, boxes, project_axis):
-    """box3dp_crop's test along the projected axis, [M, N]"""
-    points_p = points[:, [project_axis]].t()
-    boxes_p = boxes[:, [project_axis]]
-    boxes_pd = boxes[:, [3 + project_axis]] / 2
-    return (points_p - boxes_pd < boxes_p) & (boxes_p < points_p + boxes_pd)
-
-
 def _crop_batch(points, boxes, point_offsets, box_offsets, project_axis):
-    check = _check_crop2d if project_axis < 0 else _check_3d
-    P, B, poff, boff, as_list, numpy_in, odev = _point_box_inputs(points, boxes, point_offsets, box_offsets, check)
+    if _frames.empty(points):   # whatever `boxes` holds
+        return []
+    P, B, fr = _frames.inputs(points, boxes, point_offsets, box_offsets, _check_crop2d if project_axis < 0 else _check_3d, ("points", "boxes"))
+    P, B = _point_box_pair(P, B)
+    fr = fr.T   # the masks are [boxes, points] blocks
     code = _c.dtype_code(P.dtype)
-    nframes = poff.numel() - 1
-    pairs = (poff[1:] - poff[:-1]) * (boff[1:] - boff[:-1])
-    blk = _block_offsets(boff, poff)
-    mask = torch.empty(int(blk[-1]), dtype=torch.bool, device=P.device)
-    big = pairs >= int(_c.crop_grid_min_pairs())   # the single-frame grid path is faster on these
-    small = (pairs > 0) & ~big
+    n_b, n_p = fr.lengths()
+    mask = torch.empty(int(fr.blocks[-1]), dtype=torch.bool, device=P.device)
+    big = n_b * n_p >= int(_c.crop_grid_min_pairs())   # the single-frame grid path is faster on these
+    small = (n_b * n_p > 0) & ~big
     if bool(small.any()):
-        od_p, od_b, od_m = _device_offsets(poff, boff, blk, P.device)
+        od_b, od_p, od_m = _frames.to_device(P.device, fr.rows, fr.cols, fr.blocks)
+        max_b, max_p = fr.bounds(small)
         ws = _c.workspace(_c.crop_batch_workspace_bytes(len(B), code), P.device)
         with torch.cuda.device(P.device):
-            st = _c.crop2dr_batch[code](_c.ptr(P), len(P), _c.ptr(od_p), _c.ptr(B), len(B), _c.ptr(od_b), nframes,
-                                        int((poff[1:] - poff[:-1])[small].max()), int((boff[1:] - boff[:-1])[small].max()), project_axis,
+            st = _c.crop2dr_batch[code](_c.ptr(P), len(P), _c.ptr(od_p), _c.ptr(B), len(B), _c.ptr(od_b), fr.nframes, max_p, max_b, project_axis,
                                         _c.ptr(od_m), _c.ptr(mask), _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box2dr_crop_batch" if project_axis < 0 else "box3dp_crop_batch")
-    for f in torch.nonzero(big).flatten().tolist():
-        p, b = P[int(poff[f]):int(poff[f + 1])], B[int(boff[f]):int(boff[f + 1])]
-        block = mask[int(blk[f]):int(blk[f + 1])].view(len(b), len(p))
+    for _, rb, cp, k in fr.each(big):
+        p, b = P[cp], B[rb]
+        block = mask[k].view(len(b), len(p))
         if project_axis < 0:
             crop_2dr_cuda(p, b, out=block)
         else:
             pc, bc = _PLANE[project_axis]
             crop_2dr_cuda(p[:, pc].contiguous(), b[:, bc].contiguous(), out=block)
             block &= _crop_axis_mask(p, b, project_axis)
-    return _point_box_outputs(mask, blk, poff, boff, as_list, numpy_in, odev)
+    return fr.matrices(mask)
 
 
 def box2dr_crop_batch(points, boxes, point_offsets=None, box_offsets=None):
@@ -768,8 +617,6 @@ def box2dr_crop_batch(points, boxes, point_offsets=None, box_offsets=None):
     f's mask is ``mask_flat[mask_offsets[f]:mask_offsets[f + 1]].view(M_f, N_f)``, ``mask_offsets`` the running sum of M_f * N_f).
     numpy in -> numpy out, host tensors in -> host tensors out.
     '''
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _crop_batch(points, boxes, point_offsets, box_offsets, -1)
 
 
@@ -779,8 +626,6 @@ def box3dp_crop_batch(points, boxes, point_offsets=None, box_offsets=None, proje
     per frame the mask equals :func:`box3dp_crop` on that frame, bit for bit (the test along ``project_axis`` runs in the kernel).
     '''
     _check_axis(project_axis)
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _crop_batch(points, boxes, point_offsets, box_offsets, project_axis)
 
 
@@ -797,21 +642,17 @@ def _crop_assign_frame(p, b, project_axis, point_box, box_npoints):
 
 
 def _crop_assign(points, boxes, project_axis):
-    check = _check_crop2d if project_axis < 0 else _check_3d
     numpy_in = isinstance(points, np.ndarray)
     if numpy_in:
         assert isinstance(boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
         points, boxes = torch.from_numpy(points), torch.from_numpy(boxes)
-    check(points, boxes)
-    _c.dtype_code(points.dtype)
-    if boxes.dtype != points.dtype:
-        raise RuntimeError("points and boxes must have the same dtype")
-    odev = points.device
-    P, B = _c.to_device(points.detach()), _c.to_device(boxes.detach())
+    (_check_crop2d if project_axis < 0 else _check_3d)(points, boxes)
+    P, B = _point_box_pair(points.detach(), boxes.detach())
     point_box = torch.empty(len(P), dtype=torch.int64, device=P.device)
     box_npoints = torch.empty(len(B), dtype=torch.int64, device=P.device)
     _crop_assign_frame(P, B, project_axis, point_box, box_npoints)
-    return _reduction_outputs((point_box, box_npoints), odev, numpy_in)
+    fr = _frames.Frames([0, len(P)], [0, len(B)], False, numpy_in, points.device)   # one frame
+    return fr.outputs(rows=(point_box,), cols=(box_npoints,))
 
 
 def box2dr_crop_assign(points, boxes):
@@ -841,32 +682,27 @@ def box3dp_crop_assign(points, boxes, project_axis=2):
 
 
 def _crop_assign_batch(points, boxes, point_offsets, box_offsets, project_axis):
-    check = _check_crop2d if project_axis < 0 else _check_3d
-    P, B, poff, boff, as_list, numpy_in, odev = _point_box_inputs(points, boxes, point_offsets, box_offsets, check)
-    P, B = P.detach().contiguous(), B.detach().contiguous()
+    if _frames.empty(points):   # whatever `boxes` holds
+        return []
+    P, B, fr = _frames.inputs(points, boxes, point_offsets, box_offsets, _check_crop2d if project_axis < 0 else _check_3d, ("points", "boxes"))
+    P, B = _point_box_pair(P.detach(), B.detach())
+    P, B = P.contiguous(), B.contiguous()
     code = _c.dtype_code(P.dtype)
-    nframes = poff.numel() - 1
-    n_f, m_f = poff[1:] - poff[:-1], boff[1:] - boff[:-1]
+    n_p, n_b = fr.lengths()
     point_box = torch.empty(len(P), dtype=torch.int64, device=P.device)
     box_npoints = torch.empty(len(B), dtype=torch.int64, device=P.device)
-    big = n_f * m_f >= int(_c.crop_grid_min_pairs())   # the single-frame entry (grid path) computes these
-    small = (n_f * m_f > 0) & ~big
-    if nframes and len(P) + len(B):
-        offs = torch.cat([poff, boff]).to(P.device, non_blocking=True)   # one copy of both offset arrays
+    big = n_p * n_b >= int(_c.crop_grid_min_pairs())   # the single-frame entry (grid path) computes these
+    if fr.nframes and len(P) + len(B):
+        od_p, od_b = _frames.to_device(P.device, fr.rows, fr.cols)
         ws = _c.workspace(_c.crop_assign_batch_workspace_bytes(len(B), code), P.device)
-        any_small = bool(small.any())
-        with torch.cuda.device(P.device):
-            st = _c.crop2dr_assign_batch[code](_c.ptr(P), len(P), _c.ptr(offs[:nframes + 1]), _c.ptr(B), len(B), _c.ptr(offs[nframes + 1:]), nframes,
-                                               int(n_f[small].max()) if any_small else 1, int(m_f[small].max()) if any_small else 1, project_axis,
-                                               _c.ptr(point_box), _c.ptr(box_npoints), _c.ptr(ws), ws.numel(), _c.stream_ptr())
+        max_p, max_b = fr.bounds((n_p * n_b > 0) & ~big)
+        with torch.cuda.device(P.device):   # bounds of 1 when no frame is left to it: the call still initialises every output slice
+            st = _c.crop2dr_assign_batch[code](_c.ptr(P), len(P), _c.ptr(od_p), _c.ptr(B), len(B), _c.ptr(od_b), fr.nframes, max_p or 1, max_b or 1,
+                                               project_axis, _c.ptr(point_box), _c.ptr(box_npoints), _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box2dr_crop_assign_batch" if project_axis < 0 else "box3dp_crop_assign_batch")
-    for f in torch.nonzero(big).flatten().tolist():   # after the batch call, which initialises every slice
-        p0, p1, b0, b1 = int(poff[f]), int(poff[f + 1]), int(boff[f]), int(boff[f + 1])
-        _crop_assign_frame(P[p0:p1], B[b0:b1], project_axis, point_box[p0:p1], box_npoints[b0:b1])
-    pb, bn = _reduction_outputs((point_box, box_npoints), odev, numpy_in)
-    if not as_list:
-        return pb, bn
-    return [(pb[int(poff[f]):int(poff[f + 1])], bn[int(boff[f]):int(boff[f + 1])]) for f in range(nframes)]
+    for _, r, c, _ in fr.each(big):   # after the batch call, which initialises every slice
+        _crop_assign_frame(P[r], B[c], project_axis, point_box[r], box_npoints[c])
+    return fr.outputs(rows=(point_box,), cols=(box_npoints,))
 
 
 def box2dr_crop_assign_batch(points, boxes, point_offsets=None, box_offsets=None):
@@ -877,8 +713,6 @@ def box2dr_crop_assign_batch(points, boxes, point_offsets=None, box_offsets=None
     (int64 [nframes + 1], CPU) (returns the packed ``(point_box [total_points], box_npoints [total_boxes])``, with FRAME-LOCAL box indices
     as :func:`box2d_iou_max_batch` gives them).  The outputs carry no grad.  numpy in -> numpy out, host tensors in -> host tensors out.
     '''
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _crop_assign_batch(points, boxes, point_offsets, box_offsets, -1)
 
 
@@ -888,8 +722,6 @@ def box3dp_crop_assign_batch(points, boxes, point_offsets=None, box_offsets=None
     :func:`box2dr_crop_assign_batch`, and per frame the outputs equal :func:`box3dp_crop_assign` on that frame exactly.
     '''
     _check_axis(project_axis)
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _crop_assign_batch(points, boxes, point_offsets, box_offsets, project_axis)
 
 
@@ -926,17 +758,17 @@ class _PDistBatch(torch.autograd.Function):
 
 
 def _pdist_batch(points, boxes, point_offsets, box_offsets, project_axis):
-    check = _check_pdist2d if project_axis < 0 else _check_3d
-    P, B, poff, boff, as_list, numpy_in, odev = _point_box_inputs(points, boxes, point_offsets, box_offsets, check)
+    if _frames.empty(points):   # whatever `boxes` holds
+        return []
+    P, B, fr = _frames.inputs(points, boxes, point_offsets, box_offsets, _check_pdist2d if project_axis < 0 else _check_3d, ("points", "boxes"))
+    P, B = _point_box_pair(P, B)
     if project_axis >= 0:
         assert torch.all(B[:, 3 + project_axis] > 0)   # seg1d_pdist's condition, once for the batch
-    nframes = poff.numel() - 1
-    n_f, m_f = poff[1:] - poff[:-1], boff[1:] - boff[:-1]
-    blk = _block_offsets(boff, poff)
-    offsets = _device_offsets(poff, boff, blk, P.device)
-    dist = _PDistBatch.apply(P.contiguous(), B.contiguous(), offsets, nframes, int(n_f.max()) if nframes else 0, int(m_f.max()) if nframes else 0,
-                             project_axis, int(blk[-1]))
-    return _point_box_outputs(dist, blk, poff, boff, as_list, numpy_in, odev)
+    fr = fr.T   # the distances are [boxes, points] blocks
+    max_b, max_p = fr.bounds()
+    od_b, od_p, od_d = _frames.to_device(P.device, fr.rows, fr.cols, fr.blocks)
+    dist = _PDistBatch.apply(P.contiguous(), B.contiguous(), (od_p, od_b, od_d), fr.nframes, max_p, max_b, project_axis, int(fr.blocks[-1]))
+    return fr.matrices(dist)
 
 
 def box2dr_pdist_batch(points, boxes, point_offsets=None, box_offsets=None):
@@ -945,8 +777,6 @@ def box2dr_pdist_batch(points, boxes, point_offsets=None, box_offsets=None):
     Call forms and outputs as :func:`box2dr_crop_batch`, with T [M_f, N_f] distances; per frame the values equal :func:`box2dr_pdist`
     on that frame bit for bit, and the gradients agree to rounding (both sum with atomics).
     '''
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _pdist_batch(points, boxes, point_offsets, box_offsets, -1)
 
 
@@ -957,8 +787,6 @@ def box3dr_pdist_batch(points, boxes, point_offsets=None, box_offsets=None, proj
     :func:`box3dr_pdist` bit for bit.  Non-positive extents along the axis raise AssertionError, as in :func:`seg1d_pdist`.
     '''
     _check_axis(project_axis)
-    if isinstance(points, (list, tuple)) and len(points) == 0:
-        return []
     return _pdist_batch(points, boxes, point_offsets, box_offsets, project_axis)
 
 
@@ -1121,25 +949,6 @@ def match_greedy(distance, src_scores, src_tags, dst_tags, thresholds):
     return (sa.numpy(), da.numpy()) if convert_numpy else (sa, da)
 
 
-def _frame_offsets(offsets=None, lens=None):
-    """CPU int64 [nframes + 1] from given offsets or from frame lengths"""
-    if lens is not None:
-        off = torch.zeros(len(lens) + 1, dtype=torch.int64)
-        off[1:] = torch.tensor(lens, dtype=torch.int64).cumsum(0)
-        return off
-    off = torch.as_tensor(offsets).to(torch.int64).cpu().reshape(-1)
-    if off.numel() < 1 or int(off[0]) != 0 or bool((off[1:] < off[:-1]).any()):
-        raise ValueError("frame offsets must start at 0 and be ascending")
-    return off
-
-
-def _block_offsets(src_off, dst_off):
-    """start of every frame's [n_f, m_f] block in the packed distance buffer: the running sum of n_f * m_f"""
-    off = torch.zeros_like(src_off)
-    off[1:] = ((src_off[1:] - src_off[:-1]) * (dst_off[1:] - dst_off[:-1])).cumsum(0)
-    return off
-
-
 def box3d_iou_distance_batch(src_boxes, dst_boxes, src_offsets=None, dst_offsets=None, metric="riou"):
     '''
     :func:`box3d_iou_distance` on a batch of frames in one launch sequence (the detection evaluator computes one matrix per frame of a
@@ -1151,55 +960,21 @@ def box3d_iou_distance_batch(src_boxes, dst_boxes, src_offsets=None, dst_offsets
 
     :param metric: 'riou' or 'iou', as in :func:`box3d_iou_distance`
     '''
-    as_list = isinstance(src_boxes, (list, tuple))
-    if as_list:
-        if not isinstance(dst_boxes, (list, tuple)) or len(src_boxes) != len(dst_boxes):
-            raise ValueError("src_boxes and dst_boxes should hold the same number of frames")
-        if len(src_boxes) == 0:
-            return []
-        numpy_in = isinstance(src_boxes[0], np.ndarray)
-        tt = lambda x: torch.from_numpy(x) if isinstance(x, np.ndarray) else x  # noqa: E731
-        slist, dlist = [tt(b) for b in src_boxes], [tt(b) for b in dst_boxes]
-        for a, b in zip(slist, dlist):
-            _check_boxes3d(a, b)
-        odev = slist[0].device
-        src_off, dst_off = _frame_offsets(lens=[len(b) for b in slist]), _frame_offsets(lens=[len(b) for b in dlist])
-        b1 = _dist3d_input(torch.cat([b.to(torch.float32) for b in slist]))   # one copy to the device per box set
-        b2 = _dist3d_input(torch.cat([b.to(torch.float32) for b in dlist]))
-    else:
-        numpy_in = isinstance(src_boxes, np.ndarray)
-        if numpy_in:
-            assert isinstance(dst_boxes, np.ndarray), "Input should be both numpy tensor or pytorch tensor!"
-            src_boxes, dst_boxes = torch.from_numpy(src_boxes), torch.from_numpy(dst_boxes)
-        if src_offsets is None or dst_offsets is None:
-            raise ValueError("packed boxes need the frame offsets")
-        _check_boxes3d(src_boxes, dst_boxes)
-        odev = src_boxes.device
-        src_off, dst_off = _frame_offsets(src_offsets), _frame_offsets(dst_offsets)
-        b1, b2 = _dist3d_input(src_boxes), _dist3d_input(dst_boxes)
-    if src_off.numel() != dst_off.numel() or int(src_off[-1]) != len(b1) or int(dst_off[-1]) != len(b2):
-        raise ValueError("Numbers of boxes and frame offsets are inconsistent!")
+    if _frames.empty(src_boxes, dst_boxes):
+        return []
+    A, B, fr = _frames.inputs(src_boxes, dst_boxes, src_offsets, dst_offsets, _check_boxes3d, ("src_boxes", "dst_boxes"), dtype=torch.float32)
     if metric.lower() not in ("riou", "iou"):
         raise ValueError("Unrecognized distance metric!")
-    nframes = src_off.numel() - 1
-    dist_off = _block_offsets(src_off, dst_off)
-    dist = torch.empty(int(dist_off[-1]), dtype=torch.float32, device=b1.device)
+    b1, b2 = _dist3d_input(A), _dist3d_input(B)   # one copy to the device per box set
+    dist = torch.empty(int(fr.blocks[-1]), dtype=torch.float32, device=b1.device)
     if dist.numel():
-        n_f, m_f = src_off[1:] - src_off[:-1], dst_off[1:] - dst_off[:-1]
-        offs = torch.cat([src_off, dst_off, dist_off]).to(b1.device, non_blocking=True)   # one copy of the three offset arrays
-        od1, od2, odd = offs[:nframes + 1], offs[nframes + 1:2 * nframes + 2], offs[2 * nframes + 2:]
-        ws = _c.workspace(_c.iou3d_distance_batch_workspace_bytes(len(b1), len(b2), nframes), b1.device)
+        od1, od2, odd = _frames.to_device(b1.device, fr.rows, fr.cols, fr.blocks)
+        ws = _c.workspace(_c.iou3d_distance_batch_workspace_bytes(len(b1), len(b2), fr.nframes), b1.device)
         with torch.cuda.device(b1.device):
-            st = _c.iou3d_distance_batch(_c.ptr(b1), len(b1), _c.ptr(od1), _c.ptr(b2), len(b2), _c.ptr(od2), nframes, int(n_f.max()), int(m_f.max()),
+            st = _c.iou3d_distance_batch(_c.ptr(b1), len(b1), _c.ptr(od1), _c.ptr(b2), len(b2), _c.ptr(od2), fr.nframes, *fr.bounds(),
                                          1 if metric.lower() == "riou" else 0, _c.ptr(odd), _c.ptr(dist), _c.ptr(ws), ws.numel(), _c.stream_ptr())
         _c.check(st, "box3d_iou_distance_batch")
-    if odev.type != "cuda" or numpy_in:
-        dist = dist.cpu()
-    if numpy_in:
-        dist, dist_off = dist.numpy(), dist_off.numpy()
-    if not as_list:
-        return dist, dist_off
-    return [dist[int(dist_off[f]):int(dist_off[f + 1])].reshape(int(src_off[f + 1] - src_off[f]), int(dst_off[f + 1] - dst_off[f])) for f in range(nframes)]
+    return fr.matrices(dist)
 
 
 def _frame_score_order(scores, src_off_dev, nframes):
@@ -1226,21 +1001,18 @@ def match_greedy_batch(distance, src_scores, src_tags, dst_tags, thresholds, src
     shared by all frames.  Frames of more than 4096 destination boxes fall back to one :func:`match_greedy` call per frame.
     numpy in -> numpy out, host tensors in -> host tensors out.
     '''
-    as_list = src_offsets is None and dst_offsets is None
-    if as_list:
+    if src_offsets is None and dst_offsets is None:
         frames = list(distance)
         if not len(frames) == len(src_scores) == len(src_tags) == len(dst_tags):
             raise ValueError("distance, scores and tags should hold the same number of frames")
         if not frames:
             return []
-        numpy_in = isinstance(frames[0], np.ndarray)
         dl = [_as_tensor(d, torch.float32) for d in frames]
         if any(d.dim() != 2 for d in dl):
             raise ValueError("distance should be an NxM matrix")
-        odev = dl[0].device
-        src_off, dst_off = _frame_offsets(lens=[d.shape[0] for d in dl]), _frame_offsets(lens=[d.shape[1] for d in dl])
-        dist_off = _block_offsets(src_off, dst_off)
-        d = _c.to_device(torch.cat([x.reshape(-1) for x in dl]))
+        fr = _frames.Frames(_frames.offsets_of(d.shape[0] for d in dl), _frames.offsets_of(d.shape[1] for d in dl), True,
+                            isinstance(frames[0], np.ndarray), dl[0].device)
+        d = torch.cat([x.reshape(-1) for x in dl])
         cat = lambda xs, dt: torch.cat([_as_tensor(x, dt).reshape(-1) for x in xs])  # noqa: E731
         scores, st, dt_ = cat(src_scores, torch.float64), cat(src_tags, torch.int32), cat(dst_tags, torch.int32)
     else:
@@ -1249,49 +1021,34 @@ def match_greedy_batch(distance, src_scores, src_tags, dst_tags, thresholds, src
         d, given = distance
         numpy_in = isinstance(d, np.ndarray)
         d = _as_tensor(d, torch.float32)
-        odev = d.device
-        d = _c.to_device(d).reshape(-1)
-        src_off, dst_off = _frame_offsets(src_offsets), _frame_offsets(dst_offsets)
-        if src_off.numel() != dst_off.numel():
-            raise ValueError("Numbers of frames in the offsets are inconsistent!")
-        dist_off = _block_offsets(src_off, dst_off)
-        if not torch.equal(_frame_offsets(given), dist_off) or int(dist_off[-1]) != d.numel():
+        fr = _frames.Frames(src_offsets, dst_offsets, False, numpy_in, d.device)
+        d = d.reshape(-1)
+        if not torch.equal(_frames.offsets(given), fr.blocks) or int(fr.blocks[-1]) != d.numel():
             raise ValueError("distance blocks do not match the frame offsets")
         scores, st, dt_ = _as_tensor(src_scores, torch.float64).reshape(-1), _as_tensor(src_tags, torch.int32), _as_tensor(dst_tags, torch.int32)
-    dev = d.device
-    nframes, total_src, total_dst = src_off.numel() - 1, int(src_off[-1]), int(dst_off[-1])
+    total_src, total_dst = int(fr.rows[-1]), int(fr.cols[-1])
     if len(scores) != total_src or len(st) != total_src or len(dt_) != total_dst:
         raise ValueError("scores / tags do not match the distance matrix")
     thr = _as_tensor(thresholds, torch.float32)
     single = thr.dim() == 1
-    thr = (thr.reshape(1, -1) if single else thr).to(dev).contiguous()
+    thr = thr.reshape(1, -1) if single else thr
     T, ncat = thr.shape
-    scores, st, dt_ = scores.to(dev).contiguous(), st.to(dev).contiguous(), dt_.to(dev).contiguous()
-    n_f, m_f = src_off[1:] - src_off[:-1], dst_off[1:] - dst_off[:-1]
-    max_dst = int(m_f.max()) if nframes else 0
+    d = _c.to_device(d)
+    dev = d.device
+    thr, scores, st, dt_ = thr.to(dev).contiguous(), scores.to(dev).contiguous(), st.to(dev).contiguous(), dt_.to(dev).contiguous()
+    max_dst = fr.bounds()[1]
     sa = torch.full((T, total_src), -1, dtype=torch.int32, device=dev)
     da = torch.full((T, total_dst), -1, dtype=torch.int32, device=dev)
     if max_dst > 4096:   # the kernel's taken bitmask holds 4096 destinations
-        for f in range(nframes):
-            s0, s1, d0, d1 = int(src_off[f]), int(src_off[f + 1]), int(dst_off[f]), int(dst_off[f + 1])
-            sa[:, s0:s1], da[:, d0:d1] = match_greedy(d[int(dist_off[f]):int(dist_off[f + 1])].view(s1 - s0, d1 - d0), scores[s0:s1], st[s0:s1],
-                                                      dt_[d0:d1], thr)
+        for _, r, c, k in fr.each():
+            sa[:, r], da[:, c] = match_greedy(d[k].view(r.stop - r.start, c.stop - c.start), scores[r], st[r], dt_[c], thr)
     elif T and d.numel():
-        offs = torch.cat([src_off, dst_off, dist_off]).to(dev, non_blocking=True)   # one copy of the three offset arrays
-        os_, od_, odd = offs[:nframes + 1], offs[nframes + 1:2 * nframes + 2], offs[2 * nframes + 2:]
-        order = _frame_score_order(scores, os_, nframes)
+        os_, od_, odd = _frames.to_device(dev, fr.rows, fr.cols, fr.blocks)
+        order = _frame_score_order(scores, os_, fr.nframes)
         with torch.cuda.device(dev):
-            stt = _c.match_greedy_batch(_c.ptr(d), _c.ptr(odd), _c.ptr(os_), _c.ptr(od_), nframes, max_dst, _c.ptr(order), _c.ptr(st), _c.ptr(dt_),
+            stt = _c.match_greedy_batch(_c.ptr(d), _c.ptr(odd), _c.ptr(os_), _c.ptr(od_), fr.nframes, max_dst, _c.ptr(order), _c.ptr(st), _c.ptr(dt_),
                                         _c.ptr(thr), T, ncat, _c.ptr(sa), _c.ptr(da), _c.stream_ptr())
         _c.check(stt, "match_greedy_batch")
-    if odev.type != "cuda" or numpy_in:
-        sa, da = sa.cpu(), da.cpu()
-    if numpy_in:
-        sa, da = sa.numpy(), da.numpy()
-    if not as_list:
-        return (sa[0], da[0]) if single else (sa, da)
-    out = []
-    for f in range(nframes):
-        a, b = sa[:, int(src_off[f]):int(src_off[f + 1])], da[:, int(dst_off[f]):int(dst_off[f + 1])]
-        out.append((a[0], b[0]) if single else (a, b))
-    return out
+    if single:
+        sa, da = sa[0], da[0]
+    return fr.outputs(rows=(sa,), cols=(da,))
